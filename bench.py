@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the DDRL learner hot path on B200 (contract: see the task statement / DESIGN.md §Measurement).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is ONE learner iteration of the BASELINE.json configs[1] workload
@@ -231,6 +231,32 @@ def run_reference(args):
     print(json.dumps(line))
 
 
+DUMP_ROWS = 32768      # rows per policy kept of the per-row outputs: a fixed, seeded sample when the rollout has more
+
+
+def dump_outputs(out_dir, L, stats):
+    """--dump-outputs: what one FCNetLearner.learn_on_rollout call gave its caller, as out_dir/<name>.npy in float32 / float64:
+    the per-policy stats it returned (stats_<key>), the state it left (weights, Adam moments and beta powers, observation
+    filter, KL coefficient) and the per-row outputs of its forward pass and GAE in rollout order (filtered observations,
+    actions, logits, log-probabilities, values, standardised advantages, value targets; the same DUMP_ROWS rows of every
+    policy when the rollout has more).  The inputs depend on the arguments alone, and so do the outputs, except with
+    --atomic-reduce."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {f"stats_{k}": np.array([s[k] for s in stats], dtype=np.float64) for k in stats[0]}
+    arrays.update(theta=L.theta, adam_m=L.m, adam_v=L.v, adam_beta_pow=L.beta_pow, kl_coeff=L.kl_coeff,
+                  filter_n=L.filt_n, filter_M=L.filt_M, filter_S=L.filt_S)
+    b = L._bufs
+    R = b["value"].shape[1]
+    rows = np.arange(R) if R <= DUMP_ROWS else np.sort(np.random.default_rng(0).choice(R, DUMP_ROWS, replace=False))
+    rows = torch.from_numpy(rows).to(L.device)
+    for name in ("obs", "act", "logits", "logp", "value", "adv", "vtarg"):
+        arrays[name] = b[name].index_select(1, rows)
+    for name, a in arrays.items():
+        a = a.cpu().numpy() if torch.is_tensor(a) else a
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64 if a.dtype in (np.float64, np.int64) else np.float32))
+
+
 def time_graphnet(envs, epochs, steps, warmup, step_kind="tc"):
     """BASELINE.json configs[3] — shared GraphNet policy over the 4-leg graph, `envs` envs x 4 agents, T=32, one weight set,
     minibatch = rows/32; -> (ms per learner iteration, config dict)."""
@@ -393,7 +419,17 @@ def main():
                          "SingleDiagonal, SingleToFront, TwoSides, TwoDiags; append _TVel for the target-velocity obs); "
                          "the headline line is the default FullyDecentral = BASELINE.json configs[1]")
     ap.add_argument("--gn-epochs", type=int, default=WORKLOAD["epochs"])
+    ap.add_argument("--atomic-reduce", action="store_true",
+                    help="tc SGD step: add the per-CTA partial gradients into FCNetLearner's L2 accumulation vector (float "
+                         "atomics, the library default) instead of summing them in a fixed order; faster, but the order of "
+                         "the additions changes from run to run and so do the results (profiles/r03_reduction_reproducibility.txt)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed learner iteration computed as DIR/<name>.npy (same arguments, same inputs)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "fcnet"):
+        ap.error("--dump-outputs: only the FCNet workload of --impl ours")
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.arch != "FullyDecentral":      # supplementary architectures: same harness, the architecture's P / D / A
         from ddrl_b200.policies import ARCHITECTURES
         tvel = args.arch.endswith("_TVel")
@@ -443,8 +479,10 @@ def main():
     from ddrl_b200.modelv2 import fcnet_init_flat      # the product's own GlorotUniformScaled initialiser
     gen = torch.Generator().manual_seed(1234)
     theta0 = torch.stack([fcnet_init_flat(D, 2 * A, gen) for _ in range(P)])
+    # the fixed-order reduction of the partial gradients by default: with the same arguments every run computes the same
+    # results, so the outputs of two builds can be compared (--dump-outputs)
     L = FCNetLearner(P, D, A, cfg, dev, theta=theta0, use_graph=not args.no_graph, mode=args.mode,
-                     ctas_per_policy=args.ctas or None)
+                     ctas_per_policy=args.ctas or None, atomic_reduce=args.atomic_reduce)
 
     sets = [synth_rollout(P, T, C, D, A, envs, nb, E, 1234 + rank + 100 * s, device=dev) for s in range(args.sets)]
     host = {k: v.contiguous().pin_memory() for k, v in synth_rollout(P, T, C, D, A, envs, nb, E, 999 + rank).items()
@@ -515,6 +553,8 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
+    last = {}
+
     def timed(fn, warmup, steps, sampler=None):
         for i in range(warmup):
             fn(i)
@@ -524,7 +564,7 @@ def main():
             sampler.mark(True)
         e0.record()
         for i in range(steps):
-            fn(warmup + i)
+            last["out"] = fn(warmup + i)
         e1.record()
         barrier()
         if sampler is not None:
@@ -546,6 +586,10 @@ def main():
     clocks.start()
     ms_total = timed(step_resident, args.warmup, args.steps, clocks)
     clk = clocks.stop()
+    if args.dump_outputs:      # before the e2e and kernel timings below move the learner on
+        if rank == 0:
+            dump_outputs(args.dump_outputs, L, last["out"])
+        barrier()
     # kernels per iteration: API launches outside the captured graph + graph replays x nodes
     steps_per_iter = E * nb
     G_ = L._sgd_setup(R)[2]

@@ -105,7 +105,7 @@ def test_multi_gpu_learner_equals_one_gpu_learner(mode, fuse, graph, world):
     fuse=True: ONE kernel per step with the in-kernel NVLink all-reduce (csrc/sgd_tail.cuh); fuse=False: NCCL."""
     import torch.multiprocessing as mp
     if torch.cuda.device_count() < world:
-        pytest.skip(f"needs {world} GPUs (gpurun --gpus {world})")
+        pytest.skip(f"needs {world} GPUs")
     s = socket.socket(); s.bind(("127.0.0.1", 0)); port = s.getsockname()[1]; s.close()
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
@@ -221,7 +221,7 @@ def test_multi_gpu_graphnet_learner_equals_one_gpu_learner(world):
     from ddrl_b200.config import PPOConfig
     from ddrl_b200.learner import GraphNetLearner
     if torch.cuda.device_count() < world:
-        pytest.skip(f"needs {world} GPUs (gpurun --gpus {world})")
+        pytest.skip(f"needs {world} GPUs")
     s = socket.socket(); s.bind(("127.0.0.1", 0)); port = s.getsockname()[1]; s.close()
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
