@@ -7,7 +7,7 @@ import numpy as np
 import pytest
 import torch
 
-from tests.util import ARCHS, ckpt_theta, load_ckpt, scaled_err, synth_obs, t64
+from tests.util import ARCHS, assert_grad_per_variable, ckpt_theta, load_ckpt, scaled_err, synth_obs, t64
 
 pytestmark = pytest.mark.gpu
 
@@ -166,24 +166,12 @@ def test_train_step_gradients_match_float64_autograd(arch, G, tc):
     # scale for gradients — the value branch amplifies forward round-off by |v| / |v - R| ~ 10 (the float32 torch twin
     # itself sits at ~5e-6 there); forward outputs and loss statistics stay within 1e-5.
     gtol = 5e-5 if tc else TOL
+    z = load_ckpt(arch)
+    # checkpoint shape table: [rows, cols], cols = 0 for 1-D variables
+    shapes = [(int(r),) if int(c) == 0 else (int(r), int(c)) for r, c in z[[k for k in z.files if k.endswith("/shapes")][0]]]
     for p in range(b["P"]):
         assert scaled_err(grad[p], ref[p]) < gtol, (arch, p)
-        # per-variable check so a small tensor (biases, heads) cannot hide behind a large one.  A bias gradient is a
-        # cancelling sum over rows (e.g. value_out/bias = sum_r dL/dv_r ~ 3e-4 from terms ~ 2e-2): perturbing v by
-        # 3 ulp moves it by 1e-3 relative, so its own magnitude is not a usable scale for FP32 round-off.  Each
-        # variable is held to 2e-5 of max(own scale, 1 % of the whole gradient's scale), or 4x the float32 twin.
-        o = 0
-        z = load_ckpt(arch)
-        shapes = z[[k for k in z.files if k.endswith("/shapes")][0]]
-        gscale = np.abs(ref[p]).max()
-        for shp in shapes:
-            n = int(shp[0] * max(1, shp[1]))
-            err = np.abs(grad[p][o:o + n].astype(np.float64) - ref[p][o:o + n]).max()
-            e_twin = np.abs(twin[p][o:o + n].astype(np.float64) - ref[p][o:o + n]).max()
-            # 1-D variables (biases) are pure cancelling sums over rows: floor at 5 % of the gradient's scale
-            scale = max(np.abs(ref[p][o:o + n]).max(), (0.05 if shp[1] == 0 else 0.01) * gscale)
-            assert err < max(2.0 * gtol * scale, 4.0 * e_twin), (arch, p, o, err, scale, e_twin)
-            o += n
+        assert_grad_per_variable(grad[p], ref[p], twin[p], shapes, gtol, where=(arch, p))
         s = ssum[p] / MB
         assert abs(s[0] - stats[p]["policy_loss"]) < TOL * max(1.0, abs(stats[p]["policy_loss"]))
         assert abs(s[1] - stats[p]["kl"]) < TOL * max(1.0, abs(stats[p]["kl"]))

@@ -67,3 +67,25 @@ def scaled_err(a, b):
 
 def t64(x):
     return torch.from_numpy(np.asarray(x, dtype=np.float64))
+
+
+def assert_grad_per_variable(grad, ref, twin, shapes, gtol, where=(), allow=None):
+    """Per-variable gradient check, so that a small tensor (biases, heads) cannot hide behind a large one.  grad: the kernel's
+    flat gradient, ref: float64 autograd, twin: float32 autograd of the same loss; shapes: the variables' shapes in flat order.
+    A bias gradient is a cancelling sum over rows (e.g. value_out/bias = sum_r dL/dv_r ~ 3e-4 from terms ~ 2e-2): perturbing
+    v by 3 ulp moves it by 1e-3 relative, so its own magnitude is not a usable scale for FP32 round-off.  Each variable is
+    held to 2 * gtol of max(own scale, 1 % of the whole gradient's scale; 5 % for 1-D variables, which are pure cancelling
+    sums), or 4x the float32 twin's error.  allow: {flat offset of a variable: absolute error it may have} for a variable
+    whose error the caller bounds from its own derivation."""
+    grad, ref, twin = (np.asarray(a, dtype=np.float64) for a in (grad, ref, twin))
+    gscale = np.abs(ref).max()
+    o = 0
+    for shp in shapes:
+        n = int(np.prod(shp))
+        err = np.abs(grad[o:o + n] - ref[o:o + n]).max()
+        e_twin = np.abs(twin[o:o + n] - ref[o:o + n]).max()
+        scale = max(np.abs(ref[o:o + n]).max(), (0.05 if len(shp) == 1 else 0.01) * gscale)
+        lim = max(2.0 * gtol * scale, 4.0 * e_twin, (allow or {}).get(o, 0.0))
+        assert err < lim, (*where, "variable at", o, tuple(shp), err, scale, e_twin)
+        o += n
+    assert o == ref.size, (o, ref.size)
