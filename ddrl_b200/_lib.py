@@ -116,6 +116,12 @@ PROTOTYPES = {
     "ddrl_ppo_train_step_tc": (C.c_int, [C.c_void_p] + [c_f32p] * 7 + [C.c_int, C.c_int64, C.c_int, C.c_int, C.c_int, c_i32p,
                                                                      C.c_int64, c_i32p, c_f32p, C.POINTER(PPOHyper), C.c_int,
                                                                      c_f32p, c_f64p, c_i32p, C.POINTER(SgdTail), c_stream]),
+    "ddrl_ppo_train_step_coupled": (C.c_int, [c_f32p, c_f32p, c_i32p] + [c_f32p] * 7 + [C.c_int, C.c_int64, C.c_int, C.c_int, C.c_int,
+                                                                             c_i32p, C.c_int64, c_i32p, c_f32p, C.POINTER(PPOHyper),
+                                                                             C.c_int, c_f32p, c_f64p, C.POINTER(SgdTail), c_stream]),
+    "ddrl_ppo_train_step_tc_coupled": (C.c_int, [C.c_void_p, c_f32p, c_i32p] + [c_f32p] * 7 +
+                                       [C.c_int, C.c_int64, C.c_int, C.c_int, C.c_int, c_i32p, C.c_int64, c_i32p, c_f32p,
+                                        C.POINTER(PPOHyper), C.c_int, c_f32p, c_f64p, c_i32p, C.POINTER(SgdTail), c_stream]),
     "ddrl_umma_selftest": (C.c_int, [c_f32p, C.c_int, C.c_int, c_f32p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                      C.c_int, C.c_int, c_f32p, c_i32p, c_stream]),
 }

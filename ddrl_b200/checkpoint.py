@@ -237,10 +237,17 @@ def save_rllib_checkpoint(path: str, ckpt: Checkpoint) -> None:
 
 
 # ---- learner <-> checkpoint ---------------------------------------------------------------------------------------------
+def _reject_coupled(learner) -> None:
+    if getattr(learner, "coupled", False):
+        raise ValueError("checkpoints of leg-coupled ('cup') policies are not supported: no reference checkpoint pins the "
+                         "naming of the leg_coupling variable; use get_weights / set_weights")
+
+
 def apply_to_learner(ckpt: Checkpoint, learner, policy_ids: Optional[List[str]] = None) -> None:
     """Load weights, Adam moments / beta powers, filter state and KL coefficients into an ``FCNetLearner`` (policy slot
     p <- policy_ids[p], default: checkpoint order)."""
     import torch
+    _reject_coupled(learner)
     pids = list(policy_ids or ckpt.policies.keys())
     if len(pids) != learner.P:
         raise ValueError(f"checkpoint has {len(pids)} policies, learner {learner.P}")
@@ -269,6 +276,7 @@ def apply_to_learner(ckpt: Checkpoint, learner, policy_ids: Optional[List[str]] 
 def from_learner(learner, policy_ids: List[str], stats: Optional[List[Dict[str, float]]] = None,
                  counters: Optional[Dict[str, int]] = None) -> Checkpoint:
     """Snapshot an ``FCNetLearner`` as a ``Checkpoint`` (``stats`` = the list ``learn_on_rollout`` returned)."""
+    _reject_coupled(learner)
     D, A = learner.D, learner.A
     shapes = [(D, 64), (64,), (D, 64), (64,), (64, 64), (64,), (64, 64), (64,), (64, 2 * A), (2 * A,), (64, 1), (1,)]
     pols: "OrderedDict[str, PolicyCheckpoint]" = OrderedDict()

@@ -295,282 +295,20 @@ struct TrainArgs {
     SgdTail tail;
 };
 
+// CUP = true: the leg-coupled policy of SharedDecentralLegID (see fcnet_train_tc2_cup_kernel, tc2.cu): the mean logits are
+// scaled by c[node_id[r]] before the loss, the loss gradient of the mean logits by the same factor before the backward, and
+// the table gradient sum_r dlogits[r][i] * pre[r][i] (per node) goes to flat indices [NP, NP + 8) of the partial.
+// node_id [P][R]; the table is read from a.theta [P][NP + 8] (the weights themselves come from the image); an id outside
+// 0..3 sets bit 128 of *a.tail.status.
 __global__ void __launch_bounds__(NT, 1) fcnet_train_kernel(const TrainArgs a) {
-    extern __shared__ __align__(16) float sm[];
-    const int p = blockIdx.y, G = gridDim.x, bx = blockIdx.x;
-    const int D = a.D, A = a.A, A2 = 2 * A, Dp = (D + 3) & ~3;
-    const FcSmem L = fc_smem(D, A, false, true);
-    const FcOffsets o = fc_offsets(D, A);
-    const int tid = threadIdx.x, ty = tid >> 4, tx = tid & 15, lane = tid & 31, warp = tid >> 5;
-    const int br = (tx >> 3) * H, c0 = br + (tx & 7) * 4, c1 = c0 + 32;
-    const bool ext = a.ext_dlogits != nullptr;
+    constexpr bool CUP = false;
+    const int32_t* const node_id = nullptr;
+#include "fcnet_train_body.inc"
+}
 
-    // minibatch and this CTA's row range --------------------------------------------------------
-    const int step = a.step_ctr ? *a.step_ctr : 0;
-    const int mb = a.mb_perm ? a.mb_perm[(int64_t)p * a.perm_stride + step] : step;
-    const int64_t mb0 = (int64_t)mb * a.MB;
-    const int64_t mb1 = min(mb0 + a.MB, a.R);
-    const int rpc = (((a.MB + G - 1) / G) + 7) & ~7;
-    const int64_t cr0 = min(mb0 + (int64_t)bx * rpc, mb1), cr1 = min(cr0 + rpc, mb1);
-
-    // ---- prologue: weights + first x tile + first loss inputs stream in asynchronously ----------------------
-    const float* obs_p = a.obs + (int64_t)p * a.R * D;
-    for (int i = tid; i < 2 * TM * Dp; i += NT) sm[L.x + i] = 0.f;       // both x buffers (pad columns stay zero)
-    for (int i = tid; i < 2 * TM * LDD; i += NT) sm[L.out + i] = 0.f;    // out and dl (dl pad columns stay zero)
-    __syncthreads();
-    auto prefetch_loss_inputs = [&](int64_t row0, int nrows) {
-        const int64_t g0 = (int64_t)p * a.R + row0;
-        float* pa = sm + L.pf;
-        float* po = pa + TM * A;
-        float* ps = po + TM * A2;
-        if (ext) {
-            for (int i = tid; i < nrows * A2; i += NT) cp_async4(po + i, a.ext_dlogits + g0 * A2 + i);
-            for (int i = tid; i < nrows; i += NT) cp_async4(ps + i, a.ext_dvalue + g0 + i);
-        } else {
-            for (int i = tid; i < nrows * A; i += NT) cp_async4(pa + i, a.actions + g0 * A + i);
-            for (int i = tid; i < nrows * A2; i += NT) cp_async4(po + i, a.old_logits + g0 * A2 + i);
-            for (int i = tid; i < nrows; i += NT) {
-                cp_async4(ps + i, a.old_logp + g0 + i);
-                cp_async4(ps + TM + i, a.vf_preds + g0 + i);
-                cp_async4(ps + 2 * TM + i, a.adv + g0 + i);
-                cp_async4(ps + 3 * TM + i, a.vtarg + g0 + i);
-            }
-        }
-    };
-    if (cr1 > cr0) {
-        if (a.img) load_weights_img(sm, L, a.img + (int64_t)p * L.x);
-        const int n0 = (int)min((int64_t)TM, cr1 - cr0);
-        prefetch_x_tile(sm + L.x, obs_p, cr0, n0, D);
-        prefetch_loss_inputs(cr0, n0);
-        cp_async_commit();
-        if (!a.img) load_weights_flat(sm, L, a.theta + (int64_t)p * o.NP, D, A);
-    }
-
-    // gradient accumulators (registers, live across tiles) -----------------------------------
-    float gW2[4][8], gW1[4][8], gHead[MAXHEAD];
-    float gb1 = 0.f, gb2 = 0.f, gbo = 0.f;
-    zero_acc(gW2);
-    zero_acc(gW1);
-#pragma unroll
-    for (int i = 0; i < MAXHEAD; ++i) gHead[i] = 0.f;
-    double st[DDRL_NSTAT];
-#pragma unroll
-    for (int i = 0; i < DDRL_NSTAT; ++i) st[i] = 0.0;
-
-    // dW1 row-split: ngd d-groups of 4 input features; the 16 ty-groups are shared by nsplit replicas
-    const int ngd = Dp >> 2;
-    const int nsplit = max(1, 16 / ngd);
-    const int rsplit = ty / ngd, dq = ty - rsplit * ngd;
-    const bool w1_live = rsplit < nsplit;
-
-    const float klc = ext ? 0.f : a.kl_coeff[p];
-    int xb = 0;   // x buffer holding the current tile
-
-    for (int64_t row0 = cr0; row0 < cr1; row0 += TM) {
-        const int nrows = (int)min((int64_t)TM, cr1 - row0);
-        const int xoff = xb ? L.x2 : L.x;
-        cp_async_wait_all();
-        __syncthreads();          // weights / x tile / loss inputs of this tile have landed for every thread
-        {   // prefetch the next x tile into the other buffer while this one is computed
-            const int64_t nxt = row0 + TM;
-            if (nxt < cr1) prefetch_x_tile(sm + (xb ? L.x : L.x2), obs_p, nxt, (int)min((int64_t)TM, cr1 - nxt), D);
-            cp_async_commit();
-        }
-        FcSmem Lx = L;
-        Lx.x = xoff;
-        forward_tile(sm, Lx, D, A, nrows);
-
-        // ---- per-row loss gradient -> dl[r][0..2A) = dL/dlogits, dl[r][2A] = dL/dvalue ------------
-        if (tid < TM) {
-            double s[DDRL_NSTAT];
-#pragma unroll
-            for (int i = 0; i < DDRL_NSTAT; ++i) s[i] = 0.0;
-            if (tid < nrows) {
-                float* dl = sm + L.dl + tid * LDD;
-                const float* out = sm + L.out + tid * LDD;
-                const float* pa = sm + L.pf;
-                const float* po = pa + TM * A;
-                const float* ps = po + TM * A2;
-                if (ext) {
-                    for (int i = 0; i < A2; ++i) dl[i] = po[tid * A2 + i];
-                    dl[A2] = ps[tid];
-                } else {
-                    ppo_row_loss(out, A, pa + tid * A, po + tid * A2, ps[tid], ps[TM + tid], ps[2 * TM + tid],
-                                 ps[3 * TM + tid], klc, a.hp, dl, s);
-                }
-            }
-            if (!ext) {
-#pragma unroll
-                for (int i = 0; i < DDRL_NSTAT; ++i) s[i] = warp_sum(s[i]);
-                double* red = reinterpret_cast<double*>(sm + L.red);
-                if (warp == 1 && lane == 0)
-#pragma unroll
-                    for (int i = 0; i < DDRL_NSTAT; ++i) red[i] = s[i];
-                if (tid == 0)
-#pragma unroll
-                    for (int i = 0; i < DDRL_NSTAT; ++i) st[i] += s[i];
-            }
-        }
-        __syncthreads();
-        if (tid == 0 && !ext) {
-            const double* red = reinterpret_cast<const double*>(sm + L.red);
-#pragma unroll
-            for (int i = 0; i < DDRL_NSTAT; ++i) st[i] += red[i];
-        }
-        {   // the staged loss inputs are consumed: prefetch the next tile's (same cp.async group window as x)
-            const int64_t nxt = row0 + TM;
-            if (nxt < cr1) prefetch_loss_inputs(nxt, (int)min((int64_t)TM, cr1 - nxt));
-            cp_async_commit();
-        }
-
-        // ---- B1: head weight gradients  gWo[k][o] += sum_r h2[r][k] dl[r][o] ---------------------------
-#pragma unroll
-        for (int i = 0; i < MAXHEAD; ++i) {
-            const int item = tid + i * NT;
-            if (item < H * (A2 + 1)) {
-                const int k = item & 63, oo = item >> 6;
-                const float* hcol = sm + L.h2 + (oo == A2 ? H : 0) + k;
-                const float* dcol = sm + L.dl + oo;
-                float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;
-                int r = 0;
-                for (; r + 3 < nrows; r += 4) {
-                    s0 = fmaf(hcol[r * LDH], dcol[r * LDD], s0);
-                    s1 = fmaf(hcol[(r + 1) * LDH], dcol[(r + 1) * LDD], s1);
-                    s2 = fmaf(hcol[(r + 2) * LDH], dcol[(r + 2) * LDD], s2);
-                    s3 = fmaf(hcol[(r + 3) * LDH], dcol[(r + 3) * LDD], s3);
-                }
-                for (; r < nrows; ++r) s0 = fmaf(hcol[r * LDH], dcol[r * LDD], s0);
-                gHead[i] += (s0 + s1) + (s2 + s3);
-            }
-        }
-        if (tid <= A2) {
-            float s = gbo;
-            for (int r = 0; r < nrows; ++r) s += sm[L.dl + r * LDD + tid];
-            gbo = s;
-        }
-        __syncthreads();
-
-        // ---- B2: dz2 = (dl . Wh^T) * (1 - h2^2), in place over h2 (dl columns beyond 2A are zero) ----------------
-        if (ty * 4 < nrows) {
-            float dh[4][8];
-            zero_acc(dh);
-            mm_nn(sm + L.dl + ty * 4 * LDD, LDD, sm + L.WhT + c0, sm + L.WhT + c1, HC, (A2 + 4) & ~3, dh);
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-                float* hrow = sm + L.h2 + (ty * 4 + i) * LDH;
-                const float4 h0 = *reinterpret_cast<const float4*>(hrow + c0);
-                const float4 h1v = *reinterpret_cast<const float4*>(hrow + c1);
-                float4 o0, o1;
-                o0.x = dh[i][0] * (1.f - h0.x * h0.x); o0.y = dh[i][1] * (1.f - h0.y * h0.y);
-                o0.z = dh[i][2] * (1.f - h0.z * h0.z); o0.w = dh[i][3] * (1.f - h0.w * h0.w);
-                o1.x = dh[i][4] * (1.f - h1v.x * h1v.x); o1.y = dh[i][5] * (1.f - h1v.y * h1v.y);
-                o1.z = dh[i][6] * (1.f - h1v.z * h1v.z); o1.w = dh[i][7] * (1.f - h1v.w * h1v.w);
-                *reinterpret_cast<float4*>(hrow + c0) = o0;
-                *reinterpret_cast<float4*>(hrow + c1) = o1;
-            }
-        }
-        __syncthreads();
-
-        // ---- B3: gW2[k][c] += sum_r h1[r][br+k] dz2[r][c];  gb2[c] += sum_r dz2[r][c] -------------------
-        mm_tn(sm + L.h1 + br + ty * 4, LDH, sm + L.h2 + c0, sm + L.h2 + c1, LDH, 0, nrows, 1, gW2);
-        if (tid < HC) {
-            float s0 = 0.f, s1 = 0.f;
-            int r = 0;
-            for (; r + 1 < nrows; r += 2) { s0 += sm[L.h2 + r * LDH + tid]; s1 += sm[L.h2 + (r + 1) * LDH + tid]; }
-            if (r < nrows) s0 += sm[L.h2 + r * LDH + tid];
-            gb2 += s0 + s1;
-        }
-        // ---- B4: dz1 = (dz2 . W2^T) * (1 - h1^2)  (registers), then in place over h1 --------------------
-        float dz1[4][8];
-        const bool live = ty * 4 < nrows;
-        if (live) {
-            zero_acc(dz1);
-            mm_nn(sm + L.h2 + ty * 4 * LDH + br, LDH, sm + L.W2Tc + c0, sm + L.W2Tc + c1, LDT, H, dz1);
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-                const float* hrow = sm + L.h1 + (ty * 4 + i) * LDH;
-                const float4 h0 = *reinterpret_cast<const float4*>(hrow + c0);
-                const float4 h1v = *reinterpret_cast<const float4*>(hrow + c1);
-                dz1[i][0] *= (1.f - h0.x * h0.x); dz1[i][1] *= (1.f - h0.y * h0.y);
-                dz1[i][2] *= (1.f - h0.z * h0.z); dz1[i][3] *= (1.f - h0.w * h0.w);
-                dz1[i][4] *= (1.f - h1v.x * h1v.x); dz1[i][5] *= (1.f - h1v.y * h1v.y);
-                dz1[i][6] *= (1.f - h1v.z * h1v.z); dz1[i][7] *= (1.f - h1v.w * h1v.w);
-            }
-        }
-        __syncthreads();
-        if (live) {
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-                float* dst = sm + L.h1 + (ty * 4 + i) * LDH;
-                *reinterpret_cast<float4*>(dst + c0) = make_float4(dz1[i][0], dz1[i][1], dz1[i][2], dz1[i][3]);
-                *reinterpret_cast<float4*>(dst + c1) = make_float4(dz1[i][4], dz1[i][5], dz1[i][6], dz1[i][7]);
-            }
-        }
-        __syncthreads();
-        // ---- B5: gW1[d][c] += sum_r x[r][d] dz1[r][c];  gb1[c] += sum_r dz1[r][c] ------------------------
-        if (w1_live) mm_tn(sm + xoff + dq * 4, Dp, sm + L.h1 + c0, sm + L.h1 + c1, LDH, rsplit, nrows, nsplit, gW1);
-        if (tid < HC) {
-            float s0 = 0.f, s1 = 0.f;
-            int r = 0;
-            for (; r + 1 < nrows; r += 2) { s0 += sm[L.h1 + r * LDH + tid]; s1 += sm[L.h1 + (r + 1) * LDH + tid]; }
-            if (r < nrows) s0 += sm[L.h1 + r * LDH + tid];
-            gb1 += s0 + s1;
-        }
-        xb ^= 1;
-    }
-    cp_async_wait_all();
-
-    // ---- write the per-CTA partial gradient (flat checkpoint order, partial stride padded to 4 floats) -----------
-    const int NPs = (o.NP + 3) & ~3;
-    float* gp = a.grad_part + ((int64_t)p * G + bx) * NPs;
-    {   // W2 / Wv2: rows k = 4ty+i, columns (tx%8)*4 + {0..3} and +32
-        float* base = gp + (tx < 8 ? o.W2 : o.Wv2);
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-            float* row = base + (ty * 4 + i) * H + (tx & 7) * 4;
-#pragma unroll
-            for (int j = 0; j < 4; ++j) { row[j] = gW2[i][j]; row[32 + j] = gW2[i][4 + j]; }
-        }
-    }
-    if (tid < HC) {
-        gp[(tid < H ? o.b1 : o.bv1) + (tid & 63)] = gb1;
-        gp[(tid < H ? o.b2 : o.bv2) + (tid & 63)] = gb2;
-    }
-#pragma unroll
-    for (int i = 0; i < MAXHEAD; ++i) {
-        const int item = tid + i * NT;
-        if (item < H * (A2 + 1)) {
-            const int k = item & 63, oo = item >> 6;
-            gp[oo == A2 ? o.Wvo + k : o.Wo + k * A2 + oo] = gHead[i];
-        }
-    }
-    if (tid <= A2) gp[tid == A2 ? o.bvo : o.bo + tid] = gbo;
-    // W1 / Wv1: combine the row-split replicas in fixed order through shared memory (aliases h1/h2)
-    __syncthreads();
-    float* scratch = sm + L.h1;  // nsplit * Dp * HC <= 2 * TM * LDH floats
-    if (w1_live) {
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-            float* row = scratch + (rsplit * Dp + dq * 4 + i) * HC;
-            *reinterpret_cast<float4*>(row + c0) = make_float4(gW1[i][0], gW1[i][1], gW1[i][2], gW1[i][3]);
-            *reinterpret_cast<float4*>(row + c1) = make_float4(gW1[i][4], gW1[i][5], gW1[i][6], gW1[i][7]);
-        }
-    }
-    __syncthreads();
-    for (int i = tid; i < D * HC; i += NT) {
-        const int d = i >> 7, c = i & 127;
-        float s = scratch[i];
-        for (int q = 1; q < nsplit; ++q) s += scratch[q * Dp * HC + i];
-        gp[(c < H ? o.W1 : o.Wv1) + d * H + (c & 63)] = s;
-    }
-    if (tid == 0 && a.stat_part) {
-        double* sp = a.stat_part + ((int64_t)p * G + bx) * DDRL_NSTAT;
-#pragma unroll
-        for (int i = 0; i < DDRL_NSTAT; ++i) sp[i] = st[i];
-    }
-    if (a.tail.theta) {   // fused grad-reduce + clip + Adam (single-GPU SGD loop)
-        sgd_step_tail(a.tail, tail_single_step(a.tail, p), a.grad_part, a.stat_part, p, gridDim.y, bx, G, o.NP, step, D, A, sm + L.h1);
-    }
+__global__ void __launch_bounds__(NT, 1) fcnet_train_cup_kernel(const TrainArgs a, const int32_t* __restrict__ node_id) {
+    constexpr bool CUP = true;
+#include "fcnet_train_body.inc"
 }
 
 // flat theta -> packed shared-memory image (one thread per parameter)
@@ -620,6 +358,47 @@ extern "C" int ddrl_fcnet_pack(const float* theta, int P, int D, int A, float* i
     cudaMemsetAsync(img, 0, (size_t)P * fc_smem(D, A, false).x * sizeof(float), (cudaStream_t)stream);
     fcnet_pack_kernel<<<dim3((NP + 255) / 256, P), 256, 0, (cudaStream_t)stream>>>(theta, D, A, img);
     DDRL_CHECK_LAUNCH("fcnet_pack");
+    return DDRL_OK;
+}
+
+static int set_smem_attr(const void* fn, bool* done, const char* who);
+
+extern "C" int ddrl_ppo_train_step_coupled(const float* theta, const float* img, const int32_t* node_id, const float* obs,
+                                           const float* actions, const float* old_logits, const float* old_logp,
+                                           const float* vf_preds, const float* adv, const float* vtarg, int P, int64_t R,
+                                           int D, int A, int MB, const int32_t* mb_perm, int64_t perm_stride,
+                                           const int32_t* step_ctr, const float* kl_coeff, const ddrl_ppo_hyper* hyper,
+                                           int ctas_per_policy, float* grad_part, double* stat_part, const ddrl_sgd_tail* tail,
+                                           void* stream) {
+    DDRL_REQUIRE(theta && img && node_id && obs && actions && old_logits && old_logp && vf_preds && adv && vtarg && kl_coeff &&
+                     hyper && grad_part && P >= 1 && R >= 1 && MB >= 1 && ctas_per_policy >= 1,
+                 DDRL_E_BADARG, "ppo_train_step_coupled: null pointer or bad P/R/MB/ctas");
+    DDRL_REQUIRE(A == 2, DDRL_E_BADARG, "ppo_train_step_coupled: LegCoupling needs A = 2 (num_outputs == 4), got A=%d", A);
+    DDRL_REQUIRE(P == 1, DDRL_E_BADARG, "ppo_train_step_coupled: the coupled model is one shared policy (P = 1), got P=%d", P);
+    DDRL_REQUIRE(D >= 1 && D <= DDRL_MAX_OBS, DDRL_E_UNSUPPORTED_SHAPE, "ppo_train_step_coupled: unsupported D=%d", D);
+    DDRL_REQUIRE(tail != nullptr, DDRL_E_BADARG, "ppo_train_step_coupled: the fused tail is required (NP + 8 parameters)");
+    DDRL_REQUIRE(tail->theta == theta, DDRL_E_BADARG, "ppo_train_step_coupled: tail->theta must be theta");
+    DDRL_REQUIRE(tail->status != nullptr, DDRL_E_BADARG,
+                 "ppo_train_step_coupled: tail->status is required (it receives DDRL_STATUS_BAD_NODE for a node id outside 0..3)");
+    const int rc = sgd_tail_check(tail, ctas_per_policy * P, "ppo_train_step_coupled");
+    if (rc != DDRL_OK) return rc;
+    DDRL_REQUIRE(tail->nsteps <= 1, DDRL_E_UNSUPPORTED_SHAPE, "ppo_train_step_coupled: nsteps > 1 is not supported by the FP32 kernel");
+    DDRL_REQUIRE(!tail->ll_ws, DDRL_E_BADARG, "ppo_train_step_coupled: the LL tail is not supported with leg coupling");
+    TrainArgs a;
+    a.theta = theta; a.img = img; a.obs = obs; a.actions = actions; a.old_logits = old_logits; a.old_logp = old_logp;
+    a.vf_preds = vf_preds; a.adv = adv; a.vtarg = vtarg; a.ext_dlogits = nullptr; a.ext_dvalue = nullptr;
+    a.R = R; a.D = D; a.A = A; a.MB = MB; a.mb_perm = mb_perm; a.perm_stride = perm_stride; a.step_ctr = step_ctr;
+    a.kl_coeff = kl_coeff; a.hp = *hyper;
+    a.grad_part = grad_part; a.stat_part = stat_part;
+    a.tail = *tail;
+    a.tail.grad_acc = nullptr;
+    const FcSmem L = fc_smem(D, A, false, true);
+    const size_t smem = (size_t)L.total * sizeof(float);
+    DDRL_REQUIRE(smem <= 227 * 1024, DDRL_E_UNSUPPORTED_SHAPE, "ppo_train_step_coupled: shared memory %zu > 227 KB", smem);
+    static bool attr_set = false;
+    if (int rc2 = set_smem_attr((const void*)fcnet_train_cup_kernel, &attr_set, "ppo_train_step_coupled")) return rc2;
+    fcnet_train_cup_kernel<<<dim3(ctas_per_policy, P), NT, smem, (cudaStream_t)stream>>>(a, node_id);
+    DDRL_CHECK_LAUNCH("ppo_train_step_coupled");
     return DDRL_OK;
 }
 

@@ -68,10 +68,12 @@ __host__ __device__ inline TcSmem tc_smem(int D, int A) {
 // That fits KX <= 48 (D <= 46) for A <= 4, and A = 8 for 31 <= D <= 46 (the centralized controller): every published
 // architecture.
 struct Tc2Smem {
-    int X[2], H1[2][2], H2[2][2], DL[2][2], xraw, pf, po, red, bar, total;
+    int X[2], H1[2][2], H2[2][2], DL[2][2], xraw, pf, po, red, bar, nid, cup, total;
     bool dl_in_w1, po_in_w1;
 };
-__host__ __device__ inline Tc2Smem tc2_smem(int D, int A) {
+// cup: the leg-coupled step (SharedDecentralLegID) also stages the node ids of the tile ([128] int32), the rows' coupling
+// table gradients ([128][2]) and the coupling table ([4][2] floats) behind the other regions
+__host__ __device__ inline Tc2Smem tc2_smem(int D, int A, bool cup = false) {
     const int KX = tc_kx(D);
     const TcImg I = tc_img(D, A);
     Tc2Smem s;
@@ -96,6 +98,8 @@ __host__ __device__ inline Tc2Smem tc2_smem(int D, int A) {
     else            { s.po = p + TC_ROWS * A * 4;   p += ((TC_ROWS * (3 * A + 4) * 4) + 15) & ~15; }
     s.red = p;   p += 8 * 24 * 8;    // [8 loss warps][24] doubles: 5 stat sums, 16 head-bias gradient sums
     s.bar = p;   p += 64;            // 2 mbarriers, tmem slot, 2 gradient scales
+    s.nid = s.cup = 0;
+    if (cup) { s.nid = p; p += TC_ROWS * 4 * 3; s.cup = p; p += 32; }      // node ids, then the rows' table gradients [128][2]
     s.total = p;
     return s;
 }

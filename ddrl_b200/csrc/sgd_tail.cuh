@@ -92,6 +92,9 @@ __device__ __forceinline__ bool sgd_wait_weights(const SgdTail& t, int p, int G,
     return false;
 }
 
+// NX: the last NX of the NP parameters are not FCNet variables (the leg-coupling table of SharedDecentralLegID): clipped and
+// stepped like the rest, never mapped into the packed weight images.
+template <int NX = 0>
 __device__ __forceinline__ bool sgd_step_tail(const SgdTail& t, const TailStep& ts, const float* __restrict__ grad_part,
                                               const double* __restrict__ stat_part, int p, int P, int bx, int G, int NP,
                                               int step, int D, int A, float* smem, long long* dbg = nullptr, int npart = 0,
@@ -320,6 +323,7 @@ __device__ __forceinline__ bool sgd_step_tail(const SgdTail& t, const TailStep& 
         t.v[k] = vj;
         const float tnew = (pf ? th_pf : t.theta[k]) - (mj * alpha) / (sqrtf(vj) + t.eps);
         t.theta[k] = tnew;
+        if (NX > 0 && j >= NP - NX) continue;      // (compile-time: no test in the plain FCNet step)
         if (t.fcnet_img) {
             const FcSmem L = fc_smem(D, A, false);
             const FcOffsets o = fc_offsets(D, A);

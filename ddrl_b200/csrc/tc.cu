@@ -744,6 +744,43 @@ extern "C" int ddrl_ppo_train_step_tc(const void* tc_img_p, const float* obs, co
     return DDRL_OK;
 }
 
+extern "C" int ddrl_ppo_train_step_tc_coupled(const void* tc_img_p, const float* theta, const int32_t* node_id, const float* obs,
+                                              const float* actions, const float* old_logits, const float* old_logp,
+                                              const float* vf_preds, const float* adv, const float* vtarg, int P, int64_t R,
+                                              int D, int A, int MB, const int32_t* mb_perm, int64_t perm_stride,
+                                              const int32_t* step_ctr, const float* kl_coeff, const ddrl_ppo_hyper* hyper,
+                                              int ctas_per_policy, float* grad_part, double* stat_part, int* status,
+                                              const ddrl_sgd_tail* tail, void* stream) {
+    DDRL_REQUIRE(tc_img_p && theta && node_id && obs && actions && old_logits && old_logp && vf_preds && adv && vtarg && kl_coeff &&
+                     hyper && grad_part && P >= 1 && R >= 1 && MB >= 1 && ctas_per_policy >= 1,
+                 DDRL_E_BADARG, "ppo_train_step_tc_coupled: null pointer or bad P/R/MB/ctas");
+    DDRL_REQUIRE(A == 2, DDRL_E_BADARG, "ppo_train_step_tc_coupled: LegCoupling needs A = 2 (num_outputs == 4), got A=%d", A);
+    DDRL_REQUIRE(P == 1, DDRL_E_BADARG, "ppo_train_step_tc_coupled: the coupled model is one shared policy (P = 1), got P=%d", P);
+    DDRL_REQUIRE(D == 19 || D == 20, DDRL_E_UNSUPPORTED_SHAPE,
+                 "ppo_train_step_tc_coupled: instantiated for SharedDecentralLegID (D = 19 or 20), got D=%d", D);
+    DDRL_REQUIRE(tail != nullptr, DDRL_E_BADARG, "ppo_train_step_tc_coupled: the fused tail is required (NP + 8 parameters)");
+    DDRL_REQUIRE(tail->theta == theta, DDRL_E_BADARG, "ppo_train_step_tc_coupled: tail->theta must be theta");
+    DDRL_REQUIRE(status != nullptr, DDRL_E_BADARG,
+                 "ppo_train_step_tc_coupled: status is required (it receives DDRL_STATUS_BAD_NODE for a node id outside 0..3)");
+    DDRL_REQUIRE(!tail->ll_ws, DDRL_E_BADARG, "ppo_train_step_tc_coupled: the LL tail is not supported with leg coupling");
+    DDRL_REQUIRE(g_tc_variant != 1, DDRL_E_BADARG,
+                 "ppo_train_step_tc_coupled: only the ping-pong kernel has a coupled instantiation (ddrl_tc_set_variant(1) is set)");
+    DDRL_REQUIRE((reinterpret_cast<uintptr_t>(tc_img_p) & 15) == 0, DDRL_E_BADARG,
+                 "ppo_train_step_tc_coupled: the weight image must be 16-byte aligned (TMA bulk copies)");
+    const int rc0 = sgd_tail_check(tail, ctas_per_policy * P, "ppo_train_step_tc_coupled");
+    if (rc0 != DDRL_OK) return rc0;
+    TcTrainArgs a = {};
+    a.img = (const unsigned char*)tc_img_p; a.obs = obs; a.actions = actions; a.old_logits = old_logits;
+    a.old_logp = old_logp; a.vf_preds = vf_preds; a.adv = adv; a.vtarg = vtarg; a.R = R; a.D = D; a.A = A; a.MB = MB;
+    a.mb_perm = mb_perm; a.perm_stride = perm_stride; a.step_ctr = step_ctr; a.kl_coeff = kl_coeff; a.hp = *hyper;
+    a.grad_part = grad_part; a.stat_part = stat_part; a.status = status; a.dbg_clock = nullptr;
+    a.tail = *tail;
+    const int rc = launch_tc2_cup(a, node_id, theta, P, ctas_per_policy, (cudaStream_t)stream);
+    if (rc != DDRL_OK) return rc;
+    DDRL_CHECK_LAUNCH("ppo_train_step_tc_coupled");
+    return DDRL_OK;
+}
+
 extern "C" int ddrl_fcnet_forward_tc(const void* tc_img_p, const float* obs, const double* norm, float clip, int P, int64_t R,
                                      int D, int A, float* obs_out, float* logits, float* value, const float* eps, float* action,
                                      float* logp, int* status, void* stream) {

@@ -169,1002 +169,29 @@ __device__ __forceinline__ long long t2_gtime() {
 // architectures, policies.ARCHITECTURES; DT = 0 reads a.D).  Every shared-memory offset, image offset and flat-parameter offset
 // is a function of (D, A): with D in a register ptxas — at the kernel's 96-register cap — re-derived them from D at nearly
 // every use (~20 integer instructions per staged element in the x split and the write-out); as constants they cost nothing.
+// CUP = true: the leg-coupled policy of SharedDecentralLegID (models/coupling_net_glorot_uniform_init.py:11-30,135; A = 2,
+// no clusters, no LL tail, fused tail required).  The mean logits are scaled by the trainable table c[node][i] before the
+// loss, the loss gradient of the mean logits by the same factor before it enters the backward, and the table's own gradient
+// sum_r dlogits[r][i] * pre[r][i] (per node) goes to flat indices [NP, NP + 8) of the partial: the step's parameter vector
+// is [NP + 8] (FCNet variables, then leg_coupling [4][2]), and the fused tail clips and steps all of it.
+//   node_id  [P][R] int32 in the batch's row order (rows of a tile are staged in shared memory with the loss inputs)
+//   cup_theta  the flat parameter vector [P][NP + 8]: the table is read from it at the start of every step (after barrier C)
 template <int A, bool FWD, bool LL, int DT, bool DBG>
 __global__ void __launch_bounds__(T2_NT, 1) fcnet_train_tc2_kernel(const __grid_constant__ TcTrainArgs a) {
-    constexpr int A2 = 2 * A;
-    T2_STAMP(0);
-    extern __shared__ __align__(1024) unsigned char sm[];
-    const int p = blockIdx.y, G = gridDim.x, bx = blockIdx.x;
-    const int D = DT > 0 ? DT : a.D, KX = tc_kx(D);
-    const TcImg I = tc_img(D, A);
-    const Tc2Smem S = tc2_smem(D, A);
-    const FcOffsets o = fc_offsets(D, A);
-    // [branch b][hi | lo h] buffers are equally spaced: offsets by arithmetic, not by indexing the layout structs with a
-    // run-time b (that put the structs into local memory: an LDL in front of every epilogue call and every MMA batch)
-    constexpr int BUFB = TC_ROWS * 64 * 2, DLB = TC_ROWS * TC_NO * 2, W2B = 64 * 64 * 2, WOB = TC_NO * 64 * 2;
-    const int W1B = 64 * KX * 2, sH1_0 = S.H1[0][0], sH2_0 = S.H2[0][0], sDL_0 = S.DL[0][0], iW1_0 = I.W1[0][0],
-              iW2_0 = I.W2[0][0], iWoT_0 = I.WoT[0][0];
-    auto sH1 = [&](int b, int h) { return sH1_0 + (2 * b + h) * BUFB; };
-    auto sH2 = [&](int b, int h) { return sH2_0 + (2 * b + h) * BUFB; };
-    auto sDL = [&](int b, int h) { return sDL_0 + (2 * b + h) * DLB; };
-    auto iW1 = [&](int b, int h) { return iW1_0 + (2 * b + h) * W1B; };
-    auto iW2 = [&](int b, int h) { return iW2_0 + (2 * b + h) * W2B; };
-    auto iWoT = [&](int b, int h) { return iWoT_0 + (2 * b + h) * WOB; };
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, q = warp & 3, cq = warp >> 2, row = q * 32 + lane;
-    uint64_t* mbar = reinterpret_cast<uint64_t*>(sm + S.bar);          // [2]: one per branch
-    uint32_t* tslot = reinterpret_cast<uint32_t*>(sm + S.bar + 16);
-    float* sgs = reinterpret_cast<float*>(sm + S.bar + 24);             // [2]: per-branch gradient scale
-    const uint32_t sbase = umma::smem_u32(sm);
+    constexpr bool CUP = false;
+    const int32_t* const node_id = nullptr;
+    const float* const cup_theta = nullptr;
+#include "tc2_step_body.inc"
+}
 
-    // ---- once per launch: TMEM, mbarriers, launch-wide state -------------------------------------------------------------
-    if (warp == 0) umma::tmem_alloc(tslot, T2_TMEM_COLS);
-    if (tid == 0) {      // every MMA warp commits; [4] (byte 32): TMA bulk copies of the LL tail; [5] (byte 40): weight image
-        umma::mbar_init(mbar, T2_NMMA); umma::mbar_init(mbar + 1, T2_NMMA); umma::mbar_init(mbar + 4, 1); umma::mbar_init(mbar + 5, 1); umma::mbar_init(mbar + 6, 1); umma::fence_mbar_init();
-    }
-    umma::fence_before_sync();
-    __syncthreads();
-    umma::fence_after_sync();
-    const uint32_t tmem = *tslot;
-    const uint32_t tlane = (uint32_t)(q * 32) << 16;
-    uint32_t ph0 = 0, ph1 = 0;
-    unsigned int ll_phase = 0, img_phase = 0;      // parities of the TMA mbarriers: [4] LL tail, [5] weight image
-    bool ok = true;
-    int ovf = 0;   // bit mask of fp16 overflows: 2 = x, 8 = dl, 16 = dz2, 32 = dz1
-    const float klc = a.kl_coeff[p];
-    const int ch0 = (D >> 3) & ~1;     // 16-column window of X that contains the constant-1 pad column D
-    const bool gw1_split = KX <= 32;   // two product-split accumulators of KX columns per branch fit TMEM only then
-    const int NPs = (o.NP + 3) & ~3;
-    // Thread-block clusters (launch attribute; cluster = cs consecutive CTAs of one policy): the per-CTA partial gradient
-    // goes to shared memory, the cluster adds its cs partials over distributed shared memory (CTA r owns 1/cs of the
-    // vector) and only ONE partial per cluster reaches L2 — the 148 x 45 KB write / drain / re-read per step was ~9 us.
-    const int cs = LL ? 1 : (int)umma::cluster_nctarank(), crank = LL ? 0 : (int)umma::cluster_ctarank();
-    const int ncl = G / cs, cid = bx / cs;                 // clusters per policy, this CTA's cluster
-    float* stg = reinterpret_cast<float*>(sm + sH1(0, 0));   // [NPs] staging of the partial (H1 is free after the main loop)
-    // Without clusters the partial is staged as well — in H2 (64 KB >= NPs floats; both dZ2 are dead once the last B3 has
-    // completed, so gW2 / gb2 / gWh can go there while B5 still runs) — and leaves the SM as ONE coalesced copy of full
-    // 128-byte lines.  Written straight from the TMEM read-out (lane = matrix row) the partial reached L2 as ~3000 16-byte
-    // partial-sector requests per CTA, and the drain of those requests — not their bytes — set the length of the write-out,
-    // of barrier A behind it and of the slice reduce that re-reads them.
-    float* gpart = a.grad_part + ((int64_t)p * G + bx) * NPs;      // this CTA's partial in global memory
-    float* gp = LL ? gpart : (cs > 1 ? stg : reinterpret_cast<float*>(sm + sH2(0, 0)));
-    const bool stage_copy = !FWD && !LL && cs == 1;
-    bool staged = false;                                           // this step's partial sits in shared memory (CTA-uniform)
-    const bool acc_mode = stage_copy && a.tail.theta != nullptr && a.tail.grad_acc != nullptr;
-    // staged partial -> global memory, float4 range [i0, i1), full 128-byte lines; `nthr` threads (t0 = 0 .. nthr-1) take part
-    // The staged vector is ROTATED: flat index o.W2 sits at the start of the staging buffers (rot() below), so that the blocks
-    // which are complete first (gW2 / gb2 of the policy branch) land in the part of the buffers that is dead first.
-    auto copy_out = [&](int i0, int i1, int t0, int nthr) {
-        const int w2a = o.W2 >> 2, v2a = o.Wv2 >> 2, n4 = NPs >> 2;      // the two swizzled 64 x 64 blocks: 1024 float4 each
-        const uint32_t s4 = t2_launder(umma::smem_u32(gp)), s5 = t2_launder(sbase);      // the two staged halves (see `half1`)
-        // a.tail.grad_acc: ADD into the policy's one accumulation vector at L2 (sgd_tail.cuh) instead of storing this CTA's own
-        // partial.  Every CTA starts at a different place of the range so that the G CTAs of a policy do not walk the same
-        // addresses (= the same L2 slices' atomic units) in lockstep.
-        float4* g4 = reinterpret_cast<float4*>(acc_mode ? a.tail.grad_acc + (int64_t)p * NPs : gpart);
-        const int span = i1 - i0, shift = acc_mode ? (int)(((int64_t)span * bx) / G) : 0;
-#pragma unroll 2
-        for (int k = t0; k < span; k += nthr) {
-            int i = i0 + k + shift;
-            if (i >= i1) i -= span;
-            const unsigned int r0 = (unsigned int)(i - w2a), r1 = (unsigned int)(i - v2a);
-            const int sw = r0 < 1024u ? (int)((r0 >> 4) & 7u) : r1 < 1024u ? (int)((r1 >> 4) & 7u) : 0;
-            const int si = i >= w2a ? i - w2a : i + (n4 - w2a);
-            const uint32_t so = 16u * (uint32_t)(si ^ sw);      // block starts are multiples of 16 float4: the XOR stays inside the row
-            const float4 u = t2_lds4(s4 + so), w = t2_lds4(s5 + so);
-            if (acc_mode)
-                asm volatile("red.relaxed.gpu.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(g4 + i), "f"(u.x + w.x), "f"(u.y + w.y),
-                             "f"(u.z + w.z), "f"(u.w + w.w) : "memory");
-            else
-                g4[i] = make_float4(u.x + w.x, u.y + w.y, u.z + w.z, u.w + w.w);
-        }
-    };
-
-    const bool has_tail = a.tail.theta != nullptr;
-    // LL tail (sgd_tail.cuh): partial gradients and updated weights travel between CTAs as self-validating words
-    constexpr bool ll = LL;      // the launcher picks the instantiation: fused tail, ll_ws given, no clusters, slice <= CTA
-    const int LLW = ll_part_words(o.NP);
-    unsigned long long* llp = a.tail.ll_ws + ((int64_t)p * G + bx) * LLW;      // used only if LL
-    const int nsteps = (has_tail && a.tail.nsteps > 1) ? a.tail.nsteps : 1;   // consecutive SGD steps of this launch
-    const int step0 = a.step_ctr ? *a.step_ctr : 0;
-    TailStep ts;
-    ts.round = 0; ts.last = false; ts.nsteps = nsteps; ts.b1p = 0.f; ts.b2p = 0.f; ts.seq = 0u; ts.epoch = 0u;
-    if (has_tail) {
-        ts.b1p = __ldcg(a.tail.beta_pow + p * 2);
-        ts.b2p = __ldcg(a.tail.beta_pow + p * 2 + 1);
-        ts.seq = (a.tail.world > 1) ? *a.tail.seq : 0u;
-        ts.epoch = __ldcg(a.tail.barrier_ws + 4 * gridDim.y + 1);
-    }
-
-    const float* obs_p = a.obs + (int64_t)p * a.R * D;
-    float* xraw = reinterpret_cast<float*>(sm + S.xraw);
-    float* pf = reinterpret_cast<float*>(sm + S.pf);
-    const float* b1c = reinterpret_cast<const float*>(sm + I.b1c);
-    const float* b2c = reinterpret_cast<const float*>(sm + I.b2c);
-    const float* sbo = reinterpret_cast<const float*>(sm + I.bo);
-    const float* sbvo = reinterpret_cast<const float*>(sm + I.bvo);
-
-    // contiguous run of `cnt` floats global -> shared: 16-byte cp.async when both ends and the length allow it (every full
-    // tile of the shuffled batch does: a quarter of the LDGSTS instructions and of their address arithmetic)
-    auto cp_run = [&](float* dst, const float* src, int cnt) {
-        if ((((uint32_t)reinterpret_cast<uintptr_t>(src) | umma::smem_u32(dst) | ((uint32_t)cnt << 2)) & 15u) == 0u) {
-#pragma unroll 1
-            for (int i = tid; i < (cnt >> 2); i += TC_NT)
-                tc_cp16(reinterpret_cast<unsigned char*>(dst + 4 * i), reinterpret_cast<const unsigned char*>(src + 4 * i));
-        } else {
-#pragma unroll 1
-            for (int i = tid; i < cnt; i += TC_NT) tc_cp4(dst + i, src + i);
-        }
-    };
-    auto prefetch_x = [&](int64_t r0, int n) { cp_run(xraw, obs_p + r0 * D, n * D); };
-    auto prefetch_loss = [&](int64_t r0, int n) {
-        const int64_t g0 = (int64_t)p * a.R + r0;
-        float* pa = pf;
-        float* po = reinterpret_cast<float*>(sm + S.po);
-        float* ps = pa + TC_ROWS * A + (S.po_in_w1 ? 0 : TC_ROWS * A2);
-        const float* first_in = FWD ? a.eps : a.actions;      // inference: the only per-row input besides x is the noise
-        if (first_in) cp_run(pa, first_in + g0 * A, n * A);
-        if (FWD) return;
-        if (!S.po_in_w1) cp_run(po, a.old_logits + g0 * A2, n * A2);
-        cp_run(ps, a.old_logp + g0, n);
-        cp_run(ps + TC_ROWS, a.vf_preds + g0, n);
-        cp_run(ps + 2 * TC_ROWS, a.adv + g0, n);
-        cp_run(ps + 3 * TC_ROWS, a.vtarg + g0, n);
-    };
-
-    auto prefetch_po = [&](int64_t r0, int n) {   // old logits into the W1 region: only once F1 has consumed W1 (po_in_w1)
-        const int64_t g0 = (int64_t)p * a.R + r0;
-        float* po = reinterpret_cast<float*>(sm + S.po);
-        cp_run(po, a.old_logits + g0 * A2, n * A2);
-        asm volatile("cp.async.commit_group;\n" ::);
-    };
-    bool prefetched = false;   // the first tile's inputs of this step were already requested behind the previous step's tail
-
-#pragma unroll 1
-    for (int s = 0; s < nsteps; ++s) {
-    const unsigned int tag = ts.epoch + (unsigned int)s + 1u;      // LL tag of THIS step's partials / weights
-    // (the weights of this step are fetched inside the tile loop, AFTER the first tile's x has been split: the split does not
-    // depend on them and runs while the other CTAs of the policy still finish their Adam slices)
-    T2_STAMP(35);
-    T2_GSTAMP(0);
-    const int step = step0 + s;
-    const int mb = a.mb_perm ? a.mb_perm[(int64_t)p * a.perm_stride + step] : step;
-    const int64_t mb0 = (int64_t)mb * a.MB;
-    if (mb0 >= 0) T2_STAMP(36);
-    bool first = true;
-    staged = false;
-    // loss warps: 0-3 policy part (s0 = -surr, s1 = KL, s2 = entropy), 4-7 value part (s0 = vf, s1..4 = R, R^2, R-v, (R-v)^2)
-    double st[5];
-#pragma unroll
-    for (int i = 0; i < 5; ++i) st[i] = 0.0;
-    // head bias gradients: policy threads sum_r dl[r][o]; value threads use gbh[0].  Wide heads (A = 8) keep the sums per
-    // warp in shared memory instead (16 more live registers made that instantiation spill)
-    constexpr bool GBH_SMEM = A > 4;
-    float gbh[GBH_SMEM ? 1 : A2];
-#pragma unroll
-    for (int i = 0; i < (GBH_SMEM ? 1 : A2); ++i) gbh[i] = 0.f;
-    if (GBH_SMEM && warp < 8 && lane < 16) reinterpret_cast<double*>(sm + S.red)[warp * 24 + 8 + lane] = 0.0;   // read behind later barriers
-    const int64_t mb1 = min(mb0 + a.MB, a.R);
-    const int rpc = (((a.MB + G - 1) / G) + 7) & ~7;
-    const int64_t cr0 = min(mb0 + (int64_t)bx * rpc, mb1), cr1 = min(cr0 + rpc, mb1);
-    do {   // single exit towards the fused tail (one inlined copy of it)
-    if (cr1 <= cr0) {   // no rows: zero partial, no tensor work (still takes part in the fused tail)
-        asm volatile("cp.async.wait_group 0;\n" ::: "memory");
-        if (FWD) break;      // inference: a CTA without rows has nothing to write (there is no partial-gradient buffer)
-        if constexpr (LL) {
-            for (int i = tid; i < (LLW >> 1); i += T2_NT) ll_st2(llp + 2 * i, 0u, 0u, tag);
-        } else {
-            float* z = stage_copy ? gpart : gp;      // (already coalesced: straight to global memory)
-            if (!acc_mode)                           // (accumulation vector: nothing to add)
-                for (int i = tid; i < NPs; i += T2_NT) z[i] = 0.f;
-            if (tid < DDRL_NSTAT && a.stat_part) a.stat_part[((int64_t)p * G + bx) * DDRL_NSTAT + tid] = 0.0;
-        }
-        break;
-    }
-    staged = stage_copy;
-
-    // ---- this step's first tile: inputs ---------------------------------------------------------------------------------
-    if (warp < T2_MMA_WARP && !prefetched) {
-        const int n0 = (int)min((int64_t)TC_ROWS, cr1 - cr0);
-        prefetch_x(cr0, n0);
-        prefetch_loss(cr0, n0);
-        asm volatile("cp.async.commit_group;\n" ::);
-    }
-    T2_STAMP(1);
-
-    auto wait_b = [&](int b) {
-        if (b == 0) { ok = umma::mbar_wait(mbar, ph0) && ok; ph0 ^= 1; }
-        else        { ok = umma::mbar_wait(mbar + 1, ph1) && ok; ph1 ^= 1; }
-        umma::fence_after_sync();
-    };
-    // epilogue warps -> MMA warp hand-off: generic smem writes -> async proxy, TMEM reads retired, then a barrier that the
-    // MMA warp joins (it issues right behind it).  The MMA warp is a warp of its own ON PURPOSE: when the issuing lane
-    // shared a warp with lanes spinning in mbarrier.try_wait, the suspended warp delayed every issue by 0.5-2 us.
-    // Two named barriers (3 and 5) alternate from hand-off to hand-off.  The epilogue warps only ARRIVE (bar.arrive: they do
-    // not wait for their slowest sibling, they go straight on to the other branch's mbarrier); the MMA warps bar.sync and issue.
-    // A warp can run at most one hand-off ahead of the slowest one: the mbarrier it waits for next belongs to MMAs that are
-    // issued only after the previous hand-off has completed — so hand-off k + 2 (same barrier id) never starts before k is over.
-    // publish_sync (everybody waits) is kept where the epilogue warps do need each other: behind the x split / weight image and
-    // behind the loss (the branch gradient scales sgs[] are read by all warps afterwards).
-    unsigned int hand = 0;      // parity of the next hand-off (both roles toggle it in lockstep)
-    auto publish = [&]() {
-        umma::fence_async_smem();
-        umma::fence_before_sync();
-        if (hand) asm volatile("bar.arrive 5, %0;" ::"n"(T2_NT) : "memory");
-        else      asm volatile("bar.arrive 3, %0;" ::"n"(T2_NT) : "memory");
-        hand ^= 1u;
-    };
-    auto publish_sync = [&]() {
-        umma::fence_async_smem();
-        umma::fence_before_sync();
-        if (hand) asm volatile("bar.sync 5, %0;" ::"n"(T2_NT) : "memory");
-        else      asm volatile("bar.sync 3, %0;" ::"n"(T2_NT) : "memory");
-        hand ^= 1u;
-    };
-    auto mma_turn = [&]() {    // MMA warp: wait for the epilogue warps' hand-off
-        if (hand) asm volatile("bar.sync 5, %0;" ::"n"(T2_NT) : "memory");
-        else      asm volatile("bar.sync 3, %0;" ::"n"(T2_NT) : "memory");
-        hand ^= 1u;
-        umma::fence_after_sync();
-    };
-    auto epi_sync = [&]() { asm volatile("bar.sync 4, %0;" ::"n"(TC_NT) : "memory"); };   // the 16 epilogue warps only
-    // head outputs of branch b: the three product accumulators added up (whole warps: .sync.aligned loads)
-    auto load_heads = [&](int b, float (&out)[16]) {
-        umma::tmem_ld16(tmem + tlane + T2_HOUT + 16 * b, out);
-        if constexpr (A2 <= 8) {
-            uint32_t e0[8], e1[8];
-            umma::tmem_ld8_nowait(tmem + tlane + T2_DACC + 64 * b, e0);
-            umma::tmem_ld8_nowait(tmem + tlane + T2_DACC + 64 * b + 16, e1);
-            umma::tmem_ld_wait();
-#pragma unroll
-            for (int i = 0; i < 8; ++i) out[i] += __uint_as_float(e0[i]) + __uint_as_float(e1[i]);
-        } else {
-            float e[16];
-            umma::tmem_ld16(tmem + tlane + T2_DACC + 64 * b, e);
-#pragma unroll
-            for (int i = 0; i < 16; ++i) out[i] += e[i];
-            umma::tmem_ld16(tmem + tlane + T2_DACC + 64 * b + 16, e);
-#pragma unroll
-            for (int i = 0; i < 16; ++i) out[i] += e[i];
-        }
-    };
-
-    // ---- write-out pieces: TMEM accumulators (M = 64: row m lives in lane 32*(m/16) + m%16) -> flat partial, x 1/minibatch ----
-    const float inv = a.hp.inv_global_mb;
-    // LL tail: M = 64 accumulators (lanes 0-15 of every quadrant hold rows 16 q ..).  Otherwise the weight-gradient
-    // accumulators are M = 128 with the hi | lo halves of the A operand stacked (tc_gemm_stack_u): lane = row, rows 64-127
-    // (quadrants 2, 3) carry the lo-half products of parameter row m = row - 64.  The two halves are staged in TWO
-    // flat-indexed buffers — half 0 where the partial has always been staged, half 1 at the start of shared memory (the
-    // weight image: dead once the last tile's B4 has completed, reloaded by the next step, and always longer than the
-    // flat vector) — and added by the copy-out, so no thread waits for another one's store.
-    const int m = LL ? 16 * q + lane : (32 * q + lane) & 63;
-    const bool mine = LL ? lane < 16 : true;
-    const bool half1 = !LL && q >= 2;
-    // gW2_b, gb2_b, gWh_b are final once B3(b) / B1 have completed, i.e. BEFORE the last B5: they are written while B5 runs.
-    // (Not with clusters: the staging buffer of the partial lives in H1, which B5 still reads.)
-    const bool early_out = cs == 1;
-    uint32_t gps = 0;      // shared::cta address of the staged partial (laundered right before each write-out piece)
-    auto put1 = [&](int idx, float v) {
-        if constexpr (LL) ll_st1(llp + idx, __float_as_uint(v), tag);
-        else t2_sts(gps + 4u * (uint32_t)idx, v);
-    };
-    auto put4 = [&](int idx, float x0, float x1, float x2, float x3) {      // idx % 4 == 0
-        if constexpr (LL) {
-            ll_st2(llp + idx, __float_as_uint(x0), __float_as_uint(x1), tag);
-            ll_st2(llp + idx + 2, __float_as_uint(x2), __float_as_uint(x3), tag);
-        } else {
-            t2_sts4(gps + 4u * (uint32_t)idx, x0, x1, x2, x3);
-        }
-    };
-    auto write_w2_heads = [&](int b) {
-        const float sgb = sgs[b];
-        const float inv_gw2 = inv / (TC_SH * sgb), inv_gw1 = inv / (sgb * TC_SX), inv_gwh = inv_gw2;
-        {   // gW2_b: this warp's 16 columns
-            uint32_t r0[8], r1[8];
-            umma::tmem_ld8_nowait(tmem + tlane + T2_GW2 + 64 * b + 16 * cq, r0);
-            umma::tmem_ld8_nowait(tmem + tlane + T2_GW2 + 64 * b + 16 * cq + 8, r1);
-            umma::tmem_ld_wait();
-            if (mine) {
-                // staged copy: the 16 float4 of row m are XOR-swizzled by (m & 7) so that the 16 lanes (16 rows, 256 bytes
-                // apart) hit different banks; the copy-out undoes it
-                const int rowb = (b ? o.Wv2 : o.W2) + m * 64, c4 = 4 * cq, sw = stage_copy ? (m & 7) : 0;
-                put4(rowb + 4 * ((c4 + 0) ^ sw), __uint_as_float(r0[0]) * inv_gw2, __uint_as_float(r0[1]) * inv_gw2,
-                     __uint_as_float(r0[2]) * inv_gw2, __uint_as_float(r0[3]) * inv_gw2);
-                put4(rowb + 4 * ((c4 + 1) ^ sw), __uint_as_float(r0[4]) * inv_gw2, __uint_as_float(r0[5]) * inv_gw2,
-                     __uint_as_float(r0[6]) * inv_gw2, __uint_as_float(r0[7]) * inv_gw2);
-                put4(rowb + 4 * ((c4 + 2) ^ sw), __uint_as_float(r1[0]) * inv_gw2, __uint_as_float(r1[1]) * inv_gw2,
-                     __uint_as_float(r1[2]) * inv_gw2, __uint_as_float(r1[3]) * inv_gw2);
-                put4(rowb + 4 * ((c4 + 3) ^ sw), __uint_as_float(r1[4]) * inv_gw2, __uint_as_float(r1[5]) * inv_gw2,
-                     __uint_as_float(r1[6]) * inv_gw2, __uint_as_float(r1[7]) * inv_gw2);
-            }
-        }
-        if (cq == 2) {                                   // gb2_b: column of the constant-1 pad inside its 16-wide window
-            float v[8];
-            umma::tmem_ld8(tmem + tlane + T2_GB2 + 16 * b + (((D - 8 * ch0) >> 3) << 3), v);
-            const int jsel = (D - 8 * ch0) & 7;
-            const float g = jsel == 0 ? v[0] : jsel == 1 ? v[1] : jsel == 2 ? v[2] : jsel == 3 ? v[3] : jsel == 4 ? v[4]
-                          : jsel == 5 ? v[5] : jsel == 6 ? v[6] : v[7];
-            if (mine) put1((b ? o.bv2 : o.b2) + m, g * inv_gw1);
-        }
-        if (cq == 3) {                                   // gWh_b[k = m][o]
-            float w[16], w2[16];
-            umma::tmem_ld16(tmem + tlane + T2_GWH + 16 * (2 * b), w);
-            umma::tmem_ld16(tmem + tlane + T2_GWH + 16 * (2 * b + 1), w2);
-#pragma unroll
-            for (int j = 0; j < 16; ++j) w[j] += w2[j];
-            if (mine) {
-                if (b == 0) {
-#pragma unroll
-                    for (int oo = 0; oo < A2; ++oo) put1(o.Wo + m * A2 + oo, w[oo] * inv_gwh);
-                } else {
-                    put1(o.Wvo + m, w[0] * inv_gwh);
-                }
-            }
-        }
-    };
-    auto write_w1 = [&](int b) {
-        const float inv_gw1 = inv / (sgs[b] * TC_SX);
-#pragma unroll 1
-        for (int c8 = cq; c8 < (KX >> 3); c8 += 4) {   // gW1_b[c = m][d]: 8 input features at a time
-            uint32_t r2[8], r3[8];
-            const uint32_t base0 = tmem + tlane + T2_GW1 + 64 * b + 8 * c8;
-            umma::tmem_ld8_nowait(base0, r2);
-            // second column block: the other products (LL: accumulator [2b + 1]; stacked: the X lo columns) or the same again
-            umma::tmem_ld8_nowait(gw1_split ? base0 + (LL ? 32 : KX) : base0, r3);
-            umma::tmem_ld_wait();
-            if (mine) {
-                // flat order: gW1[d][m] at W1 + 64 d + m, and the bias gradient (column D: the constant-1 input) is row D
-                // of the same block (b1 == W1 + 64 D, fc_offsets) -> one base index, immediate offsets, one predicate each
-                const int i0 = (b ? o.Wv1 : o.W1) + 512 * c8 + m, jmax = D - 8 * c8;
-#pragma unroll
-                for (int j = 0; j < 8; ++j) {
-                    const float g = (__uint_as_float(r2[j]) + (gw1_split ? __uint_as_float(r3[j]) : 0.f)) * inv_gw1;
-                    if (j <= jmax) put1(i0 + 64 * j, g);
-                }
-            }
-        }
-    };
-
-    // ---- stacked accumulators (everything but the LL tail): the write-out belongs to the FOUR MMA-ISSUE WARPS --------------
-    // They are idle between two hand-offs, and warp 16 + k may read TMEM lanes 32 k .. 32 k + 31 = accumulator rows of ALL
-    // columns.  Each block of the partial is staged as soon as its accumulator is complete, in the gaps of the issue schedule:
-    //   slot 1 (behind the B4(1) issue, once B4(0) has completed)   gW2_0, gb2_0
-    //   slot 2 (behind the B5(0) issue, once B4(1) has completed)   gW2_1, gb2_1, gWh_0, gWh_1   -> bar.arrive 6
-    //   slot 3 (behind the B5(1) issue)                             gW1_0 / gb1_0 (B5(0) done), gW1_1 / gb1_1 (B5(1) done)
-    // so that the 16 epilogue warps go from their last epilogue straight to the copy-out of the early 3/4 of the vector
-    // (bar.sync 6) and only gW1_1 — 1/16 of the accumulator data — is read after the last MMA has completed.  Before, the
-    // epilogue warps did all of it behind their last epilogue: 3.0 us from the last hand-off to the barrier-A arrival.
-    // (Copy-out by the MMA warps themselves, inside the slots, was measured too: the slots overran and delayed B5(1).)
-    const int rotn = NPs - o.W2;      // rotated staging index of flat index 0
-    auto rot = [&](int idx) { return idx >= o.W2 ? idx - o.W2 : idx + rotn; };
-    auto stage_w2 = [&](int b) {      // gW2_b: the 64 columns of this quadrant's 32 rows; gb2_b
-        const float sgb = sgs[b];
-        const float inv_gw2 = inv / (TC_SH * sgb), inv_gw1 = inv / (sgb * TC_SX);
-        const int rowb = rot(b ? o.Wv2 : o.W2) + m * 64, sw = stage_copy ? (m & 7) : 0;
-        const uint32_t t0 = tmem + tlane + T2_GW2 + 64 * b;
-#pragma unroll 1
-        for (int c16 = 0; c16 < 4; ++c16) {
-            uint32_t r0[8], r1[8];
-            umma::tmem_ld8_nowait(t0 + 16 * c16, r0);
-            umma::tmem_ld8_nowait(t0 + 16 * c16 + 8, r1);
-            umma::tmem_ld_wait();
-            const int c4 = 4 * c16;
-            put4(rowb + 4 * ((c4 + 0) ^ sw), __uint_as_float(r0[0]) * inv_gw2, __uint_as_float(r0[1]) * inv_gw2,
-                 __uint_as_float(r0[2]) * inv_gw2, __uint_as_float(r0[3]) * inv_gw2);
-            put4(rowb + 4 * ((c4 + 1) ^ sw), __uint_as_float(r0[4]) * inv_gw2, __uint_as_float(r0[5]) * inv_gw2,
-                 __uint_as_float(r0[6]) * inv_gw2, __uint_as_float(r0[7]) * inv_gw2);
-            put4(rowb + 4 * ((c4 + 2) ^ sw), __uint_as_float(r1[0]) * inv_gw2, __uint_as_float(r1[1]) * inv_gw2,
-                 __uint_as_float(r1[2]) * inv_gw2, __uint_as_float(r1[3]) * inv_gw2);
-            put4(rowb + 4 * ((c4 + 3) ^ sw), __uint_as_float(r1[4]) * inv_gw2, __uint_as_float(r1[5]) * inv_gw2,
-                 __uint_as_float(r1[6]) * inv_gw2, __uint_as_float(r1[7]) * inv_gw2);
-        }
-        float v[8];      // gb2_b: column of the constant-1 pad inside its 16-wide window
-        umma::tmem_ld8(tmem + tlane + T2_GB2 + 16 * b + (((D - 8 * ch0) >> 3) << 3), v);
-        const int jsel = (D - 8 * ch0) & 7;
-        const float g = jsel == 0 ? v[0] : jsel == 1 ? v[1] : jsel == 2 ? v[2] : jsel == 3 ? v[3] : jsel == 4 ? v[4]
-                      : jsel == 5 ? v[5] : jsel == 6 ? v[6] : v[7];
-        put1(rot(b ? o.bv2 : o.b2) + m, g * inv_gw1);
-    };
-    auto stage_heads = [&](int b) {   // gWh_b[k = m][o]: the DL hi and DL lo column blocks added
-        const float inv_gwh = inv / (TC_SH * sgs[b]);
-        float w[16], w2[16];
-        umma::tmem_ld16(tmem + tlane + T2_GWH + 32 * b, w);
-        umma::tmem_ld16(tmem + tlane + T2_GWH + 32 * b + 16, w2);
-        if (b == 0) {
-#pragma unroll
-            for (int oo = 0; oo < A2; ++oo) put1(rot(o.Wo) + m * A2 + oo, (w[oo] + w2[oo]) * inv_gwh);
-        } else {
-            put1(rot(o.Wvo) + m, (w[0] + w2[0]) * inv_gwh);
-        }
-    };
-    auto stage_w1 = [&](int b) {      // gW1_b[c = m][d] and gb1_b (column D of X: the constant 1): 8 input features at a time
-        const float inv_gw1 = inv / (sgs[b] * TC_SX);
-#pragma unroll 1
-        for (int c8 = 0; c8 < (KX >> 3); ++c8) {
-            uint32_t r2[8], r3[8];
-            const uint32_t base0 = tmem + tlane + T2_GW1 + 64 * b + 8 * c8;
-            umma::tmem_ld8_nowait(base0, r2);
-            umma::tmem_ld8_nowait(gw1_split ? base0 + KX : base0, r3);      // the X lo column block (2 KX <= 64) or the same again
-            umma::tmem_ld_wait();
-            // flat order: gW1[d][m] at W1 + 64 d + m, bias gradient = row D of the same block (b1 == W1 + 64 D, fc_offsets)
-            const int i0 = rot(b ? o.Wv1 : o.W1) + 512 * c8 + m, jmax = D - 8 * c8;
-#pragma unroll
-            for (int j = 0; j < 8; ++j) {
-                const float g = (__uint_as_float(r2[j]) + (gw1_split ? __uint_as_float(r3[j]) : 0.f)) * inv_gw1;
-                if (j <= jmax) put1(i0 + 64 * j, g);
-            }
-        }
-    };
-    // MMA warps: commit to branch b's mbarrier / wait for the phase committed last (ph0 / ph1 are theirs to keep: they never
-    // call wait_b)
-    auto commit_b = [&](int b) {
-        umma::mma_commit_elect(mbar + b);
-        if (b) ph1 ^= 1u; else ph0 ^= 1u;
-    };
-    auto mma_wait = [&](int b) {
-        ok = umma::mbar_wait(mbar + b, (b ? ph1 : ph0) ^ 1u) && ok;
-        umma::fence_after_sync();
-    };
-
-    // head bias gradients and loss statistics of this CTA: the four per-warp sums of each loss half (redd[], written by the
-    // loss warps of the last tile) -> partial / stat partial.  Threads of warp 0 (half-0 staging); the caller guarantees a
-    // barrier between the loss warps' stores and this.
-    auto bias_stats = [&](int tid) {      // tid: lane of the ONE warp that runs this (a warp of TMEM quadrant 0: half-0 staging)
-        if constexpr (!LL) gps = t2_launder(umma::smem_u32(gp));
-        const double* redd = reinterpret_cast<const double*>(sm + S.red);          // [8 warps][24]
-        auto sum4 = [&](int w0, int i) { return (redd[w0 * 24 + i] + redd[(w0 + 1) * 24 + i]) + (redd[(w0 + 2) * 24 + i] + redd[(w0 + 3) * 24 + i]); };
-        auto rl = [&](int idx) { return LL ? idx : rot(idx); };
-        if (tid < A2) put1(rl(o.bo) + tid, (float)sum4(0, 8 + tid) * inv);
-        if (tid == A2) put1(rl(o.bvo), (float)sum4(4, 8) * inv);
-        if (tid > A2 && o.NP + (tid - A2 - 1) < NPs) put1(rl(o.NP) + (tid - A2 - 1), 0.f);   // padding floats of the partial
-        if constexpr (!LL) {      // these entries have no lo-half rows: zero in the half-1 staging
-            const uint32_t z = t2_launder(sbase);
-            if (tid < A2) t2_sts(z + 4u * (uint32_t)(rot(o.bo) + tid), 0.f);
-            if (tid == A2) t2_sts(z + 4u * (uint32_t)rot(o.bvo), 0.f);
-            if (tid > A2 && o.NP + (tid - A2 - 1) < NPs) t2_sts(z + 4u * (uint32_t)(rot(o.NP) + (tid - A2 - 1)), 0.f);
-        }
-        if (tid < DDRL_NSTAT && (ll || a.stat_part)) {
-            // stat slots (ddrl_b200.h): 0 -surr, 1 KL, 2 vf, 3 entropy, 4 R, 5 R^2, 6 R-v, 7 (R-v)^2
-            const int w0 = (tid == 0 || tid == 1 || tid == 3) ? 0 : 4;
-            const int idx = tid == 0 ? 0 : tid == 1 ? 1 : tid == 3 ? 2 : tid == 2 ? 0 : tid - 3;
-            const double sv = sum4(w0, idx);
-            if constexpr (LL) {
-                const unsigned long long bits = (unsigned long long)__double_as_longlong(sv);
-                ll_st2(llp + NPs + 2 * tid, (unsigned int)bits, (unsigned int)(bits >> 32), tag);
-            } else {
-                a.stat_part[((int64_t)p * G + bx) * DDRL_NSTAT + tid] = sv;
-            }
-        }
-    };
-
-    if (warp >= T2_MMA_WARP) {
-        // ================= MMA-issue warps: one hand-off barrier per batch; lane 0 of each warp issues ITS share of the batch
-        // (shares never split an accumulator) and commits to the branch's mbarrier (expected arrivals = T2_NMMA) ==========
-        // warp-uniform issue (tc_gemm_u): every lane runs the same code on provably uniform values, an elected lane issues
-        const int mw = __shfl_sync(0xffffffffu, warp, 0) - T2_MMA_WARP;
-        const uint32_t tm = __shfl_sync(0xffffffffu, tmem, 0);
-        const uint32_t sbu = __shfl_sync(0xffffffffu, sbase, 0);
-        const uint32_t Xhu = sbu + S.X[0], Xlu = sbu + S.X[1];
-#pragma unroll 1
-        for (int64_t row0 = cr0; row0 < cr1; row0 += TC_ROWS) {
-            const bool acc = !first;
-            mma_turn();      // X split done.  F1: Dacc_b = X * W1b^T   (warp b)
-            {
-                if (mw < 2)
-                    tc_gemm_u(tm + T2_DACC + 64 * mw, Xhu, Xlu, TC_ROWS, false, sbu + iW1(mw, 0), sbu + iW1(mw, 1), 64, false,
-                            128, 64, KX >> 4, false, 3);
-                commit_b(0);
-                commit_b(1);
-            }
-            __syncwarp();
-#pragma unroll 1
-            for (int b = 0; b < 2; ++b) {   // F2: Dacc_b = H1_b * W2b   (warp b)
-                mma_turn();
-                {
-                    if (mw == b)
-                        tc_gemm_u(tm + T2_DACC + 64 * b, (sbu + sH1(b, 0)), (sbu + sH1(b, 1)), TC_ROWS, false, sbu + iW2(b, 0), sbu + iW2(b, 1), 64,
-                                true, 128, 64, 4, false, 3);
-                    commit_b(b);
-                }
-                __syncwarp();
-            }
-#pragma unroll 1
-            for (int b = 0; b < 2; ++b) {   // heads: Hout_b[128][16] = H2_b * WoT_b^T, one product per warp 0-2
-                mma_turn();
-                {
-                    // three independent accumulators (chains of 4 MMAs instead of one of 12; a dependent MMA costs ~100 cycles
-                    // and nothing hides the second head): hi*hi -> Hout_b, hi*lo and lo*hi -> the first 32 columns of Dacc_b,
-                    // which the tanh2(b) epilogue has just consumed and dz2-pre rewrites only after the loss; the readers add them
-                    if (mw < 3)
-                        tc_gemm_mask_u(mw == 0 ? tm + T2_HOUT + 16 * b : tm + T2_DACC + 64 * b + 16 * (mw - 1), (sbu + sH2(b, 0)),
-                                       (sbu + sH2(b, 1)), TC_ROWS, false, sbu + iWoT(b, 0), sbu + iWoT(b, 1), TC_NO, false, 128, TC_NO,
-                                       4, false, 1 << mw);
-                    commit_b(b);
-                }
-                __syncwarp();
-            }
-            if (FWD) continue;      // inference: nothing after the heads
-            mma_turn();      // loss done.  dz2-pre: Dacc_b = DL_b * WoT_b (warp b);  gWh_b (+)= H2_b^T DL_b
-            if constexpr (LL) {      // (M = 64, split by product into two accumulators)
-                const int b = mw & 1;
-                if (mw < 2) {
-                    tc_gemm_u(tm + T2_DACC + 64 * b, (sbu + sDL(b, 0)), (sbu + sDL(b, 1)), TC_ROWS, false, sbu + iWoT(b, 0), sbu + iWoT(b, 1), TC_NO,
-                            true, 128, 64, 1, false, 3);
-                    tc_gemm_mask_u(tm + T2_GWH + 16 * (2 * b), (sbu + sH2(b, 0)), (sbu + sH2(b, 1)), TC_ROWS, true, (sbu + sDL(b, 0)), (sbu + sDL(b, 1)), TC_ROWS, true, 64, 16, 8,
-                                 acc, 1);
-                } else {
-                    tc_gemm_mask_u(tm + T2_GWH + 16 * (2 * b + 1), (sbu + sH2(b, 0)), (sbu + sH2(b, 1)), TC_ROWS, true, (sbu + sDL(b, 0)), (sbu + sDL(b, 1)), TC_ROWS, true, 64,
-                                 16, 8, acc, 6);
-                }
-                commit_b(0);
-                commit_b(1);
-            } else {                 // stacked (tc_gemm_stack_u): [H2_b hi | lo]^T [DL_b hi | lo], 8 MMAs per branch (warps 2, 3)
-                if (mw < 2)
-                    tc_gemm_u(tm + T2_DACC + 64 * mw, (sbu + sDL(mw, 0)), (sbu + sDL(mw, 1)), TC_ROWS, false, sbu + iWoT(mw, 0), sbu + iWoT(mw, 1), TC_NO,
-                            true, 128, 64, 1, false, 3);
-                else
-                    tc_gemm_stack_u(tm + T2_GWH + 32 * (mw - 2), sbu + sH2(mw - 2, 0), TC_ROWS, sbu + sDL(mw - 2, 0), 0u, TC_ROWS, 2 * TC_NO, 8, acc, 1);
-                commit_b(0);
-                commit_b(1);
-            }
-            __syncwarp();
-#pragma unroll 1
-            for (int b = 0; b < 2; ++b) {   // B4: Dacc_b = dZ2_b * W2b^T (warp 0);  gW2_b (+)= H1_b^T dZ2_b (warp 1 / 3);  gb2_b (warp 2)
-                mma_turn();
-                {
-                    if (mw == 0)
-                        tc_gemm_u(tm + T2_DACC + 64 * b, (sbu + sH2(b, 0)), (sbu + sH2(b, 1)), TC_ROWS, false, sbu + iW2(b, 0), sbu + iW2(b, 1), 64,
-                                false, 128, 64, 4, false, 3);
-                    else if (mw == (b ? 3 : 1)) {
-                        if constexpr (LL)
-                            tc_gemm_u(tm + T2_GW2 + 64 * b, (sbu + sH1(b, 0)), (sbu + sH1(b, 1)), TC_ROWS, true, (sbu + sH2(b, 0)), (sbu + sH2(b, 1)), TC_ROWS, true, 64, 64, 8, acc, 3);
-                        else      // [H1_b hi | lo]^T dZ2_b hi, then ... dZ2_b lo: 16 dependent MMAs instead of 24
-                            tc_gemm_stack_u(tm + T2_GW2 + 64 * b, sbu + sH1(b, 0), TC_ROWS, sbu + sH2(b, 0), sbu + sH2(b, 1), TC_ROWS, 64, 8, acc, 2);
-                    } else if (mw == 2) {
-                        if constexpr (LL)
-                            tc_gemm_u(tm + T2_GB2 + 16 * b, (sbu + sH2(b, 0)), (sbu + sH2(b, 1)), TC_ROWS, true, Xhu + ch0 * TC_ROWS * 16, 0, TC_ROWS, true, 64,
-                                    16, 8, acc, 2);
-                        else
-                            tc_gemm_stack_u(tm + T2_GB2 + 16 * b, sbu + sH2(b, 0), TC_ROWS, Xhu + ch0 * TC_ROWS * 16, 0u, TC_ROWS, 16, 8, acc, 1);
-                    }
-                    commit_b(b);
-                }
-                __syncwarp();
-            }
-            const bool wout = !LL && early_out && row0 + TC_ROWS >= cr1;      // last tile: stage the partial between the issues
-            if constexpr (!LL) gps = t2_launder(half1 ? sbu : umma::smem_u32(gp));
-            if (wout) {   // slot 1
-                mma_wait(0);
-                stage_w2(0);
-                umma::fence_before_sync();      // TMEM reads retired before the next hand-off barrier
-            }
-#pragma unroll 1
-            for (int b = 0; b < 2; ++b) {   // B5: gW1_b[c][d] (+)= dZ1_b^T X by product (column D of X = constant 1 -> bias gradient)
-                mma_turn();
-                {
-                    if constexpr (LL) {
-                        if (gw1_split) {
-                            if (mw == 0)
-                                tc_gemm_mask_u(tm + T2_GW1 + 32 * (2 * b), (sbu + sH1(b, 0)), (sbu + sH1(b, 1)), TC_ROWS, true, Xhu, Xlu, TC_ROWS, true, 64, KX, 8,
-                                             acc, 1);
-                            if (mw == 1)
-                                tc_gemm_mask_u(tm + T2_GW1 + 32 * (2 * b + 1), (sbu + sH1(b, 0)), (sbu + sH1(b, 1)), TC_ROWS, true, Xhu, Xlu, TC_ROWS, true, 64, KX,
-                                             8, acc, 6);
-                        } else if (mw == b) {
-                            tc_gemm_u(tm + T2_GW1 + 64 * b, (sbu + sH1(b, 0)), (sbu + sH1(b, 1)), TC_ROWS, true, Xhu, Xlu, TC_ROWS, true, 64, KX, 8, acc, 3);
-                        }
-                    } else if (mw == b) {      // [dZ1_b hi | lo]^T [X hi | lo]: 8 MMAs (2 KX <= 64 columns), else hi and lo in turn: 16
-                        if (gw1_split) tc_gemm_stack_u(tm + T2_GW1 + 64 * b, sbu + sH1(b, 0), TC_ROWS, Xhu, 0u, TC_ROWS, 2 * KX, 8, acc, 1);
-                        else           tc_gemm_stack_u(tm + T2_GW1 + 64 * b, sbu + sH1(b, 0), TC_ROWS, Xhu, Xlu, TC_ROWS, KX, 8, acc, 2);
-                    }
-                    commit_b(b);
-                }
-                __syncwarp();
-                if (wout && b == 0) {   // slot 2
-                    mma_wait(1);
-                    stage_w2(1);
-                    stage_heads(0);
-                    stage_heads(1);
-                    umma::fence_before_sync();
-                    asm volatile("bar.arrive 6, %0;" ::"n"(T2_NT) : "memory");
-                }
-            }
-            first = false;
-        }
-        if constexpr (!FWD && !LL) {   // slot 3 (clusters: everything — their staging buffer, H1, is read by B5)
-            // head-bias gradients and loss statistics: first MMA warp, while B5(1) runs (cold code executed once per step: ~0.6 us
-            // when it sat on the epilogue warps' path to the barrier-A arrival)
-            if (early_out && staged && mw == 0) bias_stats(lane);
-            gps = t2_launder(half1 ? sbu : umma::smem_u32(gp));
-            mma_wait(0);
-            if (!early_out) {
-                mma_wait(1);
-                stage_w2(0); stage_w2(1); stage_heads(0); stage_heads(1);
-            }
-            stage_w1(0);
-            mma_wait(1);
-            stage_w1(1);
-            umma::fence_before_sync();
-        }
-    } else {
-    // ================= epilogue warps ==========================================================================================
-#pragma unroll 1
-    for (int64_t row0 = cr0; row0 < cr1; row0 += TC_ROWS) {
-        const int nrows = (int)min((int64_t)TC_ROWS, cr1 - row0);
-        if (!FWD && !first) { wait_b(0); wait_b(1); }       // previous tile's B5 still reads X and dZ1
-        asm volatile("cp.async.wait_group 0;\n" ::: "memory");
-        epi_sync();
-        T2_STAMP(2);
-        // ---- x: fp32 staging -> fp16 hi/lo chunked [128][KX], constant 1 in column D, zero rows beyond nrows ----------
-        {
-            const int r = tid & (TC_ROWS - 1);
-#pragma unroll 1
-            for (int c8 = tid >> 7; c8 < (KX >> 3); c8 += 4) {
-                float v[8];
-#pragma unroll
-                for (int e = 0; e < 8; ++e) {
-                    const int d = c8 * 8 + e;
-                    float x = (r < nrows && d < D) ? xraw[r * D + d] : 0.f;
-                    if (FWD && r < nrows && d < D) {      // MeanStdFilter normalise (float64 like the FP32 kernel), clip, obs_out
-                        if (a.norm) {
-                            const double* nm = a.norm + (int64_t)p * 2 * D;
-                            x = (float)(((double)x - __ldg(nm + d)) * __ldg(nm + D + d));
-                            if (a.clip > 0.f) x = fminf(fmaxf(x, -a.clip), a.clip);
-                        }
-                        if (a.obs_out) a.obs_out[((int64_t)p * a.R + row0 + r) * D + d] = x;
-                    }
-                    v[e] = (r < nrows) ? (d < D ? x : (d == D ? 1.f : 0.f)) : 0.f;
-                }
-                uint4 hi, lo;
-                ovf |= tc_split8(v, TC_SX, hi, lo) ? 2 : 0;
-                *reinterpret_cast<uint4*>(sm + S.X[0] + (c8 * TC_ROWS + r) * 16) = hi;
-                *reinterpret_cast<uint4*>(sm + S.X[1] + (c8 * TC_ROWS + r) * 16) = lo;
-            }
-        }
-        if (first) {   // this step's weight image: ONE thread waits for the Adam slices and hands the 57-66 KB to the TMA (four
-                       // cp.async.bulk copies completing on an mbarrier); nobody else issues a load or computes an address
-            const uint32_t imb = sbase + S.bar + 40;
-            if (warp == 0) {
-                if (lane == 0) {
-                    // every CTA of this policy must have written its Adam slice of the previous step
-                    if (s > 0 && !sgd_wait_weights(a.tail, p, G, s)) { ok = false; if (a.status) atomicOr(a.status, 64); }
-                    asm volatile("fence.proxy.async;" ::: "memory");      // acquired generic-proxy writes -> async-proxy (TMA) reads
-                    const unsigned char* img_p = a.img + (int64_t)p * I.bytes;
-                    // part A (mbarrier [5]): W1 of both branches and the fp32 block (biases) — all that F1 and the first tanh
-                    // epilogue need; part B ([6]): W2 and WoT, needed from F2 on, land behind F1 and that epilogue
-                    const uint32_t a0 = (uint32_t)iW2_0, f0 = (uint32_t)I.b1c, nb = f0 - a0, hb = ((nb >> 1) + 15u) & ~15u;
-                    mbar_expect_tx(imb, a0 + ((uint32_t)I.bytes - f0));
-                    bulk_g2s(sbase, img_p, a0, imb);
-                    bulk_g2s(sbase + f0, img_p + f0, (uint32_t)I.bytes - f0, imb);
-                    mbar_expect_tx(imb + 8u, nb);
-                    bulk_g2s(sbase + a0, img_p + a0, hb, imb + 8u);
-                    bulk_g2s(sbase + a0 + hb, img_p + a0 + hb, nb - hb, imb + 8u);
-                }
-                __syncwarp();      // lanes 1-31 must not spin on the mbarrier while lane 0 is still polling (divergent try_wait
-            }                      // loops delay the other path by 0.5-2 us)
-            if (!mbar_wait_parity(imb, img_phase)) ok = false;
-            img_phase ^= 1u;
-        }
-        publish_sync();
-        T2_STAMP(3);
-        // ---- F1 (both branches): Dacc_b = X * W1b^T --------------------------------------------------------------
-        // ---- tanh epilogue 1 -> F2: Dacc_b = H1_b * W2b -------------------------------------------------------------
-#pragma unroll 1
-        for (int b = 0; b < 2; ++b) {
-            wait_b(b);
-            T2_STAMP(4 + 3 * b);
-            t2_epi_tanh(tmem + tlane + T2_DACC + 64 * b + 16 * cq, b1c + b * 64 + 16 * cq, 1.f / (TC_SX * TC_SW),
-                        sm + sH1(b, 0), sm + sH1(b, 1), row, cq);
-            T2_STAMP(5 + 3 * b);
-            if (first && b == 0 && !mbar_wait_parity(sbase + S.bar + 48, img_phase ^ 1u)) ok = false;   // W2 / WoT landed (part B)
-            publish();
-            T2_STAMP(6 + 3 * b);
-        }
-        if (!FWD && S.po_in_w1) prefetch_po(row0, nrows);     // both F1 are complete: W1 is dead, its spare part takes the old logits
-        // ---- tanh epilogue 2 -> heads: Hout_b[128][16] = H2_b * WoT_b^T ------------------------------------------------
-#pragma unroll 1
-        for (int b = 0; b < 2; ++b) {
-            wait_b(b);
-            T2_STAMP(10 + 3 * b);
-            t2_epi_tanh(tmem + tlane + T2_DACC + 64 * b + 16 * cq, b2c + b * 64 + 16 * cq, 1.f / (TC_SH * TC_SW),
-                        sm + sH2(b, 0), sm + sH2(b, 1), row, cq);
-            T2_STAMP(11 + 3 * b);
-            if (!FWD && S.po_in_w1 && b == 1) asm volatile("cp.async.wait_group 0;\n" ::: "memory");   // old logits landed (barrier follows)
-            publish();
-            T2_STAMP(12 + 3 * b);
-        }
-        // ---- PPO loss: warps 0-3 policy part, warps 4-7 value part -> DL_b (fp16 hi/lo x branch scale, chunked [128][16]) ----
-        wait_b(0);
-        wait_b(1);
-        T2_STAMP(16);
-        if (FWD) {      // inference epilogue: logits, value, DiagGaussian sample + logp (RLlib tf_action_dist.DiagGaussian)
-            float out[16];
-            if (cq < 2) load_heads(cq, out);
-            if (cq < 2 && row < nrows) {
-                const int64_t gr = (int64_t)p * a.R + row0 + row;
-                if (cq == 0) {
-                    float lg[A2];
-#pragma unroll
-                    for (int oo = 0; oo < A2; ++oo) lg[oo] = fmaf(out[oo], 1.f / (TC_SH * TC_SW), sbo[oo]);
-                    if (a.logits_out) {
-#pragma unroll
-                        for (int oo = 0; oo < A2; ++oo) a.logits_out[gr * A2 + oo] = lg[oo];
-                    }
-                    if (a.eps) {
-                        float sz2 = 0.f, sls = 0.f;
-#pragma unroll
-                        for (int i = 0; i < A; ++i) {
-                            const float mu = lg[i], ls = lg[A + i];
-                            const float sd = expf(ls);
-                            const float act = mu + sd * pf[row * A + i];
-                            const float z = (act - mu) / sd;
-                            sz2 = fmaf(z, z, sz2);
-                            sls += ls;
-                            a.action_out[gr * A + i] = act;
-                        }
-                        a.logp_out[gr] = -0.5f * sz2 - 0.5f * kLog2Pi * (float)A - sls;
-                    }
-                } else if (a.value_out) {
-                    a.value_out[gr] = fmaf(out[0], 1.f / (TC_SH * TC_SW), sbvo[0]);
-                }
-            }
-            epi_sync();      // every reader of this tile's staged noise is done; H2[1] (heads consumed) takes the next x
-            const int64_t nxt = row0 + TC_ROWS;
-            if (nxt < cr1) {
-                const int nn = (int)min((int64_t)TC_ROWS, cr1 - nxt);
-                prefetch_x(nxt, nn);
-                prefetch_loss(nxt, nn);
-            }
-            asm volatile("cp.async.commit_group;\n" ::);
-            continue;
-        }
-        if (cq < 2) {
-            const int b = cq;
-            float out[16], dl[16];
-            load_heads(b, out);
-            double s[DDRL_NSTAT];
-#pragma unroll
-            for (int i = 0; i < DDRL_NSTAT; ++i) s[i] = 0.0;
-#pragma unroll
-            for (int i = 0; i < 16; ++i) dl[i] = 0.f;
-            if (row < nrows) {
-                const float* pa = pf;
-                const float* po = reinterpret_cast<const float*>(sm + S.po);
-                const float* ps = pa + TC_ROWS * A + (S.po_in_w1 ? 0 : TC_ROWS * A2);
-                if (b == 0) {
-                    float lg[A2];
-#pragma unroll
-                    for (int oo = 0; oo < A2; ++oo) lg[oo] = fmaf(out[oo], 1.f / (TC_SH * TC_SW), sbo[oo]);
-                    ppo_row_policy(lg, A, pa + row * A, po + row * A2, ps[row], ps[2 * TC_ROWS + row], klc,
-                                   a.hp.clip_param, a.hp.entropy_coeff, 1.f, dl, s);
-#pragma unroll
-                    for (int oo = 0; oo < (GBH_SMEM ? 0 : A2); ++oo) gbh[oo] += dl[oo];
-                    st[0] += s[0]; st[1] += s[1]; st[2] += s[3];
-                } else {
-                    const float val = fmaf(out[0], 1.f / (TC_SH * TC_SW), sbvo[0]);
-                    dl[0] = ppo_row_value(val, ps[TC_ROWS + row], ps[3 * TC_ROWS + row], a.hp.vf_clip_param,
-                                          a.hp.vf_loss_coeff, 1.f, s);
-                    if (!GBH_SMEM) gbh[0] += dl[0];
-                    st[0] += s[2]; st[1] += s[4]; st[2] += s[5]; st[3] += s[6]; st[4] += s[7];
-                }
-            }
-            if constexpr (GBH_SMEM) {      // dl is zero for rows beyond nrows: whole-warp sums, one writer per warp
-                double* redg = reinterpret_cast<double*>(sm + S.red);
-#pragma unroll
-                for (int oo = 0; oo < A2; ++oo) {
-                    if (b == 0 || oo == 0) {
-                        const float sx = warp_sum(dl[oo]);
-                        if (lane == 0) redg[warp * 24 + 8 + oo] += (double)sx;
-                    }
-                }
-            }
-            if (first) {   // per-branch gradient scale of this CTA: power of two with max|dl| * scale ~ TC_GTARGET
-                float mx = 0.f;
-#pragma unroll
-                for (int i = 0; i < 16; ++i) mx = fmaxf(mx, fabsf(dl[i]));
-#pragma unroll
-                for (int off = 16; off > 0; off >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, off));
-                float* smx = reinterpret_cast<float*>(sm + S.red);      // [8 warps]
-                if (lane == 0) smx[warp] = mx;
-                if (b == 0) asm volatile("bar.sync 1, 128;" ::: "memory");   // the four loss warps of this branch only
-                else        asm volatile("bar.sync 2, 128;" ::: "memory");
-                mx = fmaxf(fmaxf(smx[4 * b], smx[4 * b + 1]), fmaxf(smx[4 * b + 2], smx[4 * b + 3]));
-                int e = 0;
-                if (mx > 0.f && mx < 3.0e38f) e = (int)floorf(log2f(TC_GTARGET / mx));
-                e = max(-20, min(20, e));
-                if (q == 0 && lane == 0) sgs[b] = exp2f((float)e);
-                if (b == 0) asm volatile("bar.sync 1, 128;" ::: "memory");
-                else        asm volatile("bar.sync 2, 128;" ::: "memory");
-            }
-            const float sg_l = sgs[b];
-#pragma unroll
-            for (int c = 0; c < 2; ++c) {
-                uint4 hi, lo;
-                ovf |= tc_split8(&dl[8 * c], sg_l, hi, lo) ? 8 : 0;
-                *reinterpret_cast<uint4*>(sm + sDL(b, 0) + (c * TC_ROWS + row) * 16) = hi;
-                *reinterpret_cast<uint4*>(sm + sDL(b, 1) + (c * TC_ROWS + row) * 16) = lo;
-            }
-        }
-        T2_STAMP(17);
-        publish_sync();
-        T2_STAMP(18);
-        const bool nxt_none = row0 + TC_ROWS >= cr1;
-        {   // both branches consumed the staged loss inputs: fetch the next tile's
-            const int64_t nxt = row0 + TC_ROWS;
-            if (nxt < cr1) prefetch_loss(nxt, (int)min((int64_t)TC_ROWS, cr1 - nxt));
-        }
-        if (nxt_none && cq < 2) {   // last tile: the loss warps add up the head-bias gradients and the loss statistics (per-warp
-            // sums, read after the write-out barrier) while they would otherwise wait for B1 — 5 float64 warp reductions that
-            // used to sit between the last epilogue and the write-out
-            double* redd = reinterpret_cast<double*>(sm + S.red);          // [8 warps][24]
-#pragma unroll
-            for (int i = 0; i < A2; ++i) {
-                if constexpr (!GBH_SMEM) {
-                    const float sx = warp_sum(gbh[i]);
-                    if (lane == 0) redd[warp * 24 + 8 + i] = (double)sx;
-                }
-            }
-#pragma unroll
-            for (int i = 0; i < 5; ++i) {
-                const double sx = warp_sum(st[i]);
-                if (lane == 0) redd[warp * 24 + i] = sx;
-            }
-        }
-        const float sg0 = sgs[0], sg1 = sgs[1];
-        // ---- B1: gWh_b[k][o] (+)= H2_b^T DL_b ;  dz2-pre: Dacc_b = DL_b * WoT_b (B MN-major) ---------------------------
-        // ---- dz2 epilogue -> B3: gW2_b (+)= H1_b^T dZ2_b; gb2_b (+)= dZ2_b^T 1;  B4: Dacc_b = dZ2_b * W2b^T -------------
-#pragma unroll 1
-        for (int b = 0; b < 2; ++b) {
-            const float sg = b ? sg1 : sg0;
-            wait_b(b);      // B1 has consumed H2_b; dz2 = pre * (1 - h2^2) overwrites it
-            T2_STAMP(19 + 3 * b);
-            ovf |= t2_epi_grad(tmem + tlane + T2_DACC + 64 * b + 16 * cq, 1.f / (sg * TC_SW), sg, sm + sH2(b, 0),
-                               sm + sH2(b, 1), row, cq) ? 16 : 0;
-            T2_STAMP(20 + 3 * b);
-            publish();
-            T2_STAMP(21 + 3 * b);
-        }
-        if (S.dl_in_w1 && row0 + TC_ROWS < cr1) {   // both B1 are complete (DL dead) and another tile follows: restore W1
-            const unsigned char* img_p = a.img + (int64_t)p * I.bytes;
-#pragma unroll 1
-            for (int i = iW1(0, 0) / 16 + tid; i < iW2(0, 0) / 16; i += TC_NT) tc_cp16(sm + 16 * i, img_p + 16 * i);
-        }
-        // ---- dz1 epilogue -> B5: gW1_b[c][d] (+)= dZ1_b^T X   (column D of X is the constant 1 -> bias gradient) --------
-#pragma unroll 1
-        for (int b = 0; b < 2; ++b) {
-            const float sg = b ? sg1 : sg0;
-            wait_b(b);      // B3 has consumed H1_b; dz1 = (dz2 W2^T) * (1 - h1^2) overwrites it
-            if (b == 1) {   // B3(1) done: dZ2_1 (in H2[1]) is dead -> stream the next tile's observations into that space
-                const int64_t nxt = row0 + TC_ROWS;
-                if (nxt < cr1) prefetch_x(nxt, (int)min((int64_t)TC_ROWS, cr1 - nxt));
-                asm volatile("cp.async.commit_group;\n" ::);
-            }
-            T2_STAMP(25 + 3 * b);
-            ovf |= t2_epi_grad(tmem + tlane + T2_DACC + 64 * b + 16 * cq, 1.f / (sg * TC_SW), sg, sm + sH1(b, 0),
-                               sm + sH1(b, 1), row, cq) ? 32 : 0;
-            T2_STAMP(26 + 3 * b);
-            publish();
-            T2_STAMP(27 + 3 * b);
-        }
-        first = false;
-    }
-    if (!FWD) {
-    if constexpr (LL) {   // B5 of the last tile is in flight: gW2 / gb2 / gWh (complete since B3 / B1) leave meanwhile
-        umma::fence_after_sync();
-        write_w2_heads(0);
-        write_w2_heads(1);
-    } else if (early_out && staged) {
-        // [W2, bo) of the flat vector (gW2, gb2 of both branches, gWo: ~3/4 of it) has been staged by the MMA warps (slots 1, 2)
-        // and leaves for global memory while B5(1) is still running
-        asm volatile("bar.sync 6, %0;" ::"n"(T2_NT) : "memory");
-        T2_STAMP(46);
-        copy_out(o.W2 >> 2, o.bo >> 2, tid, TC_NT);
-    }
-    T2_STAMP(47);
-    wait_b(0);
-    wait_b(1);
-    T2_STAMP(31);
-    T2_GSTAMP(1);
-    asm volatile("cp.async.wait_group 0;\n" ::: "memory");
-    }   // training only
-    }   // epilogue warps
-    if (FWD) break;      // inference: no partial gradient, no statistics, no tail
-
-    // ---- late write-out: what B5 produced (gW1, b1); everything else left while B5 was running (or leaves now: clusters) ----
-    __syncthreads();      // (stacked accumulators: the MMA warps arrive here once they have staged gW1 / gb1 — slot 3)
-    T2_STAMP(45);
-    if constexpr (LL) {
-        if (warp < T2_MMA_WARP) {
-            write_w1(0);
-            write_w1(1);
-        }
-        if (warp == 0) bias_stats(lane);
-    } else if (!(early_out && staged)) {
-        if (warp == 0) bias_stats(lane);
-    }
-    T2_STAMP(32);
-    } while (0);
-    if (staged) {   // the rest of the staged partial (gW1 / gb1 of both branches, head biases, gWvo) leaves (all 20 warps copy)
-        copy_out(0, o.W2 >> 2, tid, T2_NT);
-        copy_out(o.bo >> 2, NPs >> 2, tid, T2_NT);
-        T2_STAMP(48);
-        __syncthreads();      // the next step's observations are streamed into H2[1] below
-    }
-    if (!LL && cs > 1) {   // in-cluster reduction over distributed shared memory: CTA `crank` adds part `crank` of the cs staged partials
-        __syncthreads();
-        if (cr1 > cr0) {   // the lo-half rows of the stacked weight-gradient accumulators were staged at the start of shared memory
-            float4* h0 = reinterpret_cast<float4*>(stg);
-            const float4* h1 = reinterpret_cast<const float4*>(sm);
-            for (int i = tid; i < (NPs >> 2); i += T2_NT) {
-                const float4 u = h0[i], w = h1[i];
-                h0[i] = make_float4(u.x + w.x, u.y + w.y, u.z + w.z, u.w + w.w);
-            }
-            __syncthreads();
-        }
-        umma::cluster_sync_all();
-        const int n4 = NPs >> 2, pl4 = (n4 + cs - 1) / cs;          // float4s in the vector / per part
-        float4* dstp = reinterpret_cast<float4*>(a.grad_part + ((int64_t)p * G + cid) * NPs);
-        const uint32_t stg_s = umma::smem_u32(stg);
-#pragma unroll 1
-        for (int i = crank * pl4 + tid; i < min(n4, (crank + 1) * pl4); i += T2_NT) {
-            float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-#pragma unroll 1
-            for (int r0 = 0; r0 < cs; r0 += 8) {     // up to 8 remote loads in flight, rank order
-                float4 v[8];
-#pragma unroll
-                for (int k = 0; k < 8; ++k)
-                    v[k] = (r0 + k < cs) ? umma::ld_dsmem_f4(umma::dsmem_addr(stg_s + 16u * (uint32_t)i, (uint32_t)(r0 + k)))
-                                         : make_float4(0.f, 0.f, 0.f, 0.f);
-#pragma unroll
-                for (int k = 0; k < 8; ++k) { acc.x += v[k].x; acc.y += v[k].y; acc.z += v[k].z; acc.w += v[k].w; }
-            }
-            dstp[i < n4 - (o.W2 >> 2) ? i + (o.W2 >> 2) : i - (n4 - (o.W2 >> 2))] = acc;      // staging (rotated) -> flat index
-        }
-    }
-    T2_STAMP(33);
-    T2_GSTAMP(2);
-    prefetched = false;
-    // barrier-A arrival BEFORE the prefetch below is issued: the release then drains the partial's stores only (the copy-out
-    // path ends in a __syncthreads(), so every store of the CTA is ordered before this thread's arrival)
-    const bool arrive_early = !LL && staged && has_tail;
-    if (arrive_early && tid == 0) sgd_tail_arrive_a(a.tail, p);
-    if (s + 1 < nsteps && warp < T2_MMA_WARP) {   // the next step's inputs do not depend on the weights: request them now,
-        const int mbn = a.mb_perm ? a.mb_perm[(int64_t)p * a.perm_stride + step + 1] : step + 1;   // they land behind the tail
-        const int64_t n0 = (int64_t)mbn * a.MB, n1 = min(n0 + a.MB, a.R);
-        const int64_t c0n = min(n0 + (int64_t)bx * rpc, n1), c1n = min(c0n + rpc, n1);
-        if (c1n > c0n) {
-            const int nn = (int)min((int64_t)TC_ROWS, c1n - c0n);
-            prefetch_x(c0n, nn);
-            prefetch_loss(c0n, nn);
-            asm volatile("cp.async.commit_group;\n" ::);
-            prefetched = true;
-        }
-    }
-    if (has_tail) {   // fused grad-reduce + [peer all-reduce] + clip + Adam
-        ts.round = s + 1;
-        ts.last = s == nsteps - 1;
-        bool tok;
-        if constexpr (LL) {
-            __syncthreads();      // every thread is past its last use of the shared memory the tail scratches
-            tok = sgd_step_tail_ll(a.tail, ts, p, gridDim.y, bx, G, o.NP, step, D, A, reinterpret_cast<float*>(sm + S.X[0]),
-                                   sm + sH1(0, 0), sbase + S.bar + 32, ll_phase, DBG ? a.dbg_clock : nullptr);
-        } else {
-            tok = sgd_step_tail(a.tail, ts, a.grad_part, a.stat_part, p, gridDim.y, bx, G, o.NP, step, D, A,
-                                reinterpret_cast<float*>(sm + sH2(0, 0)), DBG ? a.dbg_clock : nullptr, ncl, arrive_early);
-        }
-        ok = ok && tok;
-        ts.b1p *= a.tail.beta1;
-        ts.b2p *= a.tail.beta2;
-        ts.seq += 1u;
-    }
-    T2_STAMP(34);
-    T2_GSTAMP(7);
-    }   // steps of this launch
-    if (a.status) {
-        if (tid == 0 && !ok) atomicOr(a.status, 1);
-        if (ovf) atomicOr(a.status, ovf);
-    }
-    umma::fence_before_sync();
-    __syncthreads();
-    if (warp == 0) umma::tmem_dealloc(tmem, T2_TMEM_COLS);
+// the leg-coupled step (SharedDecentralLegID): A = 2, D = DT
+template <int DT>
+__global__ void __launch_bounds__(T2_NT, 1) fcnet_train_tc2_cup_kernel(const __grid_constant__ TcTrainArgs a,
+                                                                       const int32_t* __restrict__ node_id,
+                                                                       const float* __restrict__ cup_theta) {
+    constexpr int A = 2;
+    constexpr bool FWD = false, LL = false, DBG = false, CUP = true;
+#include "tc2_step_body.inc"
 }
 
 static int g_tc2_cluster = 0;    // 0 = off (default: measured slower, DESIGN.md §4.1), -1 = automatic (largest of 16, 8, 4, 2 that
@@ -1252,6 +279,35 @@ int launch_tc2(const TcTrainArgs& a_in, int P, int G, cudaStream_t st) {
         case 8: return launch_tc2_t<8, false, false>(a, P, G, smem, st, &g_tc2_last_cluster);
         default: set_error("ppo_train_step_tc: ping-pong kernel supports A in {1,2,4,8}"); return DDRL_E_UNSUPPORTED_SHAPE;
     }
+}
+
+// leg-coupled step: no clusters, no LL tail (the entry point rejects both); instantiated for SharedDecentralLegID's D = 19, 20
+template <int DT>
+static int launch_tc2_cup_t(const TcTrainArgs& a, const int32_t* node_id, const float* theta, int P, int G, cudaStream_t st) {
+    static bool attr = false;
+    auto kern = fcnet_train_tc2_cup_kernel<DT>;
+    if (!attr) {
+        if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess) {
+            set_error("ppo_train_step_tc_coupled: cannot raise dynamic shared memory: %s", cudaGetErrorString(cudaGetLastError()));
+            return DDRL_E_CUDA;
+        }
+        attr = true;
+    }
+    const size_t smem = (size_t)tc2_smem(DT, 2, true).total;
+    kern<<<dim3(G, P), T2_NT, smem, st>>>(a, node_id, theta);
+    g_tc2_last_cluster = 1;
+    return DDRL_OK;
+}
+
+int launch_tc2_cup(const TcTrainArgs& a, const int32_t* node_id, const float* theta, int P, int G, cudaStream_t st) {
+    if (g_tc2_cluster != 0) {
+        set_error("ppo_train_step_tc_coupled: thread-block clusters are not supported with leg coupling (ddrl_tc_set_cluster(1))");
+        return DDRL_E_BADARG;
+    }
+    if (a.A == 2 && a.D == 19) return launch_tc2_cup_t<19>(a, node_id, theta, P, G, st);
+    if (a.A == 2 && a.D == 20) return launch_tc2_cup_t<20>(a, node_id, theta, P, G, st);
+    set_error("ppo_train_step_tc_coupled: instantiated for A = 2 and D in {19, 20} (SharedDecentralLegID), got D=%d A=%d", a.D, a.A);
+    return DDRL_E_UNSUPPORTED_SHAPE;
 }
 
 int launch_tc2_forward(const TcTrainArgs& a, int P, int G, cudaStream_t st) {

@@ -591,6 +591,43 @@ def ppo_train_step_tc(tc_img, obs, actions, old_logits, old_logp, vf_preds, adv,
         C.byref(tail) if tail is not None else None, _stream()), "ppo_train_step_tc")
 
 
+STATUS_BAD_NODE = 128      # DDRL_STATUS_BAD_NODE: a node id outside 0..3 reached a leg-coupled step
+
+
+def ppo_train_step_tc_coupled(tc_img, theta, node_id, obs, actions, old_logits, old_logp, vf_preds, adv, vtarg, A: int, MB: int,
+                              mb_perm, step_ctr, kl_coeff, hyper: PPOHyper, ctas_per_policy: int, grad_part, stat_part,
+                              status, tail: SgdTail):
+    """Leg-coupled tensor-core step (SharedDecentralLegID, ddrl_ppo_train_step_tc_coupled): theta [1, NP + 8] (FCNet
+    variables, then leg_coupling [4, 2]), node_id [1, R] int32, grad_part [1, G, part_stride(NP + 8)]; fused tail required."""
+    P, R, D = obs.shape
+    f32 = torch.float32
+    perm_stride = mb_perm.shape[-1] if mb_perm is not None else 0
+    _lib.check(_lib.load().ddrl_ppo_train_step_tc_coupled(
+        _p(tc_img, torch.uint8, "tc_img"), _p(theta, f32, "theta"), _p(node_id, torch.int32, "node_id"), _p(obs, f32, "obs"),
+        _p(actions, f32, "actions"), _p(old_logits, f32, "old_logits"), _p(old_logp, f32, "old_logp"),
+        _p(vf_preds, f32, "vf_preds"), _p(adv, f32, "adv"), _p(vtarg, f32, "vtarg"), P, R, D, A, MB,
+        _p(mb_perm, torch.int32, "mb_perm"), perm_stride, _p(step_ctr, torch.int32, "step_ctr"), _p(kl_coeff, f32, "kl_coeff"),
+        C.byref(hyper), ctas_per_policy, _p(grad_part, f32, "grad_part"), _p(stat_part, torch.float64, "stat_part"),
+        _p(status, torch.int32, "status"), C.byref(tail) if tail is not None else None, _stream()), "ppo_train_step_tc_coupled")
+
+
+def ppo_train_step_coupled(theta, img, node_id, obs, actions, old_logits, old_logp, vf_preds, adv, vtarg, A: int, MB: int,
+                           mb_perm, step_ctr, kl_coeff, hyper: PPOHyper, ctas_per_policy: int, grad_part, stat_part,
+                           tail: SgdTail):
+    """Leg-coupled FP32 step (ddrl_ppo_train_step_coupled): as ppo_train_step_tc_coupled with the packed FP32 image `img`
+    of the first NP entries of theta; the device flag goes to tail.status."""
+    P, R, D = obs.shape
+    f32 = torch.float32
+    perm_stride = mb_perm.shape[-1] if mb_perm is not None else 0
+    _lib.check(_lib.load().ddrl_ppo_train_step_coupled(
+        _p(theta, f32, "theta"), _p(img, f32, "img"), _p(node_id, torch.int32, "node_id"), _p(obs, f32, "obs"),
+        _p(actions, f32, "actions"), _p(old_logits, f32, "old_logits"), _p(old_logp, f32, "old_logp"),
+        _p(vf_preds, f32, "vf_preds"), _p(adv, f32, "adv"), _p(vtarg, f32, "vtarg"), P, R, D, A, MB,
+        _p(mb_perm, torch.int32, "mb_perm"), perm_stride, _p(step_ctr, torch.int32, "step_ctr"), _p(kl_coeff, f32, "kl_coeff"),
+        C.byref(hyper), ctas_per_policy, _p(grad_part, f32, "grad_part"), _p(stat_part, torch.float64, "stat_part"),
+        C.byref(tail) if tail is not None else None, _stream()), "ppo_train_step_coupled")
+
+
 def obs_gather(obs_full: torch.Tensor, table: torch.Tensor, P: int, out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """obs_full [S, Dfull] f32/f64, table [Ag, D] i32 -> [P, S*(Ag/P), D] f32 (agent a -> policy a // (Ag/P))."""
     S, Dfull = obs_full.shape

@@ -123,14 +123,35 @@ class FCNetLearner(_LearnerBase):
     def __init__(self, P: int, D: int, A: int, cfg: PPOConfig, device="cuda", theta: Optional[torch.Tensor] = None,
                  use_graph: bool = True, ctas_per_policy: Optional[int] = None, mode: str = "tc", fuse_tail: bool = True,
                  persistent: bool = True, tc_forward: bool = True, ll_tail: bool = False, vf_share_layers: bool = False,
-                 free_log_std: bool = False, atomic_reduce: bool = True):
+                 free_log_std: bool = False, atomic_reduce: bool = True, leg_coupling: bool = False):
         """mode: "tc"   = tensor-core (tcgen05) SGD step, fp16 hi/lo operand split (gradients within 5e-5 of scale);
                  "fp32" = FP32-FMA SGD step (1e-5 parity).  Inference / GAE / Adam are FP32 in both modes.
         vf_share_layers / free_log_std: the reference model's optional layouts (models/fcnet_glorot_uniform_init.py:30-36,
         85-113).  `theta` is then [P, NPm] in the MODEL's variable order (`modelv2.fcnet_variant_shapes`); the kernels run on
         its index-select (`self.theta`, tied value branch / constant zero columns), the gradients of tied copies are added
         (`ddrl_grad_tie`) and clip + Adam act on the model variables (`self.theta_model`) — the kernel-per-stage step, since
-        the fused tail owns kernel-layout slices."""
+        the fused tail owns kernel-layout slices.
+        leg_coupling: the policy of QuantrupedMultiEnv_SharedDecentralLegID (model "cup" = FCNet + LegCoupling,
+        models/coupling_net_glorot_uniform_init.py:11-30,135): ONE shared policy (P = 1), A = 2.  `theta` is then
+        [1, NP + 8] — the 12 FCNet variables in checkpoint order, then leg_coupling [4, 2] row-major (the registration order
+        of the ModelV2 class); m / v alike; default table LegCoupling.INIT.  The mean logits of a row are scaled by
+        c[node id], node id = the agent's position in agent_names (FL, HL, HR, FR); the SGD steps are
+        ddrl_ppo_train_step_tc_coupled / ddrl_ppo_train_step_coupled (fused tail required: the table is clipped and stepped
+        with the MLP weights)."""
+        self.coupled = bool(leg_coupling)
+        if self.coupled:
+            if P != 1 or A != 2:
+                raise DDRLError(f"leg_coupling: the coupled model is one shared policy with A = 2 (got P={P}, A={A})")
+            if not fuse_tail or ll_tail or vf_share_layers or free_log_std:
+                raise DDRLError("leg_coupling: fuse_tail=False, ll_tail and the optional FCNet layouts are not supported")
+            if mode == "tc" and D not in (19, 20):
+                raise DDRLError(f"leg_coupling: the tensor-core step is instantiated for D in (19, 20), got D={D}")
+            if _dist_world()[1] > 1:
+                raise DDRLError("leg_coupling: data-parallel training (world > 1) is not supported")
+            if theta is None:
+                theta = torch.zeros(1, K.fcnet_num_params(D, A) + 8, dtype=torch.float32)
+                from .modelv2 import LegCoupling
+                theta[0, -8:] = torch.tensor(LegCoupling.INIT, dtype=torch.float32).reshape(-1)
         self.variant = bool(vf_share_layers or free_log_std)
         theta_model = None
         if self.variant:
@@ -141,7 +162,9 @@ class FCNetLearner(_LearnerBase):
                 raise DDRLError(f"optional FCNet layout: theta must be [P={P}, {NPm}] in the model's variable order")
             theta_model, theta = theta, None
             fuse_tail, persistent = False, False
-        super().__init__(P, K.fcnet_num_params(D, A), cfg, device, theta)
+        self.NPf = K.fcnet_num_params(D, A)      # FCNet variables (the coupled model adds its table behind them)
+        super().__init__(P, self.NPf + (8 if self.coupled else 0), cfg, device, theta)
+        self.theta_fc = self.theta[:, :self.NPf]      # (view: the FCNet part, what the weight images are packed from)
         if self.variant:
             dev_ = self.device
             self.NPm = NPm
@@ -190,7 +213,7 @@ class FCNetLearner(_LearnerBase):
         self.tc_img = None
         self.tc_status = torch.zeros(1, dtype=torch.int32, device=dev)
         if mode == "tc":
-            self.tc_img = K.fcnet_tc_pack(self.theta, D, A)
+            self.tc_img = K.fcnet_tc_pack(self.theta_fc, D, A)
         self._bufs = None
         self._graph = None
         self._graph_key = None
@@ -214,6 +237,9 @@ class FCNetLearner(_LearnerBase):
             b[name] = torch.empty(P, R, dtype=f32, device=dev)
             b[name + "_s"] = torch.empty(P, R, dtype=f32, device=dev)
         b["vboot"] = torch.empty(P, Cc, dtype=f32, device=dev)
+        if self.coupled:      # node id of every row (learn_on_rollout: column c of an env-major [T, C] rollout is leg c % 4)
+            b["node"] = (torch.arange(R, dtype=torch.int32, device=dev) % 4).reshape(1, R).contiguous()
+            b["node_s"] = torch.empty_like(b["node"])
         b["moments"] = torch.empty(P, 3, dtype=torch.float64, device=dev)
         b["gae_ws"] = torch.empty(max(8, P * ((Cc + 255) // 256) * 16), dtype=torch.uint8, device=dev)
         b["filt_ws"] = None
@@ -274,6 +300,19 @@ class FCNetLearner(_LearnerBase):
                 self._peer_exchange(G).fill(tail)
         elif nsteps != 1:
             raise DDRLError("multi-step launches need the fused tail")
+        if self.coupled:
+            if tail is None:
+                raise DDRLError("leg_coupling: the coupled SGD step needs the fused tail")
+            if self.mode == "tc":
+                K.ppo_train_step_tc_coupled(self.tc_img, self.theta, src["node"], src["obs"], src["act"], src["logits"],
+                                            src["logp"], src["value"], src["adv"], src["vtarg"], self.A, MB, b["mb_perm"],
+                                            self.step_ctr, self.kl_coeff, hyper, G, b["grad_part"], b["stat_part"],
+                                            self.tc_status, tail)
+            else:
+                K.ppo_train_step_coupled(self.theta, self.img, src["node"], src["obs"], src["act"], src["logits"], src["logp"],
+                                         src["value"], src["adv"], src["vtarg"], self.A, MB, b["mb_perm"], self.step_ctr,
+                                         self.kl_coeff, hyper, G, b["grad_part"], b["stat_part"], tail)
+            return
         if self.mode == "tc":
             K.ppo_train_step_tc(self.tc_img, src["obs"], src["act"], src["logits"], src["logp"], src["value"], src["adv"],
                                 src["vtarg"], self.A, MB, b["mb_perm"], self.step_ctr, self.kl_coeff, hyper, G,
@@ -312,9 +351,9 @@ class FCNetLearner(_LearnerBase):
         P, R, D = obs_flat.shape
         cfg, A = self.cfg, self.A
         self.tc_status.zero_()
-        K.fcnet_pack(self.theta, D, A, self.img)
+        K.fcnet_pack(self.theta_fc, D, A, self.img)
         if self.tc_img is not None:
-            K.fcnet_tc_pack(self.theta, D, A, self.tc_img)
+            K.fcnet_tc_pack(self.theta_fc, D, A, self.tc_img)
         # (i) filter + forward + sample ------------------------------------------------------------------
         if update_filter:
             if self.world > 1:
@@ -329,7 +368,22 @@ class FCNetLearner(_LearnerBase):
                 K.filter_merge(allp, R * self.world, self.filt_n, self.filt_M, self.filt_S, self.norm)
             else:
                 K.filter_update(obs_flat, self.filt_n, self.filt_M, self.filt_S, self.norm, b["filt_ws"])
-        if self.tc_forward and self.tc_img is not None and K.tc_pingpong_eligible(D, A):
+        if self.coupled:
+            # forward without sampling, LegCoupling on the mean logits, then DiagGaussian sample + logp of the COUPLED
+            # distribution (the stored old logits are the coupled ones)
+            out = {"logits": b["logits"], "value": b["value"], "obs_out": b["obs"]}
+            if self.tc_forward and self.tc_img is not None:
+                K.fcnet_forward_tc(self.tc_img, obs_flat, A, norm=self.norm, clip=cfg.filter_clip, out=out, status=self.tc_status)
+            else:
+                K.fcnet_forward(self.theta_fc, obs_flat, A, norm=self.norm, clip=cfg.filter_clip, out=out, img=self.img)
+            self._couple_and_sample(b["logits"], b["node"], eps_flat, b["act"], b["logp"])
+            if self.tc_forward and self.tc_img is not None:
+                K.fcnet_forward_tc(self.tc_img, boot_obs, A, norm=self.norm, clip=cfg.filter_clip,
+                                   out={"logits": None, "value": b["vboot"], "obs_out": None}, status=self.tc_status)
+            else:
+                K.fcnet_forward(self.theta_fc, boot_obs, A, norm=self.norm, clip=cfg.filter_clip,
+                                out={"logits": None, "value": b["vboot"], "obs_out": None}, img=self.img)
+        elif self.tc_forward and self.tc_img is not None and K.tc_pingpong_eligible(D, A):
             # inference on the tensor cores (same pipeline as the training forward, ~3e-6 relative)
             K.fcnet_forward_tc(self.tc_img, obs_flat, A, norm=self.norm, clip=cfg.filter_clip, eps=eps_flat,
                                out={"logits": b["logits"], "value": b["value"], "obs_out": b["obs"], "action": b["act"],
@@ -352,6 +406,17 @@ class FCNetLearner(_LearnerBase):
         if shuffle is not None:
             for nme in ("obs", "act", "logits", "logp", "value", "adv", "vtarg"):
                 K.gather_rows(b[nme], shuffle, b[nme + "_s"])
+            if self.coupled:      # the node ids travel with their rows (a 4-byte row copy: the int32 bits move unchanged)
+                K.gather_rows(b["node"].view(torch.float32), shuffle, b["node_s"].view(torch.float32))
+
+    def _couple_and_sample(self, logits, node, eps, act, logp):
+        """logits [1,R,4] in place *= LegCoupling table [node] (mean half), then action / logp of the coupled DiagGaussian."""
+        from . import _lib
+        R = logits.shape[1]
+        K.leg_coupling_(logits.view(R, 4), node.view(R), self.theta[0, self.NPf:])
+        f32 = torch.float32
+        _lib.check(_lib.load().ddrl_dg_sample(K._p(logits, f32, "logits"), K._p(eps, f32, "eps"), R, self.A,
+                                              K._p(act, f32, "action"), K._p(logp, f32, "logp"), K._stream()), "dg_sample")
 
     def _prepare_cached(self, b, obs_flat, boot_obs, rewards, dones, eps_flat, shuffle, cols_per_env, update_filter, T, Cc):
         """The ~20 short launches of the preparation phase are captured once per set of input buffers and replayed (the
@@ -402,10 +467,13 @@ class FCNetLearner(_LearnerBase):
         if D != self.D or P != self.P:
             raise DDRLError(f"raw_obs shape {tuple(raw_obs.shape)} does not match learner (P={self.P}, D={self.D})")
         R = T * Cc
+        if self.coupled and (cols_per_env != 4 or Cc % 4):
+            raise DDRLError(f"leg_coupling: the rollout's columns must be env-major legs (cols_per_env=4, C % 4 == 0), got "
+                            f"cols_per_env={cols_per_env}, C={Cc}")
         b = self._alloc(T, Cc)
         obs_flat = raw_obs.reshape(P, R, D)
         eps_flat = eps.reshape(P, R, A)
-        names = ("obs", "act", "logits", "logp", "value", "adv", "vtarg")
+        names = ("obs", "act", "logits", "logp", "value", "adv", "vtarg") + (("node",) if self.coupled else ())
         src_key = "s" if shuffle is not None else "u"
         src = {n_: b[n_ + ("_s" if shuffle is not None else "")] for n_ in names}
         self._prepare_cached(b, obs_flat, boot_obs, rewards, dones, eps_flat, shuffle, cols_per_env, update_filter, T, Cc)
@@ -497,8 +565,10 @@ class FCNetLearner(_LearnerBase):
         if code:
             what = [n for bit, n in ((1, "MMA completion timed out"), (2, "x overflow"), (4, "activation overflow"),
                                      (8, "dl overflow"), (16, "dz2 overflow"), (32, "dz1 overflow"),
-                                     (64, "fused-tail barrier / peer wait timed out")) if code & bit]
+                                     (64, "fused-tail barrier / peer wait timed out"),
+                                     (K.STATUS_BAD_NODE, "leg-coupling node id outside 0..3")) if code & bit]
             hint = (" — fp16 split range exceeded: use mode='fp32' for this workload" if code & 62 else
+                    " — node ids must be 0..3 (FL, HL, HR, FR)" if code & K.STATUS_BAD_NODE else
                     " — a CTA barrier or a peer rank did not arrive in time")
             raise DDRLError("SGD step failed (" + ", ".join(what) + ")" + hint)
         self._update_kl(stats)
@@ -507,17 +577,23 @@ class FCNetLearner(_LearnerBase):
     def learn_on_batch(self, obs: torch.Tensor, actions: torch.Tensor, action_dist_inputs: torch.Tensor,
                        action_logp: torch.Tensor, vf_preds: torch.Tensor, advantages: torch.Tensor,
                        value_targets: torch.Tensor, perms: torch.Tensor, shuffle: Optional[torch.Tensor] = None,
-                       standardize: bool = True) -> List[Dict[str, float]]:
+                       standardize: bool = True, node_idx: Optional[torch.Tensor] = None) -> List[Dict[str, float]]:
         """The learner half only, on POSTPROCESSED sample-batch columns as RLlib's `Policy.learn_on_batch` receives them
         (rollout workers have already filtered the observations, sampled the actions and run `postprocess_ppo_gae`):
         obs [P,R,D] (filtered), actions [P,R,A], action_dist_inputs [P,R,2A], action_logp / vf_preds / advantages /
         value_targets [P,R] — float32 CUDA tensors, one row block per policy.  `standardize` applies
         StandardizeFields(["advantages"]) per policy; `shuffle` [P,R] int32 and `perms` [P,E,nb] as in learn_on_rollout.
-        Runs StandardizeFields -> shuffle -> E x nb minibatch steps -> KL update and returns the learner stats."""
+        Runs StandardizeFields -> shuffle -> E x nb minibatch steps -> KL update and returns the learner stats.
+        leg_coupling: node_idx [1,R] int32 CUDA (0..3: FL, HL, HR, FR) is required; action_dist_inputs are coupled logits."""
         P, R, D = obs.shape
         A = self.A
         if D != self.D or P != self.P:
             raise DDRLError(f"obs shape {tuple(obs.shape)} does not match learner (P={self.P}, D={self.D})")
+        if self.coupled != (node_idx is not None):
+            raise DDRLError("learn_on_batch: node_idx [1, R] int32 is required with leg_coupling and only then")
+        if node_idx is not None and (tuple(node_idx.shape) != (P, R) or node_idx.dtype != torch.int32 or not node_idx.is_cuda):
+            raise DDRLError(f"learn_on_batch: node_idx must be an int32 CUDA tensor of shape {(P, R)}, got {node_idx.dtype} "
+                            f"{tuple(node_idx.shape)} on {node_idx.device}")
         cols = {"obs": (obs, (P, R, D)), "act": (actions, (P, R, A)), "logits": (action_dist_inputs, (P, R, 2 * A)),
                 "logp": (action_logp, (P, R)), "value": (vf_preds, (P, R)), "adv": (advantages, (P, R)),
                 "vtarg": (value_targets, (P, R))}
@@ -527,9 +603,9 @@ class FCNetLearner(_LearnerBase):
                                 f"got {t.dtype} {tuple(t.shape)} on {t.device}")
         b = self._alloc(R, 1)
         self.tc_status.zero_()
-        K.fcnet_pack(self.theta, D, A, self.img)
+        K.fcnet_pack(self.theta_fc, D, A, self.img)
         if self.tc_img is not None:
-            K.fcnet_tc_pack(self.theta, D, A, self.tc_img)
+            K.fcnet_tc_pack(self.theta_fc, D, A, self.tc_img)
         for name, (t, _) in cols.items():
             b[name].copy_(t)
         if standardize:
@@ -538,6 +614,11 @@ class FCNetLearner(_LearnerBase):
         if shuffle is not None:
             for nme in names:
                 K.gather_rows(b[nme], shuffle, b[nme + "_s"])
+        if self.coupled:
+            b["node"].copy_(node_idx)
+            if shuffle is not None:
+                K.gather_rows(b["node"].view(torch.float32), shuffle, b["node_s"].view(torch.float32))
+            names = names + ("node",)
         src = {n_: b[n_ + ("_s" if shuffle is not None else "")] for n_ in names}
         return self._sgd_phase(b, src, "s" if shuffle is not None else "u", perms, R, R, 1)
 
@@ -561,13 +642,34 @@ class FCNetLearner(_LearnerBase):
         K.filter_merge(zero, 0, self.filt_n, self.filt_M, self.filt_S, self.norm)
 
     # ---- plain inference (sampler side) ---------------------------------------------------------------------
-    def compute_actions(self, raw_obs: torch.Tensor, eps: Optional[torch.Tensor] = None, update_filter: bool = False):
+    def compute_actions(self, raw_obs: torch.Tensor, eps: Optional[torch.Tensor] = None, update_filter: bool = False,
+                        node_idx: Optional[torch.Tensor] = None):
         """raw_obs [P,B,D] -> dict(logits, value[, action, logp]); optionally pushes the rows into the filter first
-        (RLlib sampler behaviour)."""
+        (RLlib sampler behaviour).  leg_coupling: node_idx [1,B] int32 (required); logits / action / logp are those of the
+        coupled distribution."""
+        if self.coupled != (node_idx is not None):
+            raise DDRLError("compute_actions: node_idx [1, B] int32 is required with leg_coupling and only then")
         if update_filter:
             K.filter_update(raw_obs, self.filt_n, self.filt_M, self.filt_S, self.norm)
         use_norm = self.norm if int(self.filt_n.max().item()) > 0 else None
-        return K.fcnet_forward(self.theta, raw_obs, self.A, norm=use_norm, clip=self.cfg.filter_clip, eps=eps)
+        if not self.coupled:
+            return K.fcnet_forward(self.theta, raw_obs, self.A, norm=use_norm, clip=self.cfg.filter_clip, eps=eps)
+        P, B, _ = raw_obs.shape
+        if tuple(node_idx.shape) != (P, B) or node_idx.dtype != torch.int32 or not node_idx.is_cuda:
+            raise DDRLError(f"compute_actions: node_idx must be an int32 CUDA tensor of shape {(P, B)}")
+        if int(((node_idx < 0) | (node_idx > 3)).sum().item()):
+            raise DDRLError("compute_actions: node ids must be 0..3 (FL, HL, HR, FR)")
+        res = K.fcnet_forward(self.theta_fc, raw_obs, self.A, norm=use_norm, clip=self.cfg.filter_clip)
+        K.leg_coupling_(res["logits"].view(B, 4), node_idx.reshape(B).contiguous(), self.theta[0, self.NPf:])
+        if eps is not None:
+            res["action"] = torch.empty(P, B, self.A, dtype=torch.float32, device=raw_obs.device)
+            res["logp"] = torch.empty(P, B, dtype=torch.float32, device=raw_obs.device)
+            from . import _lib
+            f32 = torch.float32
+            _lib.check(_lib.load().ddrl_dg_sample(K._p(res["logits"], f32, "logits"), K._p(eps, f32, "eps"), B, self.A,
+                                                  K._p(res["action"], f32, "action"), K._p(res["logp"], f32, "logp"),
+                                                  K._stream()), "dg_sample")
+        return res
 
 
 class GraphNetLearner(_LearnerBase):

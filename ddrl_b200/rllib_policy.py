@@ -37,8 +37,25 @@ ADVANTAGES, VALUE_TARGETS = "advantages", "value_targets"
 TRAIN_COLUMNS = (OBS, ACTIONS, ACTION_DIST_INPUTS, ACTION_LOGP, VF_PREDS, ADVANTAGES, VALUE_TARGETS)
 
 
+NODE_IDX = "node_idx"      # leg-coupled policy (SharedDecentralLegID): the Discrete(4) part of the Tuple observation
+
+
 class BatchError(ValueError):
     pass
+
+
+def check_node_idx(node_idx, rows: int, where: str) -> np.ndarray:
+    """The node-id part of the SharedDecentralLegID observation: [rows] integers 0..3 (FL, HL, HR, FR) -> int32."""
+    a = np.asarray(node_idx)
+    if a.ndim == 2 and a.shape[1] == 1:
+        a = a[:, 0]
+    if a.ndim != 1 or a.shape[0] != rows:
+        raise BatchError(f"{where}: node_idx must have shape [{rows}], got {a.shape}")
+    if a.dtype.kind not in "iu" and not (a.dtype.kind == "f" and np.all(np.isfinite(a)) and np.all(a == np.round(a))):
+        raise BatchError(f"{where}: node_idx must hold integers, got {a.dtype}")
+    if a.size and (a.min() < 0 or a.max() > 3):
+        raise BatchError(f"{where}: node_idx must be in 0..3 (FL, HL, HR, FR), got range [{a.min()}, {a.max()}]")
+    return np.ascontiguousarray(a.astype(np.int32))
 
 
 def stack_policy_batches(policy_batches: Mapping[str, Mapping[str, Any]], policy_names: Sequence[str], D: int, A: int,
@@ -118,7 +135,10 @@ class PPOPolicyGroup:
         import torch
         from .learner import FCNetLearner
         env = _policies.ARCHITECTURES[policy_scope]
-        if getattr(env, "model", "fc_glorot_uniform_init") != "fc_glorot_uniform_init":
+        self.coupled = getattr(env, "model", "fc_glorot_uniform_init") == "cup"
+        if self.coupled:
+            learner_kw = dict(learner_kw, leg_coupling=True)
+        elif getattr(env, "model", "fc_glorot_uniform_init") != "fc_glorot_uniform_init":
             raise NotImplementedError(f"{policy_scope}: PPOPolicyGroup serves the FCNet architectures; the shared GraphNet "
                                       "policy is driven through learner.GraphNetLearner")
         self.env = env
@@ -137,13 +157,25 @@ class PPOPolicyGroup:
     def compute_actions(self, obs_by_policy: Mapping[str, np.ndarray], explore: bool = True, update_filter: bool = False):
         """`Policy.compute_actions` for every policy at once: {pid: raw obs [B, D]} ->
         {pid: (actions [B, A], [], {"action_dist_inputs", "action_logp", "vf_preds"})}.  With `explore` actions are
-        DiagGaussian samples (noise from this group's RandomState), otherwise the distribution mean (logp of the mean)."""
+        DiagGaussian samples (noise from this group's RandomState), otherwise the distribution mean (logp of the mean).
+        Leg-coupled policy (SharedDecentralLegID): {pid: (node_idx [B], obs [B, D])} — the Tuple observation."""
         import torch
+        node = None
+        if self.coupled:
+            pid = self.policy_names[0]
+            if set(obs_by_policy) != {pid}:
+                raise BatchError(f"expected observations of {pid!r} only, got {list(obs_by_policy)}")
+            tup = obs_by_policy[pid]
+            if not isinstance(tup, (tuple, list)) or len(tup) != 2:
+                raise BatchError(f"{pid}: the observation is the tuple (node_idx [B], obs [B, D])")
+            node_h = check_node_idx(tup[0], np.asarray(tup[1]).shape[0], pid)
+            node = torch.from_numpy(node_h[None]).to(self.device)
+            obs_by_policy = {pid: tup[1]}
         obs = stack_policy_batches({p: {OBS: obs_by_policy[p]} for p in obs_by_policy}, self.policy_names, self.D, self.A, (OBS,))[OBS]
         P, B = obs.shape[:2]
         noise = self.rng.standard_normal((P, B, self.A)).astype(np.float32) if explore else np.zeros((P, B, self.A), np.float32)
         out = self.learner.compute_actions(torch.from_numpy(obs).to(self.device), torch.from_numpy(noise).to(self.device),
-                                           update_filter=update_filter)
+                                           update_filter=update_filter, **({"node_idx": node} if self.coupled else {}))
         host = {k: v.cpu().numpy() for k, v in out.items() if v is not None}
         res = {}
         for i, p in enumerate(self.policy_names):
@@ -166,6 +198,14 @@ class PPOPolicyGroup:
     def learn_on_batch(self, policy_batches: Mapping[str, Mapping[str, Any]], standardize: bool = True):
         """`RolloutWorker.learn_on_batch(MultiAgentBatch)`: one PPO update of every policy from postprocessed columns."""
         import torch
+        node = None
+        if self.coupled:      # the node-id column beside the Box part of the observation
+            pid = self.policy_names[0]
+            pb = policy_batches.get(pid, {})
+            if NODE_IDX not in pb:
+                raise BatchError(f"batch of {pid!r} lacks column {NODE_IDX!r} (the node-id part of the observation)")
+            node = check_node_idx(pb[NODE_IDX], np.asarray(pb[OBS]).shape[0], f"{pid}/{NODE_IDX}")[None]
+            policy_batches = {p: {k: v for k, v in b.items() if k != NODE_IDX} for p, b in policy_batches.items()}
         cols = stack_policy_batches(policy_batches, self.policy_names, self.D, self.A)
         R = cols[OBS].shape[1]
         used, nb = usable_rows(R, self.ppo.sgd_minibatch_size)
@@ -173,6 +213,8 @@ class PPOPolicyGroup:
         shuffle, perms = draw_minibatch_order(self.rng, P, R, self.ppo.num_sgd_iter, nb, self.shuffle_sequences)
         dev = lambda a: torch.from_numpy(a).to(self.device)
         d = {k: dev(v) for k, v in cols.items()}
+        if node is not None:
+            d[NODE_IDX] = dev(node)
         if standardize:        # StandardizeFields sees the WHOLE train batch, before the loader drops the ragged tail
             self.learner.standardize_advantages(d[ADVANTAGES])
         shuf = None if shuffle is None else dev(shuffle)
@@ -182,7 +224,8 @@ class PPOPolicyGroup:
                  for k, v in d.items()}
             shuf = None
         stats = self.learner.learn_on_batch(d[OBS], d[ACTIONS], d[ACTION_DIST_INPUTS], d[ACTION_LOGP], d[VF_PREDS],
-                                            d[ADVANTAGES], d[VALUE_TARGETS], dev(perms), shuf, standardize=False)
+                                            d[ADVANTAGES], d[VALUE_TARGETS], dev(perms), shuf, standardize=False,
+                                            node_idx=d.get(NODE_IDX))
         self.num_steps_trained += used
         return {p: {"learner_stats": stats[i]} for i, p in enumerate(self.policy_names)}
 
@@ -190,12 +233,25 @@ class PPOPolicyGroup:
     def get_weights(self) -> Dict[str, Dict[str, np.ndarray]]:
         from .checkpoint import theta_to_variables
         th = self.learner.theta.cpu().numpy()
-        return {p: theta_to_variables(p, th[i], self.D, self.A) for i, p in enumerate(self.policy_names)}
+        NPf = self.learner.NPf
+        out = {p: theta_to_variables(p, th[i, :NPf], self.D, self.A) for i, p in enumerate(self.policy_names)}
+        if self.coupled:      # the registration order of the ModelV2 class: the 12 FCNet variables, then the table
+            for i, p in enumerate(self.policy_names):
+                out[p][f"{p}/leg_coupling"] = th[i, NPf:].reshape(4, 2).copy()
+        return out
 
     def set_weights(self, weights: Mapping[str, Mapping[str, np.ndarray]]) -> None:
         import torch
         from .checkpoint import variables_to_theta
         th = np.stack([variables_to_theta(p, weights[p], self.D, self.A) for p in self.policy_names]).astype(np.float32)
+        if self.coupled:
+            tabs = []
+            for p in self.policy_names:
+                t = np.asarray(weights[p].get(f"{p}/leg_coupling"), dtype=np.float32) if f"{p}/leg_coupling" in weights[p] else None
+                if t is None or t.shape != (4, 2):
+                    raise ValueError(f"{p}: set_weights needs '{p}/leg_coupling' of shape (4, 2)")
+                tabs.append(t.reshape(-1))
+            th = np.concatenate([th, np.stack(tabs)], axis=1)
         self.learner.theta.copy_(torch.from_numpy(th).to(self.device))
 
     # ---- curriculum callback ------------------------------------------------------------------------------------------

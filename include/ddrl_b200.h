@@ -444,6 +444,40 @@ int ddrl_ppo_train_step_tc(const void* tc_img, const float* obs, const float* ac
                            float* grad_part, double* stat_part, int* status, const ddrl_sgd_tail* tail,
                            void* stream);
 
+/* Leg-coupled SGD steps: the policy of QuantrupedMultiEnv_SharedDecentralLegID, model "cup" = FCNet + LegCoupling
+ * (models/__init__.py:7-13, models/coupling_net_glorot_uniform_init.py:11-30,135; ModelV2 class
+ * FullyConnectedNetwork_Coupling_GlorotUniformInitializer).  Same batch arrays, minibatch selection and partial / stat
+ * outputs as ddrl_ppo_train_step / ddrl_ppo_train_step_tc, with:
+ *   logits[r][i] = pre[r][i] * coupling[node_id[r]][i]   (i < 2: the mean logits; the log-std half and the value are not scaled)
+ *   the PPO loss taken of the coupled logits (old_logits are the coupled logits the actions were sampled from);
+ *   d pre[r][i] = d logits[r][i] * coupling[node_id[r]][i];  d coupling[n][i] = sum_{r: node_id[r] = n} d logits[r][i] * pre[r][i]
+ *   node_id [P][R] int32 in 0..3 (the agent's position in agent_names: FL, HL, HR, FR), in the batch's row order;
+ *   theta [P][NP + 8]: the 12 FCNet variables in checkpoint order (NP = ddrl_fcnet_num_params(D, 2)), then leg_coupling [4][2]
+ *     row-major — the registration order of the ModelV2 class; the coupling table is read from it every step;
+ *   grad_part [P][G][(NP + 8 + 3) & ~3]; the fused tail is REQUIRED (tail->theta == theta, m / v / grad [P][NP + 8]) and
+ *     clips + steps all NP + 8 parameters (the packed weight images get the first NP);
+ *   A = 2 and P = 1 only (the reference builds this model as one shared policy; a wider action or several policies return
+ *   DDRL_E_BADARG); no LL tail, no thread-block clusters (DDRL_E_BADARG).
+ * A node id outside 0..3 read on the device sets *status |= DDRL_STATUS_BAD_NODE (the row is then coupled as node id & 3).
+ * ddrl_ppo_train_step_coupled is the FP32 step (nsteps <= 1; *tail->status, REQUIRED, receives the flag; weights from the
+ * packed image img, ddrl_fcnet_pack of the first NP entries); ddrl_ppo_train_step_tc_coupled the ping-pong tensor-core step
+ * (tail->nsteps consecutive steps per launch; D in {19, 20}; status REQUIRED; weights from the tensor-core image tc_img,
+ * ddrl_fcnet_tc_pack of the first NP).  A NULL status is rejected with DDRL_E_BADARG, so a bad node id cannot go unreported. */
+#define DDRL_STATUS_BAD_NODE 128
+int ddrl_ppo_train_step_coupled(const float* theta, const float* img, const int32_t* node_id, const float* obs,
+                                const float* actions, const float* old_logits, const float* old_logp, const float* vf_preds,
+                                const float* adv, const float* vtarg, int P, int64_t R, int D, int A, int MB,
+                                const int32_t* mb_perm, int64_t perm_stride, const int32_t* step_ctr, const float* kl_coeff,
+                                const ddrl_ppo_hyper* hyper, int ctas_per_policy, float* grad_part, double* stat_part,
+                                const ddrl_sgd_tail* tail, void* stream);
+int ddrl_ppo_train_step_tc_coupled(const void* tc_img, const float* theta, const int32_t* node_id, const float* obs,
+                                   const float* actions, const float* old_logits, const float* old_logp,
+                                   const float* vf_preds, const float* adv, const float* vtarg, int P, int64_t R, int D,
+                                   int A, int MB, const int32_t* mb_perm, int64_t perm_stride, const int32_t* step_ctr,
+                                   const float* kl_coeff, const ddrl_ppo_hyper* hyper, int ctas_per_policy,
+                                   float* grad_part, double* stat_part, int* status, const ddrl_sgd_tail* tail,
+                                   void* stream);
+
 /* Diagnostic: one tcgen05 (UMMA) GEMM through TMEM with the chunked shared-memory operand layout the tensor-core
  * training step uses (csrc/umma.cuh): D[m][n] = sum_k A(m,k) B(n,k), m < M (64 or 128), A(m,k) = A[m][k] (a_mn = 0, K-major) or
  * A[k][m] (a_mn = 1, MN-major view); B alike; split != 0 -> fp16 (hi, lo) operand split with three products.
