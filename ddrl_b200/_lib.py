@@ -82,6 +82,8 @@ PROTOTYPES = {
                                            c_stream]),
     "ddrl_graphnet_forward": (C.c_int, [c_f32p, c_i32p, c_f32p, c_f32p, C.c_int64, C.c_int, c_f32p, c_f32p,
                                         c_stream]),
+    "ddrl_graphnet_act": (C.c_int, [c_f32p, c_i32p, c_f32p, c_f32p, c_f32p, C.c_int64, C.c_int, c_f32p, c_f32p, c_f32p,
+                                    c_f32p, c_stream]),
     "ddrl_graphnet_backward": (C.c_int, [c_f32p, c_i32p, c_f32p, c_f32p, c_f32p, c_f32p, C.c_int64, C.c_int,
                                          C.c_int, c_f32p, c_stream]),
     "ddrl_gcn_forward": (C.c_int, [c_f32p, c_f32p, c_f32p, c_f32p, C.c_int64, C.c_int, C.c_int, C.c_int, c_f32p,

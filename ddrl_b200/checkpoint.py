@@ -238,6 +238,10 @@ def save_rllib_checkpoint(path: str, ckpt: Checkpoint) -> None:
 
 # ---- learner <-> checkpoint ---------------------------------------------------------------------------------------------
 def _reject_coupled(learner) -> None:
+    from .learner import GraphNetLearner
+    if isinstance(learner, GraphNetLearner):
+        raise ValueError("checkpoints of the shared GraphNet policy are not supported: no GraphNet checkpoint was published, "
+                         "so none pins the format; use GraphNetPolicyGroup.get_weights / set_weights")
     if getattr(learner, "coupled", False):
         raise ValueError("checkpoints of leg-coupled ('cup') policies are not supported: no reference checkpoint pins the "
                          "naming of the leg_coupling variable; use get_weights / set_weights")

@@ -53,6 +53,27 @@ __host__ __device__ inline FcOffsets fc_offsets(int D, int A) {
     return o;
 }
 
+constexpr float kLog2Pi = 1.8378770664093453f;
+
+// RLlib DiagGaussian (models/tf/tf_action_dist.py) sample of row r: action[r][i] = mean + exp(log_std) * eps[r][i] for
+// logits[r] = (mean | log_std) [2A]; returns logp(action) = -0.5 sum z^2 - 0.5 log(2 pi) A - sum log_std,
+// z = (action - mean) / exp(log_std), summed in the order i = 0..A-1.  dg_sample_kernel and graphnet_fwd_warp_kernel<true>
+// both call it, so their actions and logp are bit-identical.
+__device__ __forceinline__ float dg_sample_row(const float* __restrict__ logits, const float* __restrict__ eps, int64_t r,
+                                               int A, float* __restrict__ action) {
+    float sz2 = 0.f, sls = 0.f;
+    for (int i = 0; i < A; ++i) {
+        const float mu = logits[r * 2 * A + i], ls = logits[r * 2 * A + A + i];
+        const float sd = expf(ls);
+        const float a = mu + sd * eps[r * A + i];
+        const float z = (a - mu) / sd;
+        sz2 = fmaf(z, z, sz2);
+        sls += ls;
+        action[r * A + i] = a;
+    }
+    return -0.5f * sz2 - 0.5f * kLog2Pi * (float)A - sls;
+}
+
 __device__ __forceinline__ double warp_sum(double v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

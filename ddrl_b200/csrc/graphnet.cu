@@ -325,10 +325,14 @@ constexpr int GWF_WO = GMAXO + 1;             // stride of the head matrix: lane
 constexpr int GWF_SMEM_FLOATS = GE * GF * GH + GF * GH + 2 * GH * GH + GH * GWF_WO + GMAXO + GWF_WARPS * GWF_ROW +
                                 GWF_WARPS * GN * GH;
 
+// SAMPLE (ddrl_graphnet_act): the actor warps also draw the row's DiagGaussian action from eps [B][A] -> action [B][A],
+// logp [B] with dg_sample_kernel's row body (bit-identical to ddrl_dg_sample on the logits written here).
+template <bool SAMPLE>
 __global__ void __launch_bounds__(GWF_NT, 3)
 graphnet_fwd_warp_kernel(const float* __restrict__ theta, const int32_t* __restrict__ node_idx,
                          const float* __restrict__ state, const float* __restrict__ adj, int64_t B, int A,
-                         float* __restrict__ logits, float* __restrict__ value) {
+                         float* __restrict__ logits, float* __restrict__ value, const float* __restrict__ eps,
+                         float* __restrict__ action, float* __restrict__ logp) {
     extern __shared__ __align__(16) float gsm[];
     float* sWe = gsm;                           // [GE][GF*GH]
     float* sbe = sWe + GE * GF * GH;            // [GF*GH]
@@ -451,8 +455,13 @@ graphnet_fwd_warp_kernel(const float* __restrict__ theta, const int32_t* __restr
                 if (lane == q) {
                     v += sbo[q];
                     if (net == 0) logits[b * O + q] = v; else value[b] = v;
+                    if (SAMPLE) sRow[GH + q] = v;   // sRow[GH..) is free since the encoder's barrier (the MPNN uses [0, GH))
                 }
             }
+        }
+        if (SAMPLE && net == 0) {
+            __syncwarp();
+            if (lane == 0) logp[b] = dg_sample_row(sRow + GH, eps + b * A, 0, A, action + b * A);
         }
         __syncwarp();      // every lane is done with sRow / sX before the next row overwrites them
     }
@@ -849,35 +858,55 @@ static int gn_ctas(int64_t B) {
     return (int)std::max<int64_t>(1, std::min<int64_t>(B, sms / 2));
 }
 
+// One launch of graphnet_fwd_warp_kernel<SAMPLE> (forward schedule 1).  B >= 1.
+template <bool SAMPLE>
+static int launch_fwd_warp(const float* theta, const int32_t* node_idx, const float* state, const float* adj,
+                           const float* eps, int64_t B, int A, float* logits, float* value, float* action, float* logp,
+                           void* stream, const char* who) {
+    static bool attr_set = false;       // per process and instantiation; the attribute is sticky for the function
+    const size_t smem = (size_t)GWF_SMEM_FLOATS * sizeof(float);
+    if (!attr_set) {
+        cudaError_t e = cudaFuncSetAttribute(graphnet_fwd_warp_kernel<SAMPLE>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                             (int)smem);
+        DDRL_REQUIRE(e == cudaSuccess, DDRL_E_CUDA, "%s: cudaFuncSetAttribute: %s", who, cudaGetErrorString(e));
+        attr_set = true;
+    }
+    int dev = 0, sms = 148;
+    if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    // 3 CTAs per SM, the two nets side by side: (3 * sms / 2) CTAs per net, never more than one warp per row
+    const int gx = (int)std::max<int64_t>(1, std::min<int64_t>((B + GWF_WARPS - 1) / GWF_WARPS, 3 * sms / 2));
+    graphnet_fwd_warp_kernel<SAMPLE><<<dim3(gx, 2), GWF_NT, smem, (cudaStream_t)stream>>>(theta, node_idx, state, adj, B, A,
+                                                                                         logits, value, eps, action, logp);
+    DDRL_CHECK_LAUNCH(who);
+    return DDRL_OK;
+}
+
 extern "C" int ddrl_graphnet_forward(const float* theta, const int32_t* node_idx, const float* state, const float* adj,
                                      int64_t B, int A, float* logits, float* value, void* stream) {
     DDRL_REQUIRE(theta && node_idx && state && adj && logits && value && B >= 0, DDRL_E_BADARG,
                  "graphnet_forward: null pointer or bad B");
     DDRL_REQUIRE(A >= 1 && A <= DDRL_MAX_ACT, DDRL_E_UNSUPPORTED_SHAPE, "graphnet_forward: unsupported A=%d", A);
     if (B == 0) return DDRL_OK;
-    if (gn_fwd_variant() == 1) {
-        static bool attr_set = false;       // per process; the attribute is sticky for the function
-        const size_t smem = (size_t)GWF_SMEM_FLOATS * sizeof(float);
-        if (!attr_set) {
-            cudaError_t e = cudaFuncSetAttribute(graphnet_fwd_warp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-            DDRL_REQUIRE(e == cudaSuccess, DDRL_E_CUDA, "graphnet_forward: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-            attr_set = true;
-        }
-        int dev = 0, sms = 148;
-        if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        // 3 CTAs per SM, the two nets side by side: (3 * sms / 2) CTAs per net, never more than one warp per row
-        const int gx = (int)std::max<int64_t>(1, std::min<int64_t>((B + GWF_WARPS - 1) / GWF_WARPS, 3 * sms / 2));
-        graphnet_fwd_warp_kernel<<<dim3(gx, 2), GWF_NT, smem, (cudaStream_t)stream>>>(theta, node_idx, state, adj, B, A, logits,
-                                                                                      value);
-        DDRL_CHECK_LAUNCH("graphnet_forward");
-        return DDRL_OK;
-    }
+    if (gn_fwd_variant() == 1)
+        return launch_fwd_warp<false>(theta, node_idx, state, adj, nullptr, B, A, logits, value, nullptr, nullptr, stream,
+                                      "graphnet_forward");
     graphnet_kernel<false><<<dim3(gn_ctas(B), 2), GT2, 0, (cudaStream_t)stream>>>(theta, node_idx, state, adj, nullptr,
                                                                                  nullptr, B, A, logits, value, nullptr);
     DDRL_CHECK_LAUNCH("graphnet_forward");
     return DDRL_OK;
 }
 
+extern "C" int ddrl_graphnet_act(const float* theta, const int32_t* node_idx, const float* state, const float* adj,
+                                 const float* eps, int64_t B, int A, float* logits, float* value, float* action, float* logp,
+                                 void* stream) {
+    DDRL_REQUIRE(theta && node_idx && state && adj && eps && logits && value && action && logp && B >= 0, DDRL_E_BADARG,
+                 "graphnet_act: null pointer or bad B");
+    DDRL_REQUIRE(A >= 1 && A <= DDRL_MAX_ACT, DDRL_E_UNSUPPORTED_SHAPE, "graphnet_act: unsupported A=%d", A);
+    if (B == 0) return DDRL_OK;
+    return launch_fwd_warp<true>(theta, node_idx, state, adj, eps, B, A, logits, value, action, logp, stream, "graphnet_act");
+}
+
+// The variant selects the schedule of ddrl_graphnet_forward only; ddrl_graphnet_act always runs schedule 1.
 extern "C" int ddrl_graphnet_set_variant(int variant) {
     DDRL_REQUIRE(variant >= -1 && variant <= 1, DDRL_E_BADARG, "graphnet_set_variant: variant must be -1 (default), 0 or 1");
     g_gn_fwd_variant = variant;

@@ -8,7 +8,6 @@
 
 namespace ddrl {
 
-constexpr float kLog2Pi = 1.8378770664093453f;
 constexpr float kHalfLog2PiE = 1.4189385332046727f;  // 0.5*log(2*pi*e)
 
 // Policy part.  logits[0..2A) = (mean | log_std).  Writes dl[0..2A) = scale * d(-surr + klc*KL - ent_coeff*H)/dlogits

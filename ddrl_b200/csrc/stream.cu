@@ -479,19 +479,8 @@ __global__ void concat_actions_kernel(const float* __restrict__ act, const int32
 // DiagGaussian sample + logp (RLlib models/tf/tf_action_dist.py) for models without a fused epilogue.
 __global__ void dg_sample_kernel(const float* __restrict__ logits, const float* __restrict__ eps, int64_t R, int A,
                                  float* __restrict__ action, float* __restrict__ logp) {
-    for (int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; r < R; r += (int64_t)gridDim.x * blockDim.x) {
-        float sz2 = 0.f, sls = 0.f;
-        for (int i = 0; i < A; ++i) {
-            const float mu = logits[r * 2 * A + i], ls = logits[r * 2 * A + A + i];
-            const float sd = expf(ls);
-            const float a = mu + sd * eps[r * A + i];
-            const float z = (a - mu) / sd;
-            sz2 = fmaf(z, z, sz2);
-            sls += ls;
-            action[r * A + i] = a;
-        }
-        logp[r] = -0.5f * sz2 - 0.5f * kLog2Pi * (float)A - sls;
-    }
+    for (int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; r < R; r += (int64_t)gridDim.x * blockDim.x)
+        logp[r] = dg_sample_row(logits, eps, r, A, action);
 }
 
 __global__ void leg_coupling_kernel(float* __restrict__ logits, const int32_t* __restrict__ node_id,

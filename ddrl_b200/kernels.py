@@ -244,6 +244,32 @@ def graphnet_forward(theta, node_idx, state, adj, A: int, out: Optional[Tuple[to
     return logits, value
 
 
+def graphnet_act(theta, node_idx, state, adj, eps, A: int, out: Optional[Tuple[torch.Tensor, ...]] = None):
+    """GraphNet forward + DiagGaussian sample in ONE launch: theta [NP], node_idx [B] i32, state [B,4,23], adj [B,4,4],
+    eps [B,A] -> logits [B,2A], value [B], action [B,A], logp [B] (written into ``out`` = (logits, value, action, logp) when
+    given).  Bit-identical to ``graphnet_forward`` under forward variant 1 followed by ``dg_sample``."""
+    B = state.shape[0]
+    f32 = torch.float32
+    shapes = ((B, 2 * A), (B,), (B, A), (B,))
+    if out is not None:
+        if len(out) != 4 or any(tuple(t.shape) != s for t, s in zip(out, shapes)):
+            raise DDRLError(f"graphnet_act: out shapes {[tuple(t.shape) for t in out]} != {list(shapes)}")
+        logits, value, action, logp = out
+    else:
+        logits, value, action, logp = (torch.empty(s, dtype=f32, device=state.device) for s in shapes)
+    if tuple(state.shape[1:]) != (GN_NODES, GN_FEATS + GN_ENC_IN) or tuple(adj.shape[1:]) != (GN_NODES, GN_NODES):
+        raise DDRLError(f"graphnet: state {tuple(state.shape)} / adj {tuple(adj.shape)} must be [B,4,23] / [B,4,4]")
+    if tuple(eps.shape) != (B, A):
+        raise DDRLError(f"graphnet_act: eps {tuple(eps.shape)} must be [{B}, {A}]")
+    if theta.numel() != graphnet_num_params(2 * A):
+        raise DDRLError(f"graphnet: theta has {theta.numel()} params, expected {graphnet_num_params(2 * A)}")
+    _lib.check(_lib.load().ddrl_graphnet_act(_p(theta, f32, "theta"), _p(node_idx, torch.int32, "node_idx"),
+                                             _p(state, f32, "state"), _p(adj, f32, "adj"), _p(eps, f32, "eps"), B, A,
+                                             _p(logits, f32, "logits"), _p(value, f32, "value"), _p(action, f32, "action"),
+                                             _p(logp, f32, "logp"), _stream()), "graphnet_act")
+    return logits, value, action, logp
+
+
 def graphnet_backward(theta, node_idx, state, adj, dlogits, dvalue, A: int, ctas: Optional[int] = None):
     B = state.shape[0]
     f32 = torch.float32

@@ -99,6 +99,19 @@ class _LearnerBase:
                     c.grad_clip, self.sync_ws, self.gnorm, self.step_ctr, img, getattr(self, "D", 0) if img is not None else 0,
                     self.A if img is not None else 0, tc_img=getattr(self, "tc_img", None))
 
+    def standardize_advantages(self, adv: torch.Tensor) -> torch.Tensor:
+        """StandardizeFields(["advantages"]) in place on adv [P,R] (float32, CUDA): per policy (adv - mean) / max(1e-4, std)
+        over ALL rows of the train batch (all ranks' rows at world > 1).  The three moments are float64 torch reductions
+        (plumbing); the rescale is `ddrl_adv_standardize`."""
+        P = adv.shape[0]
+        a64 = adv.reshape(P, -1).double()
+        moments = torch.stack([torch.full((P,), float(a64.shape[1]), dtype=torch.float64, device=adv.device),
+                               a64.sum(dim=1), (a64 * a64).sum(dim=1)], dim=1).contiguous()
+        if self.world > 1:
+            self.dist.all_reduce(moments)
+        K.adv_standardize(adv, moments)
+        return adv
+
     def _update_kl(self, stats: List[Dict[str, float]]):
         # KLCoeffMixin.update_kl (RLlib 1.0.1): x1.5 if kl > 2*target, x0.5 if kl < 0.5*target
         for p, s in enumerate(stats):
@@ -622,19 +635,6 @@ class FCNetLearner(_LearnerBase):
         src = {n_: b[n_ + ("_s" if shuffle is not None else "")] for n_ in names}
         return self._sgd_phase(b, src, "s" if shuffle is not None else "u", perms, R, R, 1)
 
-    def standardize_advantages(self, adv: torch.Tensor) -> torch.Tensor:
-        """StandardizeFields(["advantages"]) in place on adv [P,R] (float32, CUDA): per policy (adv - mean) / max(1e-4, std)
-        over ALL rows of the train batch (all ranks' rows at world > 1).  The three moments are float64 torch reductions
-        (plumbing); the rescale is `ddrl_adv_standardize`."""
-        P = adv.shape[0]
-        a64 = adv.reshape(P, -1).double()
-        moments = torch.stack([torch.full((P,), float(a64.shape[1]), dtype=torch.float64, device=adv.device),
-                               a64.sum(dim=1), (a64 * a64).sum(dim=1)], dim=1).contiguous()
-        if self.world > 1:
-            self.dist.all_reduce(moments)
-        K.adv_standardize(adv, moments)
-        return adv
-
     def refresh_filter_norm(self):
         """Recompute the normalisation table (mean, 1/(std+1e-8)) from filt_n / filt_M / filt_S — after the state was
         written from outside (checkpoint import)."""
@@ -699,6 +699,24 @@ class GraphNetLearner(_LearnerBase):
     def forward(self, node_idx, state, adj):
         return K.graphnet_forward(self.theta.reshape(-1), node_idx, state, adj, self.A)
 
+    # ---- plain inference (sampler side) ---------------------------------------------------------------------
+    def compute_actions(self, node_idx: torch.Tensor, state: torch.Tensor, adj: torch.Tensor,
+                        eps: Optional[torch.Tensor] = None):
+        """node_idx [B] int32 (0..3: FL, HL, HR, FR), state [B,4,23], adj [B,4,4], eps [B,A] or None ->
+        dict(logits, value[, action, logp]).  With eps ONE launch (`ddrl_graphnet_act`: forward + DiagGaussian sample),
+        without it `ddrl_graphnet_forward`.  A node id outside 0..3 raises (the kernels would clamp it)."""
+        B = state.shape[0]
+        if tuple(node_idx.shape) != (B,) or node_idx.dtype != torch.int32 or not node_idx.is_cuda:
+            raise DDRLError(f"compute_actions: node_idx must be an int32 CUDA tensor of shape {(B,)}")
+        if int(((node_idx < 0) | (node_idx > 3)).sum().item()):
+            raise DDRLError("compute_actions: node ids must be 0..3 (FL, HL, HR, FR)")
+        th = self.theta.reshape(-1)
+        if eps is None:
+            logits, value = K.graphnet_forward(th, node_idx, state, adj, self.A)
+            return {"logits": logits, "value": value}
+        logits, value, action, logp = K.graphnet_act(th, node_idx, state, adj, eps, self.A)
+        return {"logits": logits, "value": value, "action": action, "logp": logp}
+
     def learn_on_rollout(self, node_idx, state, adj, boot_node_idx, boot_state, boot_adj, rewards, dones, eps, perms,
                          shuffle=None, cols_per_env: int = 4) -> List[Dict[str, float]]:
         """node_idx [T,C] i32, state [T,C,4,23], adj [T,C,4,4], boot_* the same without T, rewards [T,C],
@@ -729,12 +747,7 @@ class GraphNetLearner(_LearnerBase):
         R = state.shape[0]
         adv = advantages.reshape(1, R).clone()
         if standardize:
-            a64 = adv.double()
-            moments = torch.stack([torch.full((1,), float(R), dtype=torch.float64, device=adv.device), a64.sum(dim=1),
-                                   (a64 * a64).sum(dim=1)], dim=1).contiguous()
-            if self.world > 1:
-                self.dist.all_reduce(moments)
-            K.adv_standardize(adv, moments)
+            self.standardize_advantages(adv)
         cols = {"idx": node_idx.reshape(R), "st": state, "adj": adj, "act": actions, "logits": action_dist_inputs,
                 "logp": action_logp, "value": vf_preds, "adv": adv.reshape(R), "vtarg": value_targets}
         for name, t in cols.items():

@@ -295,10 +295,18 @@ int ddrl_graphnet_num_params(int num_outputs);
 int ddrl_graphnet_forward(const float* theta, const int32_t* node_idx, const float* state,
                           const float* adj, int64_t B, int A, float* logits, float* value,
                           void* stream);
-/* Forward schedule (A/B timing and tests): 0 = one row per CTA, 1 = one row per warp with the weights in shared memory,
- * -1 = library default (overridable by the environment variable DDRL_GN_FWD_VARIANT=0|1).  Same results up to the FP32
- * summation order. */
+/* Forward schedule (A/B timing and tests) of ddrl_graphnet_forward: 0 = one row per CTA, 1 = one row per warp with the
+ * weights in shared memory, -1 = library default (overridable by the environment variable DDRL_GN_FWD_VARIANT=0|1).  Same
+ * results up to the FP32 summation order.  ddrl_graphnet_act always runs the row-per-warp schedule. */
 int ddrl_graphnet_set_variant(int variant);
+/* GraphNet inference + DiagGaussian sampling in ONE launch (the sampler-side call of the shared graph policy):
+ *   theta, node_idx [B], state [B][4][23], adj [B][4][4] as in ddrl_graphnet_forward, eps [B][A] (all required)
+ *   -> logits [B][2A], value [B], action [B][A] = mean + exp(log_std) * eps, logp [B] (the logp of that action).
+ * logits / value are bit-identical to ddrl_graphnet_forward under forward schedule 1 (one warp per row); action / logp
+ * are bit-identical to ddrl_dg_sample applied to those logits. */
+int ddrl_graphnet_act(const float* theta, const int32_t* node_idx, const float* state, const float* adj,
+                      const float* eps, int64_t B, int A, float* logits, float* value, float* action, float* logp,
+                      void* stream);
 /* Backward of the wrapper w.r.t. theta from dlogits [B][2A], dvalue [B]:
  *   grad_part [G][NPs] per-CTA partials, NPs = (NP+3)&~3 (reduce with ddrl_grad_reduce(P=1)); G = ctas. */
 int ddrl_graphnet_backward(const float* theta, const int32_t* node_idx, const float* state,
