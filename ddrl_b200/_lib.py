@@ -96,6 +96,11 @@ PROTOTYPES = {
     "ddrl_fcnet_tc_image_bytes": (C.c_int, [C.c_int, C.c_int]),
     "ddrl_fcnet_forward_tc": (C.c_int, [C.c_void_p, c_f32p, c_f64p, C.c_float, C.c_int, C.c_int64, C.c_int, C.c_int,
                                          c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_i32p, c_stream]),
+    "ddrl_fcnet_forward_coupled": (C.c_int, [c_f32p, c_f32p, c_i32p, c_f32p, c_f32p, c_f64p, C.c_float, C.c_int, C.c_int64,
+                                             C.c_int, C.c_int, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_i32p, c_stream]),
+    "ddrl_fcnet_forward_tc_coupled": (C.c_int, [C.c_void_p, c_i32p, c_f32p, c_f32p, c_f64p, C.c_float, C.c_int, C.c_int64,
+                                                C.c_int, C.c_int, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_i32p,
+                                                c_stream]),
     "ddrl_tc_set_variant": (C.c_int, [C.c_int]),
     "ddrl_mpnn2_forward": (C.c_int, [c_f32p] * 5 + [C.c_int64, C.c_int, C.c_int, C.c_int, c_f32p, c_stream]),
     "ddrl_gat1_forward": (C.c_int, [c_f32p] * 5 + [C.c_int64, C.c_int, C.c_int, C.c_int, c_f32p, c_stream]),

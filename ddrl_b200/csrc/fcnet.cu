@@ -212,12 +212,17 @@ __device__ __forceinline__ void load_x_tile(float* sm, const FcSmem& L, const fl
 
 // =================================================================================================
 // K1: grouped forward (+filter-normalise prologue, +DiagGaussian sample/logp epilogue)
+// CUP = true (ddrl_fcnet_forward_coupled): the leg-coupled policy of SharedDecentralLegID — row r's mean logits are
+// multiplied by coupling[node_id[r]] (one rounding, as leg_coupling_kernel) before they are stored and sampled from; an id
+// outside 0..3 sets DDRL_STATUS_BAD_NODE and is coupled as id & 3.  The three trailing parameters are unused by <false>.
 // =================================================================================================
+template <bool CUP>
 __global__ void __launch_bounds__(NT, 1)
 fcnet_forward_kernel(const float* __restrict__ theta, const float* __restrict__ img, const float* __restrict__ obs,
                      const double* __restrict__ norm, float clip, int64_t R, int D, int A, float* __restrict__ obs_out,
                      float* __restrict__ logits, float* __restrict__ value, const float* __restrict__ eps,
-                     float* __restrict__ action, float* __restrict__ logp) {
+                     float* __restrict__ action, float* __restrict__ logp, const int32_t* __restrict__ node_id,
+                     const float* __restrict__ coupling, int* __restrict__ status) {
     extern __shared__ __align__(16) float sm[];
     const int p = blockIdx.y;
     const FcSmem L = fc_smem(D, A, norm != nullptr);
@@ -247,6 +252,13 @@ fcnet_forward_kernel(const float* __restrict__ theta, const float* __restrict__ 
         __syncthreads();
         forward_tile(sm, L, D, A, nrows);
         // epilogue ---------------------------------------------------------------------------------
+        if (CUP && tid < nrows) {      // LegCoupling of row tid (this thread samples it below: no barrier in between)
+            int nd = node_id[(int64_t)p * R + row0 + tid];
+            if ((unsigned)nd > 3u) { atomicOr(status, DDRL_STATUS_BAD_NODE); nd &= 3; }
+            float* mrow = sm + L.out + tid * LDD;
+            mrow[0] = __fmul_rn(mrow[0], __ldg(coupling + 2 * nd));      // (never contracted into the sample's FMA)
+            mrow[1] = __fmul_rn(mrow[1], __ldg(coupling + 2 * nd + 1));
+        }
         if (eps && tid < nrows) {
             const int r = tid;
             const int64_t gr = (int64_t)p * R + row0 + r;
@@ -262,7 +274,7 @@ fcnet_forward_kernel(const float* __restrict__ theta, const float* __restrict__ 
             }
             logp[gr] = -0.5f * sz2 - 0.5f * kLog2Pi * (float)A - sls;
         }
-        if (eps) __syncthreads();
+        if (CUP || eps) __syncthreads();
         if (logits)
             for (int i = tid; i < nrows * A2; i += NT) {
                 const int r = i / A2, c = i - r * A2;
@@ -426,13 +438,38 @@ extern "C" int ddrl_fcnet_forward(const float* theta, const float* img, const fl
     const size_t smem = (size_t)L.total * sizeof(float);
     DDRL_REQUIRE(smem <= 227 * 1024, DDRL_E_UNSUPPORTED_SHAPE, "fcnet_forward: shared memory %zu > 227 KB", smem);
     static bool attr_set = false;
-    if (int rc = set_smem_attr((const void*)fcnet_forward_kernel, &attr_set, "fcnet_forward")) return rc;
+    if (int rc = set_smem_attr((const void*)fcnet_forward_kernel<false>, &attr_set, "fcnet_forward")) return rc;
     const int64_t ntiles = (R + TM - 1) / TM;
     const int per_policy = (int)std::min<int64_t>(ntiles, std::max(1, num_sms() / P));
     dim3 grid(per_policy, P);
-    fcnet_forward_kernel<<<grid, NT, smem, (cudaStream_t)stream>>>(theta, img, obs, norm, clip, R, D, A, obs_out,
-                                                                   logits, value, eps, action, logp);
+    fcnet_forward_kernel<false><<<grid, NT, smem, (cudaStream_t)stream>>>(theta, img, obs, norm, clip, R, D, A, obs_out,
+                                                                          logits, value, eps, action, logp, nullptr,
+                                                                          nullptr, nullptr);
     DDRL_CHECK_LAUNCH("fcnet_forward");
+    return DDRL_OK;
+}
+
+extern "C" int ddrl_fcnet_forward_coupled(const float* theta, const float* img, const int32_t* node_id, const float* coupling,
+                                          const float* obs, const double* norm, float clip, int P, int64_t R, int D, int A,
+                                          float* obs_out, float* logits, float* value, const float* eps, float* action,
+                                          float* logp, int* status, void* stream) {
+    DDRL_REQUIRE((theta || img) && node_id && coupling && obs && status && R >= 0, DDRL_E_BADARG,
+                 "fcnet_forward_coupled: null theta/node_id/coupling/obs/status or bad R");
+    DDRL_REQUIRE(A == 2, DDRL_E_BADARG, "fcnet_forward_coupled: LegCoupling needs A = 2 (num_outputs == 4), got A=%d", A);
+    DDRL_REQUIRE(P == 1, DDRL_E_BADARG, "fcnet_forward_coupled: the coupled model is one shared policy (P = 1), got P=%d", P);
+    DDRL_REQUIRE(D >= 1 && D <= DDRL_MAX_OBS, DDRL_E_UNSUPPORTED_SHAPE, "fcnet_forward_coupled: unsupported D=%d", D);
+    DDRL_REQUIRE(!eps || (action && logp), DDRL_E_BADARG, "fcnet_forward_coupled: eps given without action/logp outputs");
+    if (R == 0) return DDRL_OK;
+    const FcSmem L = fc_smem(D, A, norm != nullptr);
+    const size_t smem = (size_t)L.total * sizeof(float);
+    DDRL_REQUIRE(smem <= 227 * 1024, DDRL_E_UNSUPPORTED_SHAPE, "fcnet_forward_coupled: shared memory %zu > 227 KB", smem);
+    static bool attr_set = false;
+    if (int rc = set_smem_attr((const void*)fcnet_forward_kernel<true>, &attr_set, "fcnet_forward_coupled")) return rc;
+    const int64_t ntiles = (R + TM - 1) / TM;
+    const int per_policy = (int)std::min<int64_t>(ntiles, std::max(1, num_sms()));
+    fcnet_forward_kernel<true><<<dim3(per_policy, 1), NT, smem, (cudaStream_t)stream>>>(
+        theta, img, obs, norm, clip, R, D, A, obs_out, logits, value, eps, action, logp, node_id, coupling, status);
+    DDRL_CHECK_LAUNCH("fcnet_forward_coupled");
     return DDRL_OK;
 }
 

@@ -807,3 +807,33 @@ extern "C" int ddrl_fcnet_forward_tc(const void* tc_img_p, const float* obs, con
     return DDRL_OK;
 }
 
+extern "C" int ddrl_fcnet_forward_tc_coupled(const void* tc_img_p, const int32_t* node_id, const float* coupling, const float* obs,
+                                             const double* norm, float clip, int P, int64_t R, int D, int A, float* obs_out,
+                                             float* logits, float* value, const float* eps, float* action, float* logp, int* status,
+                                             void* stream) {
+    DDRL_REQUIRE(tc_img_p && node_id && coupling && obs && status && R >= 0, DDRL_E_BADARG,
+                 "fcnet_forward_tc_coupled: null tc_img/node_id/coupling/obs/status or bad R");
+    DDRL_REQUIRE(A == 2, DDRL_E_BADARG, "fcnet_forward_tc_coupled: LegCoupling needs A = 2 (num_outputs == 4), got A=%d", A);
+    DDRL_REQUIRE(P == 1, DDRL_E_BADARG, "fcnet_forward_tc_coupled: the coupled model is one shared policy (P = 1), got P=%d", P);
+    DDRL_REQUIRE(!eps || (action && logp), DDRL_E_BADARG, "fcnet_forward_tc_coupled: eps given without action / logp outputs");
+    DDRL_REQUIRE(D == 19 || D == 20, DDRL_E_UNSUPPORTED_SHAPE,
+                 "fcnet_forward_tc_coupled: instantiated for SharedDecentralLegID (D = 19 or 20), got D=%d", D);
+    DDRL_REQUIRE(R <= 0x7fffffff, DDRL_E_UNSUPPORTED_SHAPE, "fcnet_forward_tc_coupled: R must fit 31 bits");
+    DDRL_REQUIRE((reinterpret_cast<uintptr_t>(tc_img_p) & 15) == 0, DDRL_E_BADARG,
+                 "fcnet_forward_tc_coupled: the weight image must be 16-byte aligned (TMA bulk copies)");
+    if (R == 0) return DDRL_OK;
+    TcTrainArgs a = {};
+    a.img = (const unsigned char*)tc_img_p; a.obs = obs; a.R = R; a.D = D; a.A = A; a.MB = (int)R;
+    a.hp = ddrl_ppo_hyper{0.f, 0.f, 0.f, 0.f, 1.f};
+    a.status = status; a.dbg_clock = nullptr; a.tail = SgdTail{};
+    a.norm = norm; a.clip = clip; a.obs_out = obs_out; a.logits_out = logits; a.value_out = value; a.eps = eps;
+    a.action_out = action; a.logp_out = logp;
+    int dev = 0, sms = 0;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const int G = (int)std::max<int64_t>(1, std::min<int64_t>((R + TC_ROWS - 1) / TC_ROWS, std::max(1, sms)));
+    const int rc = launch_tc2_forward_cup(a, node_id, coupling, G, (cudaStream_t)stream);
+    if (rc != DDRL_OK) return rc;
+    DDRL_CHECK_LAUNCH("fcnet_forward_tc_coupled");
+    return DDRL_OK;
+}

@@ -181,6 +181,7 @@ __global__ void __launch_bounds__(T2_NT, 1) fcnet_train_tc2_kernel(const __grid_
     constexpr bool CUP = false;
     const int32_t* const node_id = nullptr;
     const float* const cup_theta = nullptr;
+    const float* const coupling = nullptr;
 #include "tc2_step_body.inc"
 }
 
@@ -191,6 +192,19 @@ __global__ void __launch_bounds__(T2_NT, 1) fcnet_train_tc2_cup_kernel(const __g
                                                                        const float* __restrict__ cup_theta) {
     constexpr int A = 2;
     constexpr bool FWD = false, LL = false, DBG = false, CUP = true;
+    const float* const coupling = nullptr;
+#include "tc2_step_body.inc"
+}
+
+// the leg-coupled inference forward (ddrl_fcnet_forward_tc_coupled): the FWD pipeline with the mean logits scaled by
+// coupling[node_id[r]] before they are stored and sampled from.  node_id [R] (staged with the tile's noise), coupling [4][2].
+// D is read from a.D, as in the uncoupled forward: with D as a compile-time constant (DT = 19, 20) ptxas spilled 16 bytes.
+__global__ void __launch_bounds__(T2_NT, 1) fcnet_forward_tc2_cup_kernel(const __grid_constant__ TcTrainArgs a,
+                                                                         const int32_t* __restrict__ node_id,
+                                                                         const float* __restrict__ coupling) {
+    constexpr int A = 2, DT = 0;
+    constexpr bool FWD = true, LL = false, DBG = false, CUP = true;
+    const float* const cup_theta = nullptr;
 #include "tc2_step_body.inc"
 }
 
@@ -308,6 +322,19 @@ int launch_tc2_cup(const TcTrainArgs& a, const int32_t* node_id, const float* th
     if (a.A == 2 && a.D == 20) return launch_tc2_cup_t<20>(a, node_id, theta, P, G, st);
     set_error("ppo_train_step_tc_coupled: instantiated for A = 2 and D in {19, 20} (SharedDecentralLegID), got D=%d A=%d", a.D, a.A);
     return DDRL_E_UNSUPPORTED_SHAPE;
+}
+
+int launch_tc2_forward_cup(const TcTrainArgs& a, const int32_t* node_id, const float* coupling, int G, cudaStream_t st) {
+    static bool attr = false;
+    if (!attr) {
+        if (cudaFuncSetAttribute(fcnet_forward_tc2_cup_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess) {
+            set_error("fcnet_forward_tc_coupled: cannot raise dynamic shared memory: %s", cudaGetErrorString(cudaGetLastError()));
+            return DDRL_E_CUDA;
+        }
+        attr = true;
+    }
+    fcnet_forward_tc2_cup_kernel<<<dim3(G, 1), T2_NT, (size_t)tc2_smem(a.D, 2, true).total, st>>>(a, node_id, coupling);
+    return DDRL_OK;
 }
 
 int launch_tc2_forward(const TcTrainArgs& a, int P, int G, cudaStream_t st) {

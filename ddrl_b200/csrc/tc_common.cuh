@@ -38,6 +38,8 @@ int launch_tc2(const TcTrainArgs& a, int P, int G, cudaStream_t st);
 int launch_tc2_forward(const TcTrainArgs& a, int P, int G, cudaStream_t st);
 // leg-coupled ping-pong step (SharedDecentralLegID): A = 2, D in {19, 20}; node_id [P][R], theta [P][NP + 8]
 int launch_tc2_cup(const TcTrainArgs& a, const int32_t* node_id, const float* theta, int P, int G, cudaStream_t st);
+// leg-coupled inference forward (P = 1, A = 2, tc2_eligible D): node_id [R], coupling [4][2]
+int launch_tc2_forward_cup(const TcTrainArgs& a, const int32_t* node_id, const float* coupling, int G, cudaStream_t st);
 
 // Power-of-two operand scales (see header comment).  What matters is the absolute error relative to the tensor's
 // scale: entries too small for a normal lo half lose at most 2^-25/scale, negligible next to the entries that dominate.

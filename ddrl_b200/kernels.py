@@ -584,6 +584,61 @@ def fcnet_forward_tc(tc_img, obs, A: int, norm=None, clip: float = 0.0, eps=None
     return o
 
 
+def _coupled_outputs(obs, A: int, eps, out: Optional[dict], want_obs_out: bool) -> dict:
+    P, R, D = obs.shape
+    f32, dev = torch.float32, obs.device
+    o = dict(out) if out is not None else {}
+    shapes = {"logits": (P, R, 2 * A), "value": (P, R), "obs_out": (P, R, D) if want_obs_out else None}
+    if eps is not None:
+        shapes.update(action=(P, R, A), logp=(P, R))
+    for k, shp in shapes.items():
+        if k not in o:
+            o[k] = torch.empty(shp, dtype=f32, device=dev) if shp is not None else None
+    return o
+
+
+def fcnet_forward_coupled(theta, obs, node_id, coupling, A: int = 2, norm=None, clip: float = 0.0, eps=None,
+                          status: Optional[torch.Tensor] = None, out: Optional[dict] = None, img=None,
+                          want_obs_out: bool = False) -> dict:
+    """Leg-coupled inference in ONE launch (ddrl_fcnet_forward_coupled, FP32): theta [1,NP] (or the packed image img),
+    obs [1,R,D], node_id [1,R] int32 0..3, coupling [4,2] (or the flat 8 entries) -> dict(logits (coupled), value
+    [, obs_out][, action, logp], status).  Bit-identical to fcnet_forward -> leg_coupling_ -> dg_sample.  A node id outside
+    0..3 sets STATUS_BAD_NODE in ``status`` (a new zeroed int32 [1] unless given); ``out`` entries set to None are skipped."""
+    P, R, D = obs.shape
+    f32 = torch.float32
+    o = _coupled_outputs(obs, A, eps, out, want_obs_out)
+    if status is None:
+        status = torch.zeros(1, dtype=torch.int32, device=obs.device)
+    _lib.check(_lib.load().ddrl_fcnet_forward_coupled(
+        _p(theta, f32, "theta"), _p(img, f32, "img"), _p(node_id, torch.int32, "node_id"), _p(coupling, f32, "coupling"),
+        _p(obs, f32, "obs"), _p(norm, torch.float64, "norm"), float(clip or 0.0), P, R, D, A,
+        _p(o.get("obs_out"), f32, "obs_out"), _p(o.get("logits"), f32, "logits"), _p(o.get("value"), f32, "value"),
+        _p(eps, f32, "eps"), _p(o.get("action"), f32, "action"), _p(o.get("logp"), f32, "logp"),
+        _p(status, torch.int32, "status"), _stream()), "fcnet_forward_coupled")
+    o["status"] = status
+    return o
+
+
+def fcnet_forward_tc_coupled(tc_img, obs, node_id, coupling, A: int = 2, norm=None, clip: float = 0.0, eps=None,
+                             status: Optional[torch.Tensor] = None, out: Optional[dict] = None,
+                             want_obs_out: bool = False) -> dict:
+    """Leg-coupled inference on the tensor cores in ONE launch (ddrl_fcnet_forward_tc_coupled; D in {19, 20}): as
+    fcnet_forward_coupled with the tensor-core weight image.  Bit-identical to fcnet_forward_tc -> leg_coupling_ -> dg_sample."""
+    P, R, D = obs.shape
+    f32 = torch.float32
+    o = _coupled_outputs(obs, A, eps, out, want_obs_out)
+    if status is None:
+        status = torch.zeros(1, dtype=torch.int32, device=obs.device)
+    _lib.check(_lib.load().ddrl_fcnet_forward_tc_coupled(
+        _p(tc_img, torch.uint8, "tc_img"), _p(node_id, torch.int32, "node_id"), _p(coupling, f32, "coupling"),
+        _p(obs, f32, "obs"), _p(norm, torch.float64, "norm"), float(clip or 0.0), P, R, D, A,
+        _p(o.get("obs_out"), f32, "obs_out"), _p(o.get("logits"), f32, "logits"), _p(o.get("value"), f32, "value"),
+        _p(eps, f32, "eps"), _p(o.get("action"), f32, "action"), _p(o.get("logp"), f32, "logp"),
+        _p(status, torch.int32, "status"), _stream()), "fcnet_forward_tc_coupled")
+    o["status"] = status
+    return o
+
+
 def tc_set_variant(variant: int) -> None:
     """0 = automatic (ping-pong kernel when D <= 30 and A <= 4), 1 = branch-sequential kernel, 2 = ping-pong kernel."""
     _lib.check(_lib.load().ddrl_tc_set_variant(int(variant)), "tc_set_variant")

@@ -382,14 +382,16 @@ class FCNetLearner(_LearnerBase):
             else:
                 K.filter_update(obs_flat, self.filt_n, self.filt_M, self.filt_S, self.norm, b["filt_ws"])
         if self.coupled:
-            # forward without sampling, LegCoupling on the mean logits, then DiagGaussian sample + logp of the COUPLED
-            # distribution (the stored old logits are the coupled ones)
-            out = {"logits": b["logits"], "value": b["value"], "obs_out": b["obs"]}
+            # ONE launch: forward, LegCoupling on the mean logits, DiagGaussian sample + logp of the COUPLED distribution
+            # (the stored old logits are the coupled ones)
+            out = {"logits": b["logits"], "value": b["value"], "obs_out": b["obs"], "action": b["act"], "logp": b["logp"]}
+            coupling = self.theta[0, self.NPf:]
             if self.tc_forward and self.tc_img is not None:
-                K.fcnet_forward_tc(self.tc_img, obs_flat, A, norm=self.norm, clip=cfg.filter_clip, out=out, status=self.tc_status)
+                K.fcnet_forward_tc_coupled(self.tc_img, obs_flat, b["node"], coupling, A, norm=self.norm, clip=cfg.filter_clip,
+                                           eps=eps_flat, status=self.tc_status, out=out)
             else:
-                K.fcnet_forward(self.theta_fc, obs_flat, A, norm=self.norm, clip=cfg.filter_clip, out=out, img=self.img)
-            self._couple_and_sample(b["logits"], b["node"], eps_flat, b["act"], b["logp"])
+                K.fcnet_forward_coupled(self.theta_fc, obs_flat, b["node"], coupling, A, norm=self.norm, clip=cfg.filter_clip,
+                                        eps=eps_flat, status=self.tc_status, out=out, img=self.img)
             if self.tc_forward and self.tc_img is not None:
                 K.fcnet_forward_tc(self.tc_img, boot_obs, A, norm=self.norm, clip=cfg.filter_clip,
                                    out={"logits": None, "value": b["vboot"], "obs_out": None}, status=self.tc_status)
@@ -421,15 +423,6 @@ class FCNetLearner(_LearnerBase):
                 K.gather_rows(b[nme], shuffle, b[nme + "_s"])
             if self.coupled:      # the node ids travel with their rows (a 4-byte row copy: the int32 bits move unchanged)
                 K.gather_rows(b["node"].view(torch.float32), shuffle, b["node_s"].view(torch.float32))
-
-    def _couple_and_sample(self, logits, node, eps, act, logp):
-        """logits [1,R,4] in place *= LegCoupling table [node] (mean half), then action / logp of the coupled DiagGaussian."""
-        from . import _lib
-        R = logits.shape[1]
-        K.leg_coupling_(logits.view(R, 4), node.view(R), self.theta[0, self.NPf:])
-        f32 = torch.float32
-        _lib.check(_lib.load().ddrl_dg_sample(K._p(logits, f32, "logits"), K._p(eps, f32, "eps"), R, self.A,
-                                              K._p(act, f32, "action"), K._p(logp, f32, "logp"), K._stream()), "dg_sample")
 
     def _prepare_cached(self, b, obs_flat, boot_obs, rewards, dones, eps_flat, shuffle, cols_per_env, update_filter, T, Cc):
         """The ~20 short launches of the preparation phase are captured once per set of input buffers and replayed (the
@@ -657,18 +650,11 @@ class FCNetLearner(_LearnerBase):
         P, B, _ = raw_obs.shape
         if tuple(node_idx.shape) != (P, B) or node_idx.dtype != torch.int32 or not node_idx.is_cuda:
             raise DDRLError(f"compute_actions: node_idx must be an int32 CUDA tensor of shape {(P, B)}")
-        if int(((node_idx < 0) | (node_idx > 3)).sum().item()):
+        res = K.fcnet_forward_coupled(self.theta_fc, raw_obs, node_idx.contiguous(), self.theta[0, self.NPf:], self.A,
+                                      norm=use_norm, clip=self.cfg.filter_clip, eps=eps)
+        if int(res.pop("status").item()) & K.STATUS_BAD_NODE:
             raise DDRLError("compute_actions: node ids must be 0..3 (FL, HL, HR, FR)")
-        res = K.fcnet_forward(self.theta_fc, raw_obs, self.A, norm=use_norm, clip=self.cfg.filter_clip)
-        K.leg_coupling_(res["logits"].view(B, 4), node_idx.reshape(B).contiguous(), self.theta[0, self.NPf:])
-        if eps is not None:
-            res["action"] = torch.empty(P, B, self.A, dtype=torch.float32, device=raw_obs.device)
-            res["logp"] = torch.empty(P, B, dtype=torch.float32, device=raw_obs.device)
-            from . import _lib
-            f32 = torch.float32
-            _lib.check(_lib.load().ddrl_dg_sample(K._p(res["logits"], f32, "logits"), K._p(eps, f32, "eps"), B, self.A,
-                                                  K._p(res["action"], f32, "action"), K._p(res["logp"], f32, "logp"),
-                                                  K._stream()), "dg_sample")
+        res.pop("obs_out")
         return res
 
 

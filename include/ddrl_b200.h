@@ -485,6 +485,25 @@ int ddrl_ppo_train_step_tc_coupled(const void* tc_img, const float* theta, const
                                    const float* kl_coeff, const ddrl_ppo_hyper* hyper, int ctas_per_policy,
                                    float* grad_part, double* stat_part, int* status, const ddrl_sgd_tail* tail,
                                    void* stream);
+/* Inference of the leg-coupled policy in ONE launch (the sampler-side call and the rollout forward of SharedDecentralLegID):
+ * the contract of ddrl_fcnet_forward / ddrl_fcnet_forward_tc (filter prologue, obs_out, logits, value, DiagGaussian sample
+ * epilogue; any of obs_out / logits / value / eps (+ action, logp) may be NULL) with LegCoupling applied to the logits:
+ *   node_id [P][R] int32 in 0..3, coupling [4][2] (the table, theta[NP .. NP + 8) of the coupled learner);
+ *   logits[r][i] = pre[r][i] * coupling[node_id[r]][i] for i < 2 (one rounding; the log-std half and value unchanged), and
+ *   action / logp are drawn from that coupled DiagGaussian.
+ * Bit-identical to ddrl_fcnet_forward (resp. ddrl_fcnet_forward_tc) -> ddrl_leg_coupling -> ddrl_dg_sample on the same
+ * inputs.  A node id outside 0..3 sets *status |= DDRL_STATUS_BAD_NODE (the row is then coupled as node id & 3); status is
+ * REQUIRED.  A = 2 and P = 1 only (DDRL_E_BADARG otherwise, as for the null pointers and R < 0); R = 0 does nothing.
+ * ddrl_fcnet_forward_coupled is the FP32 kernel (weights from theta [P][NP] or the packed image img); the tensor-core entry
+ * takes the tensor-core image and is instantiated for D in {19, 20} (DDRL_E_UNSUPPORTED_SHAPE otherwise). */
+int ddrl_fcnet_forward_coupled(const float* theta, const float* img, const int32_t* node_id, const float* coupling,
+                               const float* obs, const double* norm, float clip, int P, int64_t R, int D, int A,
+                               float* obs_out, float* logits, float* value, const float* eps, float* action, float* logp,
+                               int* status, void* stream);
+int ddrl_fcnet_forward_tc_coupled(const void* tc_img, const int32_t* node_id, const float* coupling, const float* obs,
+                                  const double* norm, float clip, int P, int64_t R, int D, int A, float* obs_out,
+                                  float* logits, float* value, const float* eps, float* action, float* logp, int* status,
+                                  void* stream);
 
 /* Diagnostic: one tcgen05 (UMMA) GEMM through TMEM with the chunked shared-memory operand layout the tensor-core
  * training step uses (csrc/umma.cuh): D[m][n] = sum_k A(m,k) B(n,k), m < M (64 or 128), A(m,k) = A[m][k] (a_mn = 0, K-major) or

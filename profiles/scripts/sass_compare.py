@@ -8,7 +8,10 @@ import sys
 
 RENAMED = {  # graphnet_fwd_warp_kernel became a template on SAMPLE; <false> is the former kernel
     "_ZN4ddrl24graphnet_fwd_warp_kernelEPKfPKiS1_S1_liPfS4_":
-        "_ZN4ddrl24graphnet_fwd_warp_kernelILb0EEEvPKfPKiS2_S2_liPfS5_S2_S5_S5_"}
+        "_ZN4ddrl24graphnet_fwd_warp_kernelILb0EEEvPKfPKiS2_S2_liPfS5_S2_S5_S5_",
+    # fcnet_forward_kernel became a template on CUP (leg coupling); <false> is the former kernel
+    "_ZN4ddrl20fcnet_forward_kernelEPKfS1_S1_PKdfliiPfS4_S4_S1_S4_S4_":
+        "_ZN4ddrl20fcnet_forward_kernelILb0EEEvPKfS2_S2_PKdfliiPfS5_S5_S2_S5_S5_PKiS2_Pi"}
 
 
 def functions(obj):
