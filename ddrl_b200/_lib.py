@@ -94,6 +94,7 @@ PROTOTYPES = {
     "ddrl_grad_tie": (C.c_int, [c_f32p, c_i32p, C.c_int, C.c_int, C.c_int, c_f32p, c_stream]),
     "ddrl_leg_coupling_backward": (C.c_int, [c_f32p, c_f32p, c_i32p, c_f32p, C.c_int64, C.c_int, c_f32p, c_stream]),
     "ddrl_fcnet_tc_image_bytes": (C.c_int, [C.c_int, C.c_int]),
+    "ddrl_fcnet_train_supported": (C.c_int, [C.c_int, C.c_int, C.c_int]),
     "ddrl_fcnet_forward_tc": (C.c_int, [C.c_void_p, c_f32p, c_f64p, C.c_float, C.c_int, C.c_int64, C.c_int, C.c_int,
                                          c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_i32p, c_stream]),
     "ddrl_fcnet_forward_coupled": (C.c_int, [c_f32p, c_f32p, c_i32p, c_f32p, c_f32p, c_f64p, C.c_float, C.c_int, C.c_int64,

@@ -65,8 +65,8 @@ __host__ __device__ inline TcSmem tc_smem(int D, int A) {
 //   * the loss-gradient operand DL[b] sits in the W1 part of the weight image (W1 is only read by F1; a CTA with another
 //     tile to go reloads it from L2 behind the backward, and every step reloads the whole image anyway);
 //   * the fp32 staging of the observations (xraw) sits in H2[1] (free from B3(1) of one tile to tanh2(1) of the next).
-// That fits KX <= 48 (D <= 46) for A <= 4, and A = 8 for 31 <= D <= 46 (the centralized controller): every published
-// architecture.
+// That fits KX <= 48 (D <= 47) for every A in {1, 2, 4, 8}; below KX = 32 DL (and for A = 8 the old logits) get regions of
+// their own.
 struct Tc2Smem {
     int X[2], H1[2][2], H2[2][2], DL[2][2], xraw, pf, po, red, bar, nid, cup, total;
     bool dl_in_w1, po_in_w1;

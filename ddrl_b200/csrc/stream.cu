@@ -658,6 +658,14 @@ extern "C" int ddrl_grad_reduce(const float* grad_part, const double* stat_part,
     return DDRL_OK;
 }
 
+extern "C" int ddrl_fcnet_train_supported(int D, int A, int tensor_cores) {
+    if (tensor_cores)      // ddrl_ppo_train_step_tc: shape check, then its shared memory (branch-sequential kernel)
+        return ddrl_fcnet_tc_image_bytes(D, A) > 0 && tc_smem(D, A).total <= 227 * 1024;
+    // ddrl_ppo_train_step: shape check, then the train kernel's shared memory
+    return D >= 1 && D <= DDRL_MAX_OBS && A >= 1 && A <= DDRL_MAX_ACT &&
+           (size_t)fc_smem(D, A, false, true).total * sizeof(float) <= 227 * 1024;
+}
+
 extern "C" int ddrl_clip_adam(float* theta, float* m, float* v, float* beta_pow, const float* grad, int P, int NP,
                               float lr, float beta1, float beta2, float eps, float grad_clip, float* gnorm_out,
                               int32_t* step_ctr, int32_t* sync_ws, float* fcnet_img, void* fcnet_tc_img, int img_D,
@@ -667,6 +675,8 @@ extern "C" int ddrl_clip_adam(float* theta, float* m, float* v, float* beta_pow,
     DDRL_REQUIRE(!(fcnet_img || fcnet_tc_img) || (img_D >= 1 && img_D <= DDRL_MAX_OBS && img_A >= 1 && img_A <= DDRL_MAX_ACT &&
                                 fc_offsets(img_D, img_A).NP == NP),
                  DDRL_E_BADARG, "clip_adam: fcnet image given but (D=%d, A=%d) does not match NP=%d", img_D, img_A, NP);
+    DDRL_REQUIRE(!fcnet_tc_img || ddrl_fcnet_tc_image_bytes(img_D, img_A) > 0, DDRL_E_UNSUPPORTED_SHAPE,
+                 "clip_adam: no tensor-core image exists for D=%d A=%d (A in {1,2,4,8}, D <= 63)", img_D, img_A);
     clip_adam_kernel<<<dim3((NP + AT - 1) / AT, P), AT, 0, (cudaStream_t)stream>>>(
         theta, m, v, beta_pow, grad, NP, lr, beta1, beta2, eps, grad_clip, gnorm_out, step_ctr, sync_ws, fcnet_img,
         (unsigned char*)fcnet_tc_img, img_D, img_A);

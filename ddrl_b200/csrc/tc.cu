@@ -644,14 +644,14 @@ __global__ void fcnet_tc_pack_kernel(const float* __restrict__ theta, int D, int
 }  // namespace ddrl
 
 extern "C" int ddrl_fcnet_tc_image_bytes(int D, int A) {
-    if (D < 1 || D > DDRL_MAX_OBS - 1 || A < 1 || A > DDRL_MAX_ACT) return DDRL_E_UNSUPPORTED_SHAPE;
+    if (D < 1 || D > DDRL_MAX_OBS - 1 || !(A == 1 || A == 2 || A == 4 || A == 8)) return DDRL_E_UNSUPPORTED_SHAPE;
     return tc_img(D, A).bytes;
 }
 
 extern "C" int ddrl_fcnet_tc_pack(const float* theta, int P, int D, int A, void* img, void* stream) {
     DDRL_REQUIRE(theta && img && P >= 1, DDRL_E_BADARG, "fcnet_tc_pack: null pointer or bad P");
-    DDRL_REQUIRE(D >= 1 && D <= DDRL_MAX_OBS - 1 && A >= 1 && A <= DDRL_MAX_ACT, DDRL_E_UNSUPPORTED_SHAPE,
-                 "fcnet_tc_pack: unsupported D=%d A=%d", D, A);
+    DDRL_REQUIRE(D >= 1 && D <= DDRL_MAX_OBS - 1 && (A == 1 || A == 2 || A == 4 || A == 8), DDRL_E_UNSUPPORTED_SHAPE,
+                 "fcnet_tc_pack: unsupported D=%d A=%d (A in {1,2,4,8}, D <= 63)", D, A);
     const int NP = fc_offsets(D, A).NP;
     cudaMemsetAsync(img, 0, (size_t)P * tc_img(D, A).bytes, (cudaStream_t)stream);
     fcnet_tc_pack_kernel<<<dim3((NP + 255) / 256, P), 256, 0, (cudaStream_t)stream>>>(theta, D, A, (unsigned char*)img);
@@ -718,7 +718,7 @@ extern "C" int ddrl_ppo_train_step_tc(const void* tc_img_p, const float* obs, co
         a.tail = *tail;
         const bool pp = g_tc_variant == 2 || (g_tc_variant == 0 && tc2_eligible(D, A));
         DDRL_REQUIRE(tail->nsteps <= 1 || pp, DDRL_E_UNSUPPORTED_SHAPE,
-                     "ppo_train_step_tc: nsteps > 1 needs the ping-pong kernel (D <= 46; A = 8: D >= 31)");
+                     "ppo_train_step_tc: nsteps > 1 needs the ping-pong kernel (D <= 47)");
     }
     const size_t smem = (size_t)tc_smem(D, A).total;
     DDRL_REQUIRE(smem <= 227 * 1024, DDRL_E_UNSUPPORTED_SHAPE, "ppo_train_step_tc: shared memory %zu > 227 KB", smem);
@@ -726,7 +726,7 @@ extern "C" int ddrl_ppo_train_step_tc(const void* tc_img_p, const float* obs, co
     const bool pingpong = g_tc_variant == 2 || (g_tc_variant == 0 && tc2_eligible(D, A));
     if (pingpong) {
         DDRL_REQUIRE(tc2_eligible(D, A), DDRL_E_UNSUPPORTED_SHAPE,
-                     "ppo_train_step_tc: ping-pong variant needs D <= 46 (A = 8: 31 <= D <= 46) (D=%d, A=%d)", D, A);
+                     "ppo_train_step_tc: ping-pong variant needs D <= 47 (D=%d, A=%d)", D, A);
         rc = launch_tc2(a, P, ctas_per_policy, (cudaStream_t)stream);
         if (rc != DDRL_OK) return rc;
         DDRL_CHECK_LAUNCH("ppo_train_step_tc");
@@ -787,7 +787,7 @@ extern "C" int ddrl_fcnet_forward_tc(const void* tc_img_p, const float* obs, con
     DDRL_REQUIRE(tc_img_p && obs && P >= 1 && R >= 0, DDRL_E_BADARG, "fcnet_forward_tc: null pointer or bad P/R");
     DDRL_REQUIRE(!eps || (action && logp), DDRL_E_BADARG, "fcnet_forward_tc: eps given without action / logp outputs");
     DDRL_REQUIRE(D >= 1 && D <= DDRL_MAX_OBS - 1 && (A == 1 || A == 2 || A == 4 || A == 8) && tc2_eligible(D, A),
-                 DDRL_E_UNSUPPORTED_SHAPE, "fcnet_forward_tc: unsupported D=%d A=%d (D <= 46; A = 8: D >= 31)", D, A);
+                 DDRL_E_UNSUPPORTED_SHAPE, "fcnet_forward_tc: unsupported D=%d A=%d (A in {1,2,4,8}, D <= 47)", D, A);
     DDRL_REQUIRE(R <= 0x7fffffff, DDRL_E_UNSUPPORTED_SHAPE, "fcnet_forward_tc: R must fit 31 bits");
     if (R == 0) return DDRL_OK;
     TcTrainArgs a = {};

@@ -14,7 +14,7 @@
 //     them because one thread issues a tcgen05.mma only every ~72 cycles whatever its shape (tests/umma_bench.py).
 //   * the two PPO-loss halves (policy part on warps 0-3, value part on warps 4-7) run concurrently.
 //   * H1/H2 of both branches live in shared memory (128 KB); DL, the observation staging and (A = 8) the old logits reuse
-//     space that is dead at the time (fcnet_tc_layout.cuh): D <= 46, every published architecture (tc2_eligible).
+//     space that is dead at the time (fcnet_tc_layout.cuh): D <= 47, every published architecture (tc2_eligible).
 //   * the weight-gradient GEMMs stack the hi | lo halves of their A operand along M (tc_gemm_stack_u: one M = 128 MMA gives
 //     A_hi^T B and A_lo^T B; dependent chains of 16 / 8 instead of 24 / 16 MMAs), and the four MMA-issue warps — idle between
 //     two hand-offs — read the finished accumulators out of TMEM and stage the partial gradient in shared memory in the gaps

@@ -33,7 +33,7 @@ struct TcTrainArgs {
     const float* eps;
 };
 
-// ping-pong variant (tc2.cu); A in {1,2,4}, tc2_eligible(D, A)
+// ping-pong variant (tc2.cu); A in {1,2,4,8}, tc2_eligible(D, A): D <= 47
 int launch_tc2(const TcTrainArgs& a, int P, int G, cudaStream_t st);
 int launch_tc2_forward(const TcTrainArgs& a, int P, int G, cudaStream_t st);
 // leg-coupled ping-pong step (SharedDecentralLegID): A = 2, D in {19, 20}; node_id [P][R], theta [P][NP + 8]

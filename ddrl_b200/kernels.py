@@ -640,7 +640,7 @@ def fcnet_forward_tc_coupled(tc_img, obs, node_id, coupling, A: int = 2, norm=No
 
 
 def tc_set_variant(variant: int) -> None:
-    """0 = automatic (ping-pong kernel when D <= 30 and A <= 4), 1 = branch-sequential kernel, 2 = ping-pong kernel."""
+    """0 = automatic (ping-pong kernel when D <= 47), 1 = branch-sequential kernel, 2 = ping-pong kernel (D <= 47)."""
     _lib.check(_lib.load().ddrl_tc_set_variant(int(variant)), "tc_set_variant")
 
 

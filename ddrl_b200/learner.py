@@ -65,6 +65,16 @@ def finalize_stats(sums: np.ndarray, kl_coeff: np.ndarray, cfg: PPOConfig, rows:
              "cur_lr": lr, "entropy_coeff": ec} for p in range(P)]
 
 
+_ENVELOPE = {"tc": "the tensor-core SGD step runs 1 <= D <= 63 and A in (1, 2, 4, 8)",
+             "fp32": "the FP32 SGD step runs 1 <= D <= 64 and 1 <= A <= 8, with D <= 60 for A = 8 (shared memory)"}
+
+
+def fcnet_mode_supports(D: int, A: int, mode: str) -> bool:
+    """True if the SGD step of `mode` runs an FCNet of observation width D and action width A (ddrl_fcnet_train_supported)."""
+    from . import _lib
+    return bool(_lib.load().ddrl_fcnet_train_supported(int(D), int(A), int(mode == "tc")))
+
+
 class _LearnerBase:
     def __init__(self, P: int, NP: int, cfg: PPOConfig, device, theta: Optional[torch.Tensor]):
         if not torch.cuda.is_available():
@@ -151,6 +161,10 @@ class FCNetLearner(_LearnerBase):
         c[node id], node id = the agent's position in agent_names (FL, HL, HR, FR); the SGD steps are
         ddrl_ppo_train_step_tc_coupled / ddrl_ppo_train_step_coupled (fused tail required: the table is clipped and stepped
         with the MLP weights)."""
+        if mode not in ("tc", "fp32"):
+            raise DDRLError(f"mode must be 'tc' or 'fp32', got {mode!r}")
+        if not fcnet_mode_supports(D, A, mode):
+            raise DDRLError(f"mode={mode!r} cannot train an FCNet with D={D}, A={A}: " + _ENVELOPE[mode])
         self.coupled = bool(leg_coupling)
         if self.coupled:
             if P != 1 or A != 2:
@@ -192,8 +206,6 @@ class FCNetLearner(_LearnerBase):
                     inv[j, 0 if inv[j, 0] < 0 else 1] = i
             self.inverse_map = inv.to(dev_)
             K.param_expand(self.theta_model, self.layout_map, self.theta)
-        if mode not in ("tc", "fp32"):
-            raise DDRLError(f"mode must be 'tc' or 'fp32', got {mode!r}")
         self.mode = mode
         self.fuse_tail = fuse_tail
         self.persistent = persistent      # one persistent launch per epoch where the kernel supports it
@@ -573,7 +585,9 @@ class FCNetLearner(_LearnerBase):
                                      (8, "dl overflow"), (16, "dz2 overflow"), (32, "dz1 overflow"),
                                      (64, "fused-tail barrier / peer wait timed out"),
                                      (K.STATUS_BAD_NODE, "leg-coupling node id outside 0..3")) if code & bit]
-            hint = (" — fp16 split range exceeded: use mode='fp32' for this workload" if code & 62 else
+            fp32 = ("use mode='fp32' for this workload" if fcnet_mode_supports(self.D, self.A, "fp32") else
+                    f"mode='fp32' cannot train this shape either ({_ENVELOPE['fp32']})")
+            hint = (" — fp16 split range exceeded: " + fp32 if code & 62 else
                     " — node ids must be 0..3 (FL, HL, HR, FR)" if code & K.STATUS_BAD_NODE else
                     " — a CTA barrier or a peer rank did not arrive in time")
             raise DDRLError("SGD step failed (" + ", ".join(what) + ")" + hint)

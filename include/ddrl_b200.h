@@ -166,6 +166,8 @@ int ddrl_gather_rows(const float* src, const int32_t* perm, int P, int64_t R, in
 /* One minibatch of: model forward + PPOLoss + backward (no optimizer).
  * Replaces: one session.run of loss+grads in TrainTFMultiGPU for all P policies at once
  * (RLlib agents/ppo/ppo_tf_policy.py PPOLoss; DiagGaussian logp/kl/entropy).
+ * Shapes: D <= 64, A <= 8, and D <= 60 for A = 8 (the kernel's shared memory exceeds 227 KB beyond that:
+ * DDRL_E_UNSUPPORTED_SHAPE).
  * Batch arrays are [P][R][*] float32; the minibatch is rows [mb*MB, (mb+1)*MB) where
  *   mb = mb_perm[p][*step_ctr]          (device ints; lets one CUDA graph serve every step)
  *   kl_coeff [P] float32 (device),  hyper (host values): clip_param, vf_clip_param, vf_loss_coeff,
@@ -249,6 +251,11 @@ int ddrl_ppo_train_step(const float* theta, const float* img, const float* obs, 
                         const int32_t* mb_perm, int64_t perm_stride, const int32_t* step_ctr,
                         const float* kl_coeff, const ddrl_ppo_hyper* hyper, int ctas_per_policy,
                         float* grad_part, double* stat_part, const ddrl_sgd_tail* tail, void* stream);
+
+/* 1 if the SGD step accepts an FCNet of observation width D and action width A, else 0 (pure host):
+ * tensor_cores = 0: ddrl_ppo_train_step (D <= 64, A <= 8, D <= 60 for A = 8);
+ * tensor_cores = 1: ddrl_ppo_train_step_tc (D <= 63, A in {1,2,4,8}). */
+int ddrl_fcnet_train_supported(int D, int A, int tensor_cores);
 
 /* Stand-alone PPOLoss gradient w.r.t. the model outputs (same arithmetic as the fused kernel), for
  * models whose forward/backward are separate kernels (GraphNet):
@@ -414,19 +421,19 @@ int ddrl_grad_tie(const float* grad_kernel, const int32_t* inv, int P, int NPm, 
  * three products per GEMM, which keeps the 1e-5 parity bar.  Same batch arrays, minibatch selection, outputs
  * (grad_part [P][G][NPs], stat_part) and semantics as ddrl_ppo_train_step; the weights come from a tensor-core
  * image tc_img [P][ddrl_fcnet_tc_image_bytes(D, A)] built by ddrl_fcnet_tc_pack (or kept in step by
- * ddrl_clip_adam).  D <= 63, A in {1,2,4,8}.  *status (device int, may be NULL) receives OR-ed flags: 1 = an MMA
+ * ddrl_clip_adam).  D <= 63, A in {1,2,4,8} (ddrl_fcnet_tc_image_bytes / ddrl_fcnet_tc_pack refuse other shapes).  *status (device int, may be NULL) receives OR-ed flags: 1 = an MMA
  * completion wait timed out; 64 = a fused-tail barrier timed out; 2/4/8/16/32 = fp16 overflow (clamped) while splitting x / activations / dl / dz2 / dz1 —
  * the result is then unreliable and the step should be redone with ddrl_ppo_train_step. */
 int ddrl_fcnet_tc_image_bytes(int D, int A);
 /* Inference on the tensor cores: same contract as ddrl_fcnet_forward (filter normalise prologue, logits / value,
  * DiagGaussian sample + logp epilogue) with the GEMMs on tcgen05 (fp16 hi/lo split, ~3e-6 relative); weights from the
- * tensor-core image.  Shapes the ping-pong kernel covers (D <= 46; A = 8: D >= 31).  Any of obs_out / logits / value /
+ * tensor-core image.  Shapes the ping-pong kernel covers: D <= 47, A in {1,2,4,8}.  Any of obs_out / logits / value /
  * eps (+ action, logp) may be NULL. */
 int ddrl_fcnet_forward_tc(const void* tc_img, const float* obs, const double* norm, float clip, int P, int64_t R,
                           int D, int A, float* obs_out, float* logits, float* value, const float* eps,
                           float* action, float* logp, int* status, void* stream);
 /* Two schedules of the same arithmetic exist: 1 = branch-sequential (any D <= 63), 2 = "ping-pong" (both branches
- * resident, the tensor core runs one branch while the CTA runs the other's epilogue; D <= 46, A <= 4).
+ * resident, the tensor core runs one branch while the CTA runs the other's epilogue; D <= 47, A in {1,2,4,8}).
  * 0 (default) picks ping-pong whenever the shape allows it.  Process-wide; meant for tests and A/B timing. */
 int ddrl_tc_set_variant(int variant);
 /* 1 if ddrl_ppo_train_step_tc will use the ping-pong kernel for (D, A) under the current variant setting (the kernel that

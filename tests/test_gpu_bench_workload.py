@@ -88,8 +88,10 @@ def _learner(mode, **kw):
 
 def _assert_bench_shape(L, mode, persistent=True):
     """The launch shape this file claims to test; fails if the learner's choice drifts."""
+    from ddrl_b200 import kernels as K
     MB_, nb, G = L._sgd_setup(R)
     if MODES[mode]["mode"] == "tc":
+        assert K.tc_pingpong_eligible(D, A)                    # the ping-pong kernel (persistent launch)
         assert (MB_, nb, G) == (4096, 32, 32), (MB_, nb, G)
         assert MB_ // G == 128                                 # one full 128-row tile per CTA
         assert L._persistent_steps(G) == persistent

@@ -2,7 +2,7 @@
 the stacked M = 128 weight-gradient accumulators are read out by the four MMA-issue warps into TWO flat-indexed, ROTATED staging
 buffers (half 0 over H2, half 1 over the weight image), XOR-swizzled inside the two 64 x 64 blocks, and the copy-out adds the
 halves and undoes rotation and swizzle.  The arithmetic below is copied from the kernel (stage_w2 / stage_heads / stage_w1 /
-bias_stats / copy_out); the test checks for every published (D, A) and a few odd shapes that
+bias_stats / copy_out); the test checks for every shape the ping-pong kernel runs (D <= 47, A in {1, 2, 4, 8}) that
   * both staging buffers fit the memory they live in, and what is staged in "slot 1" (while B4(1) still runs) only touches
     memory that is dead at that time,
   * every flat index of the partial is written exactly once per half (half 1: zeros for the entries without lo-half rows),
@@ -11,8 +11,7 @@ import numpy as np
 import pytest
 
 H, TC_ROWS, TC_NO = 64, 128, 16
-SHAPES = [(19, 2), (20, 2), (27, 2), (27, 4), (28, 2), (28, 4), (35, 2), (36, 2), (43, 8), (44, 8), (5, 1), (14, 2), (15, 2), (31, 4),
-          (46, 4), (33, 8)]
+SHAPES = [(D, A) for A in (1, 2, 4, 8) for D in range(1, 48)]      # every ping-pong shape (tests/test_fcnet_envelope.py)
 
 
 def fc_offsets(D, A):      # csrc/common.cuh
