@@ -29,6 +29,21 @@ void count_launch(int n = 1);
         ::ddrl::count_launch();                                                        \
     } while (0)
 
+// Raises the dynamic shared-memory limit of kernel Kern to 227 KB (the sm_100a opt-in maximum) before its first launch;
+// the flag is a static of each instantiation, i.e. one per kernel.
+template <auto Kern>
+inline int raise_smem_once(const char* who) {
+    static bool done = false;
+    if (!done) {
+        if (cudaFuncSetAttribute(Kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess) {
+            set_error("%s: cannot raise dynamic shared memory: %s", who, cudaGetErrorString(cudaGetLastError()));
+            return DDRL_E_CUDA;
+        }
+        done = true;
+    }
+    return DDRL_OK;
+}
+
 // FCNet flat-parameter offsets (checkpoint order, include/ddrl_b200.h).
 struct FcOffsets {
     int W1, b1, Wv1, bv1, W2, b2, Wv2, bv2, Wo, bo, Wvo, bvo, NP;

@@ -373,7 +373,24 @@ extern "C" int ddrl_fcnet_pack(const float* theta, int P, int D, int A, float* i
     return DDRL_OK;
 }
 
-static int set_smem_attr(const void* fn, bool* done, const char* who);
+// TrainArgs of the two FP32 train steps and their dynamic shared memory.
+static int fp32_train_args(TrainArgs& a, size_t& smem, const char* who, const float* theta, const float* img, const float* obs,
+                           const float* actions, const float* old_logits, const float* old_logp, const float* vf_preds,
+                           const float* adv, const float* vtarg, const float* ext_dlogits, const float* ext_dvalue, int64_t R,
+                           int D, int A, int MB, const int32_t* mb_perm, int64_t perm_stride, const int32_t* step_ctr,
+                           const float* kl_coeff, const ddrl_ppo_hyper* hyper, float* grad_part, double* stat_part,
+                           const ddrl_sgd_tail* tail) {
+    a.theta = theta; a.img = img; a.obs = obs; a.actions = actions; a.old_logits = old_logits; a.old_logp = old_logp;
+    a.vf_preds = vf_preds; a.adv = adv; a.vtarg = vtarg; a.ext_dlogits = ext_dlogits; a.ext_dvalue = ext_dvalue;
+    a.R = R; a.D = D; a.A = A; a.MB = MB; a.mb_perm = mb_perm; a.perm_stride = perm_stride; a.step_ctr = step_ctr;
+    a.kl_coeff = kl_coeff;
+    a.hp = hyper ? *hyper : ddrl_ppo_hyper{0.f, 0.f, 0.f, 0.f, 1.f};
+    a.grad_part = grad_part; a.stat_part = stat_part;
+    a.tail = launch_tail(tail, false);
+    smem = (size_t)fc_smem(D, A, false, true).total * sizeof(float);
+    DDRL_REQUIRE(smem <= 227 * 1024, DDRL_E_UNSUPPORTED_SHAPE, "%s: shared memory %zu > 227 KB", who, smem);
+    return DDRL_OK;
+}
 
 extern "C" int ddrl_ppo_train_step_coupled(const float* theta, const float* img, const int32_t* node_id, const float* obs,
                                            const float* actions, const float* old_logits, const float* old_logp,
@@ -397,31 +414,33 @@ extern "C" int ddrl_ppo_train_step_coupled(const float* theta, const float* img,
     DDRL_REQUIRE(tail->nsteps <= 1, DDRL_E_UNSUPPORTED_SHAPE, "ppo_train_step_coupled: nsteps > 1 is not supported by the FP32 kernel");
     DDRL_REQUIRE(!tail->ll_ws, DDRL_E_BADARG, "ppo_train_step_coupled: the LL tail is not supported with leg coupling");
     TrainArgs a;
-    a.theta = theta; a.img = img; a.obs = obs; a.actions = actions; a.old_logits = old_logits; a.old_logp = old_logp;
-    a.vf_preds = vf_preds; a.adv = adv; a.vtarg = vtarg; a.ext_dlogits = nullptr; a.ext_dvalue = nullptr;
-    a.R = R; a.D = D; a.A = A; a.MB = MB; a.mb_perm = mb_perm; a.perm_stride = perm_stride; a.step_ctr = step_ctr;
-    a.kl_coeff = kl_coeff; a.hp = *hyper;
-    a.grad_part = grad_part; a.stat_part = stat_part;
-    a.tail = *tail;
-    a.tail.grad_acc = nullptr;
-    const FcSmem L = fc_smem(D, A, false, true);
-    const size_t smem = (size_t)L.total * sizeof(float);
-    DDRL_REQUIRE(smem <= 227 * 1024, DDRL_E_UNSUPPORTED_SHAPE, "ppo_train_step_coupled: shared memory %zu > 227 KB", smem);
-    static bool attr_set = false;
-    if (int rc2 = set_smem_attr((const void*)fcnet_train_cup_kernel, &attr_set, "ppo_train_step_coupled")) return rc2;
+    size_t smem = 0;
+    if (int rc2 = fp32_train_args(a, smem, "ppo_train_step_coupled", theta, img, obs, actions, old_logits, old_logp, vf_preds, adv,
+                                  vtarg, nullptr, nullptr, R, D, A, MB, mb_perm, perm_stride, step_ctr, kl_coeff, hyper,
+                                  grad_part, stat_part, tail))
+        return rc2;
+    if (int rc2 = raise_smem_once<fcnet_train_cup_kernel>("ppo_train_step_coupled")) return rc2;
     fcnet_train_cup_kernel<<<dim3(ctas_per_policy, P), NT, smem, (cudaStream_t)stream>>>(a, node_id);
     DDRL_CHECK_LAUNCH("ppo_train_step_coupled");
     return DDRL_OK;
 }
 
-static int set_smem_attr(const void* fn, bool* done, const char* who) {
-    if (!*done) {
-        if (cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess) {
-            set_error("%s: cannot raise dynamic shared memory: %s", who, cudaGetErrorString(cudaGetLastError()));
-            return DDRL_E_CUDA;
-        }
-        *done = true;
-    }
+// The launch both FP32 forwards share (CUP = true: ddrl_fcnet_forward_coupled, P = 1).
+template <bool CUP>
+static int fcnet_forward_launch(const char* who, const float* theta, const float* img, const float* obs, const double* norm,
+                                float clip, int P, int64_t R, int D, int A, float* obs_out, float* logits, float* value,
+                                const float* eps, float* action, float* logp, const int32_t* node_id, const float* coupling,
+                                int* status, void* stream) {
+    if (R == 0) return DDRL_OK;
+    const FcSmem L = fc_smem(D, A, norm != nullptr);
+    const size_t smem = (size_t)L.total * sizeof(float);
+    DDRL_REQUIRE(smem <= 227 * 1024, DDRL_E_UNSUPPORTED_SHAPE, "%s: shared memory %zu > 227 KB", who, smem);
+    if (int rc = raise_smem_once<fcnet_forward_kernel<CUP>>(who)) return rc;
+    const int64_t ntiles = (R + TM - 1) / TM;
+    const int per_policy = (int)std::min<int64_t>(ntiles, std::max(1, num_sms() / P));
+    fcnet_forward_kernel<CUP><<<dim3(per_policy, P), NT, smem, (cudaStream_t)stream>>>(
+        theta, img, obs, norm, clip, R, D, A, obs_out, logits, value, eps, action, logp, node_id, coupling, status);
+    DDRL_CHECK_LAUNCH(who);
     return DDRL_OK;
 }
 
@@ -433,20 +452,8 @@ extern "C" int ddrl_fcnet_forward(const float* theta, const float* img, const fl
                  "fcnet_forward: unsupported D=%d A=%d (D<=%d, A<=%d, hiddens [64,64], tanh)", D, A, DDRL_MAX_OBS,
                  DDRL_MAX_ACT);
     DDRL_REQUIRE(!eps || (action && logp), DDRL_E_BADARG, "fcnet_forward: eps given without action/logp outputs");
-    if (R == 0) return DDRL_OK;
-    const FcSmem L = fc_smem(D, A, norm != nullptr);
-    const size_t smem = (size_t)L.total * sizeof(float);
-    DDRL_REQUIRE(smem <= 227 * 1024, DDRL_E_UNSUPPORTED_SHAPE, "fcnet_forward: shared memory %zu > 227 KB", smem);
-    static bool attr_set = false;
-    if (int rc = set_smem_attr((const void*)fcnet_forward_kernel<false>, &attr_set, "fcnet_forward")) return rc;
-    const int64_t ntiles = (R + TM - 1) / TM;
-    const int per_policy = (int)std::min<int64_t>(ntiles, std::max(1, num_sms() / P));
-    dim3 grid(per_policy, P);
-    fcnet_forward_kernel<false><<<grid, NT, smem, (cudaStream_t)stream>>>(theta, img, obs, norm, clip, R, D, A, obs_out,
-                                                                          logits, value, eps, action, logp, nullptr,
-                                                                          nullptr, nullptr);
-    DDRL_CHECK_LAUNCH("fcnet_forward");
-    return DDRL_OK;
+    return fcnet_forward_launch<false>("fcnet_forward", theta, img, obs, norm, clip, P, R, D, A, obs_out, logits, value, eps,
+                                       action, logp, nullptr, nullptr, nullptr, stream);
 }
 
 extern "C" int ddrl_fcnet_forward_coupled(const float* theta, const float* img, const int32_t* node_id, const float* coupling,
@@ -459,18 +466,8 @@ extern "C" int ddrl_fcnet_forward_coupled(const float* theta, const float* img, 
     DDRL_REQUIRE(P == 1, DDRL_E_BADARG, "fcnet_forward_coupled: the coupled model is one shared policy (P = 1), got P=%d", P);
     DDRL_REQUIRE(D >= 1 && D <= DDRL_MAX_OBS, DDRL_E_UNSUPPORTED_SHAPE, "fcnet_forward_coupled: unsupported D=%d", D);
     DDRL_REQUIRE(!eps || (action && logp), DDRL_E_BADARG, "fcnet_forward_coupled: eps given without action/logp outputs");
-    if (R == 0) return DDRL_OK;
-    const FcSmem L = fc_smem(D, A, norm != nullptr);
-    const size_t smem = (size_t)L.total * sizeof(float);
-    DDRL_REQUIRE(smem <= 227 * 1024, DDRL_E_UNSUPPORTED_SHAPE, "fcnet_forward_coupled: shared memory %zu > 227 KB", smem);
-    static bool attr_set = false;
-    if (int rc = set_smem_attr((const void*)fcnet_forward_kernel<true>, &attr_set, "fcnet_forward_coupled")) return rc;
-    const int64_t ntiles = (R + TM - 1) / TM;
-    const int per_policy = (int)std::min<int64_t>(ntiles, std::max(1, num_sms()));
-    fcnet_forward_kernel<true><<<dim3(per_policy, 1), NT, smem, (cudaStream_t)stream>>>(
-        theta, img, obs, norm, clip, R, D, A, obs_out, logits, value, eps, action, logp, node_id, coupling, status);
-    DDRL_CHECK_LAUNCH("fcnet_forward_coupled");
-    return DDRL_OK;
+    return fcnet_forward_launch<true>("fcnet_forward_coupled", theta, img, obs, norm, clip, P, R, D, A, obs_out, logits, value,
+                                      eps, action, logp, node_id, coupling, status, stream);
 }
 
 extern "C" int ddrl_ppo_train_step(const float* theta, const float* img, const float* obs, const float* actions,
@@ -488,29 +485,20 @@ extern "C" int ddrl_ppo_train_step(const float* theta, const float* img, const f
     DDRL_REQUIRE(ext ? (ext_dvalue != nullptr)
                      : (actions && old_logits && old_logp && vf_preds && adv && vtarg && kl_coeff && hyper),
                  DDRL_E_BADARG, "ppo_train_step: missing batch arrays for the %s path", ext ? "external-gradient" : "PPO");
-    TrainArgs a;
-    a.theta = theta; a.img = img; a.obs = obs; a.actions = actions; a.old_logits = old_logits; a.old_logp = old_logp;
-    a.vf_preds = vf_preds; a.adv = adv; a.vtarg = vtarg; a.ext_dlogits = ext_dlogits; a.ext_dvalue = ext_dvalue;
-    a.R = R; a.D = D; a.A = A; a.MB = MB; a.mb_perm = mb_perm; a.perm_stride = perm_stride; a.step_ctr = step_ctr;
-    a.kl_coeff = kl_coeff;
-    if (hyper) a.hp = *hyper; else a.hp = ddrl_ppo_hyper{0.f, 0.f, 0.f, 0.f, 1.f};
-    a.grad_part = grad_part; a.stat_part = stat_part;
-    a.tail = SgdTail{};
     if (tail) {
         DDRL_REQUIRE(!ext, DDRL_E_BADARG, "ppo_train_step: the fused tail cannot be combined with external gradients");
         const int rc = sgd_tail_check(tail, ctas_per_policy * P, "ppo_train_step");
         if (rc != DDRL_OK) return rc;
         DDRL_REQUIRE(tail->nsteps <= 1, DDRL_E_UNSUPPORTED_SHAPE, "ppo_train_step: nsteps > 1 is not supported by the FP32 kernel");
-        a.tail = *tail;
-        a.tail.grad_acc = nullptr;      // (accumulation vector: ping-pong tcgen05 kernel only; this kernel writes per-CTA partials)
     }
-    const FcSmem L = fc_smem(D, A, false, true);
-    const size_t smem = (size_t)L.total * sizeof(float);
-    DDRL_REQUIRE(smem <= 227 * 1024, DDRL_E_UNSUPPORTED_SHAPE, "ppo_train_step: shared memory %zu > 227 KB", smem);
-    static bool attr_set = false;
-    if (int rc = set_smem_attr((const void*)fcnet_train_kernel, &attr_set, "ppo_train_step")) return rc;
-    dim3 grid(ctas_per_policy, P);
-    fcnet_train_kernel<<<grid, NT, smem, (cudaStream_t)stream>>>(a);
+    TrainArgs a;
+    size_t smem = 0;
+    if (int rc = fp32_train_args(a, smem, "ppo_train_step", theta, img, obs, actions, old_logits, old_logp, vf_preds, adv, vtarg,
+                                 ext_dlogits, ext_dvalue, R, D, A, MB, mb_perm, perm_stride, step_ctr, kl_coeff, hyper,
+                                 grad_part, stat_part, tail))
+        return rc;
+    if (int rc = raise_smem_once<fcnet_train_kernel>("ppo_train_step")) return rc;
+    fcnet_train_kernel<<<dim3(ctas_per_policy, P), NT, smem, (cudaStream_t)stream>>>(a);
     DDRL_CHECK_LAUNCH("ppo_train_step");
     return DDRL_OK;
 }

@@ -721,4 +721,13 @@ inline int sgd_tail_check(const ddrl_sgd_tail* tail, int ctas_total, const char*
     return DDRL_OK;
 }
 
+// The tail descriptor one launch receives (SgdTail{}: no fused tail).  Only a kernel that ADDS its partial gradient into
+// the accumulation vector keeps grad_acc: the ping-pong tcgen05 step without thread-block clusters and without the LL tail
+// (`pingpong_unclustered`).  Every other kernel writes per-CTA partials, which the tail must then read.
+inline SgdTail launch_tail(const ddrl_sgd_tail* tail, bool pingpong_unclustered) {
+    SgdTail t = tail ? *tail : SgdTail{};
+    if (!pingpong_unclustered || t.ll_ws) t.grad_acc = nullptr;
+    return t;
+}
+
 }  // namespace ddrl

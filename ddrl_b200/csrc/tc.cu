@@ -680,15 +680,35 @@ extern "C" int ddrl_tc_set_variant(int variant) {
 
 template <int A>
 static int launch_tc(const TcTrainArgs& a, int P, int G, size_t smem, cudaStream_t st) {
-    static bool attr = false;
-    if (!attr) {
-        if (cudaFuncSetAttribute(fcnet_train_tc_kernel<A>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess) {
-            set_error("ppo_train_step_tc: cannot raise dynamic shared memory: %s", cudaGetErrorString(cudaGetLastError()));
-            return DDRL_E_CUDA;
-        }
-        attr = true;
-    }
+    if (int rc = raise_smem_once<fcnet_train_tc_kernel<A>>("ppo_train_step_tc")) return rc;
     fcnet_train_tc_kernel<A><<<dim3(G, P), TC_NT, smem, st>>>(a);
+    return DDRL_OK;
+}
+
+// What the two tensor-core train steps share: the pointer and P/R/MB/ctas check, then the entry's own checks
+// (`entry_checks`), the weight-image alignment, the fused-tail check, and the TcTrainArgs fields (dbg_clock stays null).
+// `pingpong`: the step runs on the ping-pong kernel (the only one that can keep the accumulation vector, launch_tail).
+template <class EntryChecks>
+static int tc_train_args(TcTrainArgs& a, const char* who, bool entry_ptrs, EntryChecks&& entry_checks, bool pingpong,
+                         const void* tc_img_p, const float* obs, const float* actions, const float* old_logits,
+                         const float* old_logp, const float* vf_preds, const float* adv, const float* vtarg, int P, int64_t R,
+                         int D, int A, int MB, const int32_t* mb_perm, int64_t perm_stride, const int32_t* step_ctr,
+                         const float* kl_coeff, const ddrl_ppo_hyper* hyper, int ctas_per_policy, float* grad_part,
+                         double* stat_part, int* status, const ddrl_sgd_tail* tail) {
+    DDRL_REQUIRE(entry_ptrs && tc_img_p && obs && actions && old_logits && old_logp && vf_preds && adv && vtarg && kl_coeff &&
+                     hyper && grad_part && P >= 1 && R >= 1 && MB >= 1 && ctas_per_policy >= 1,
+                 DDRL_E_BADARG, "%s: null pointer or bad P/R/MB/ctas", who);
+    if (int rc = entry_checks()) return rc;
+    DDRL_REQUIRE((reinterpret_cast<uintptr_t>(tc_img_p) & 15) == 0, DDRL_E_BADARG,
+                 "%s: the weight image must be 16-byte aligned (TMA bulk copies)", who);
+    if (tail)
+        if (int rc = sgd_tail_check(tail, ctas_per_policy * P, who)) return rc;
+    a = TcTrainArgs{};
+    a.img = (const unsigned char*)tc_img_p; a.obs = obs; a.actions = actions; a.old_logits = old_logits;
+    a.old_logp = old_logp; a.vf_preds = vf_preds; a.adv = adv; a.vtarg = vtarg; a.R = R; a.D = D; a.A = A; a.MB = MB;
+    a.mb_perm = mb_perm; a.perm_stride = perm_stride; a.step_ctr = step_ctr; a.kl_coeff = kl_coeff; a.hp = *hyper;
+    a.grad_part = grad_part; a.stat_part = stat_part; a.status = status;
+    a.tail = launch_tail(tail, pingpong && !tc2_clusters_requested());
     return DDRL_OK;
 }
 
@@ -698,49 +718,36 @@ extern "C" int ddrl_ppo_train_step_tc(const void* tc_img_p, const float* obs, co
                                       const int32_t* step_ctr, const float* kl_coeff, const ddrl_ppo_hyper* hyper,
                                       int ctas_per_policy, float* grad_part, double* stat_part, int* status,
                                       const ddrl_sgd_tail* tail, void* stream) {
-    DDRL_REQUIRE(tc_img_p && obs && actions && old_logits && old_logp && vf_preds && adv && vtarg && kl_coeff && hyper &&
-                     grad_part && P >= 1 && R >= 1 && MB >= 1 && ctas_per_policy >= 1,
-                 DDRL_E_BADARG, "ppo_train_step_tc: null pointer or bad P/R/MB/ctas");
-    DDRL_REQUIRE(D >= 1 && D <= DDRL_MAX_OBS - 1 && (A == 1 || A == 2 || A == 4 || A == 8), DDRL_E_UNSUPPORTED_SHAPE,
-                 "ppo_train_step_tc: unsupported D=%d A=%d (A in {1,2,4,8}, D <= 63)", D, A);
+    const char* who = "ppo_train_step_tc";
+    const bool pingpong = g_tc_variant == 2 || (g_tc_variant == 0 && tc2_eligible(D, A));
     TcTrainArgs a;
-    DDRL_REQUIRE((reinterpret_cast<uintptr_t>(tc_img_p) & 15) == 0, DDRL_E_BADARG, "ppo_train_step_tc: the weight image must be 16-byte aligned (TMA bulk copies)");
-    a.img = (const unsigned char*)tc_img_p; a.obs = obs; a.actions = actions; a.old_logits = old_logits;
-    a.old_logp = old_logp; a.vf_preds = vf_preds; a.adv = adv; a.vtarg = vtarg; a.R = R; a.D = D; a.A = A; a.MB = MB;
-    a.mb_perm = mb_perm; a.perm_stride = perm_stride; a.step_ctr = step_ctr; a.kl_coeff = kl_coeff; a.hp = *hyper;
-    a.grad_part = grad_part; a.stat_part = stat_part; a.status = status;
+    const int rc = tc_train_args(
+        a, who, true,
+        [&]() -> int {
+            DDRL_REQUIRE(D >= 1 && D <= DDRL_MAX_OBS - 1 && (A == 1 || A == 2 || A == 4 || A == 8), DDRL_E_UNSUPPORTED_SHAPE,
+                         "ppo_train_step_tc: unsupported D=%d A=%d (A in {1,2,4,8}, D <= 63)", D, A);
+            return DDRL_OK;
+        },
+        pingpong, tc_img_p, obs, actions, old_logits, old_logp, vf_preds, adv, vtarg, P, R, D, A, MB, mb_perm, perm_stride,
+        step_ctr, kl_coeff, hyper, ctas_per_policy, grad_part, stat_part, status, tail);
+    if (rc != DDRL_OK) return rc;
     a.dbg_clock = g_tc_dbg_clock;
-    a.norm = nullptr; a.clip = 0.f; a.obs_out = a.logits_out = a.value_out = a.action_out = a.logp_out = nullptr; a.eps = nullptr;
-    a.tail = SgdTail{};
-    if (tail) {
-        const int rc = sgd_tail_check(tail, ctas_per_policy * P, "ppo_train_step_tc");
-        if (rc != DDRL_OK) return rc;
-        a.tail = *tail;
-        const bool pp = g_tc_variant == 2 || (g_tc_variant == 0 && tc2_eligible(D, A));
-        DDRL_REQUIRE(tail->nsteps <= 1 || pp, DDRL_E_UNSUPPORTED_SHAPE,
-                     "ppo_train_step_tc: nsteps > 1 needs the ping-pong kernel (D <= 47)");
-    }
+    DDRL_REQUIRE(!tail || tail->nsteps <= 1 || pingpong, DDRL_E_UNSUPPORTED_SHAPE,
+                 "ppo_train_step_tc: nsteps > 1 needs the ping-pong kernel (D <= 47)");
     const size_t smem = (size_t)tc_smem(D, A).total;
     DDRL_REQUIRE(smem <= 227 * 1024, DDRL_E_UNSUPPORTED_SHAPE, "ppo_train_step_tc: shared memory %zu > 227 KB", smem);
-    int rc;
-    const bool pingpong = g_tc_variant == 2 || (g_tc_variant == 0 && tc2_eligible(D, A));
+    int lrc;
     if (pingpong) {
         DDRL_REQUIRE(tc2_eligible(D, A), DDRL_E_UNSUPPORTED_SHAPE,
                      "ppo_train_step_tc: ping-pong variant needs D <= 47 (D=%d, A=%d)", D, A);
-        rc = launch_tc2(a, P, ctas_per_policy, (cudaStream_t)stream);
-        if (rc != DDRL_OK) return rc;
-        DDRL_CHECK_LAUNCH("ppo_train_step_tc");
-        return DDRL_OK;
+        lrc = launch_tc2(a, P, ctas_per_policy, (cudaStream_t)stream);
+    } else {
+        lrc = dispatch_A(A, "ppo_train_step_tc: unsupported A", [&](auto A_) {
+            return launch_tc<decltype(A_)::value>(a, P, ctas_per_policy, smem, (cudaStream_t)stream);
+        });
     }
-    a.tail.grad_acc = nullptr;      // the branch-sequential kernel writes per-CTA partials
-    switch (A) {
-        case 1: rc = launch_tc<1>(a, P, ctas_per_policy, smem, (cudaStream_t)stream); break;
-        case 2: rc = launch_tc<2>(a, P, ctas_per_policy, smem, (cudaStream_t)stream); break;
-        case 4: rc = launch_tc<4>(a, P, ctas_per_policy, smem, (cudaStream_t)stream); break;
-        default: rc = launch_tc<8>(a, P, ctas_per_policy, smem, (cudaStream_t)stream); break;
-    }
-    if (rc != DDRL_OK) return rc;
-    DDRL_CHECK_LAUNCH("ppo_train_step_tc");
+    if (lrc != DDRL_OK) return lrc;
+    DDRL_CHECK_LAUNCH(who);
     return DDRL_OK;
 }
 
@@ -751,33 +758,51 @@ extern "C" int ddrl_ppo_train_step_tc_coupled(const void* tc_img_p, const float*
                                               const int32_t* step_ctr, const float* kl_coeff, const ddrl_ppo_hyper* hyper,
                                               int ctas_per_policy, float* grad_part, double* stat_part, int* status,
                                               const ddrl_sgd_tail* tail, void* stream) {
-    DDRL_REQUIRE(tc_img_p && theta && node_id && obs && actions && old_logits && old_logp && vf_preds && adv && vtarg && kl_coeff &&
-                     hyper && grad_part && P >= 1 && R >= 1 && MB >= 1 && ctas_per_policy >= 1,
-                 DDRL_E_BADARG, "ppo_train_step_tc_coupled: null pointer or bad P/R/MB/ctas");
-    DDRL_REQUIRE(A == 2, DDRL_E_BADARG, "ppo_train_step_tc_coupled: LegCoupling needs A = 2 (num_outputs == 4), got A=%d", A);
-    DDRL_REQUIRE(P == 1, DDRL_E_BADARG, "ppo_train_step_tc_coupled: the coupled model is one shared policy (P = 1), got P=%d", P);
-    DDRL_REQUIRE(D == 19 || D == 20, DDRL_E_UNSUPPORTED_SHAPE,
-                 "ppo_train_step_tc_coupled: instantiated for SharedDecentralLegID (D = 19 or 20), got D=%d", D);
-    DDRL_REQUIRE(tail != nullptr, DDRL_E_BADARG, "ppo_train_step_tc_coupled: the fused tail is required (NP + 8 parameters)");
-    DDRL_REQUIRE(tail->theta == theta, DDRL_E_BADARG, "ppo_train_step_tc_coupled: tail->theta must be theta");
-    DDRL_REQUIRE(status != nullptr, DDRL_E_BADARG,
-                 "ppo_train_step_tc_coupled: status is required (it receives DDRL_STATUS_BAD_NODE for a node id outside 0..3)");
-    DDRL_REQUIRE(!tail->ll_ws, DDRL_E_BADARG, "ppo_train_step_tc_coupled: the LL tail is not supported with leg coupling");
-    DDRL_REQUIRE(g_tc_variant != 1, DDRL_E_BADARG,
-                 "ppo_train_step_tc_coupled: only the ping-pong kernel has a coupled instantiation (ddrl_tc_set_variant(1) is set)");
-    DDRL_REQUIRE((reinterpret_cast<uintptr_t>(tc_img_p) & 15) == 0, DDRL_E_BADARG,
-                 "ppo_train_step_tc_coupled: the weight image must be 16-byte aligned (TMA bulk copies)");
-    const int rc0 = sgd_tail_check(tail, ctas_per_policy * P, "ppo_train_step_tc_coupled");
-    if (rc0 != DDRL_OK) return rc0;
-    TcTrainArgs a = {};
-    a.img = (const unsigned char*)tc_img_p; a.obs = obs; a.actions = actions; a.old_logits = old_logits;
-    a.old_logp = old_logp; a.vf_preds = vf_preds; a.adv = adv; a.vtarg = vtarg; a.R = R; a.D = D; a.A = A; a.MB = MB;
-    a.mb_perm = mb_perm; a.perm_stride = perm_stride; a.step_ctr = step_ctr; a.kl_coeff = kl_coeff; a.hp = *hyper;
-    a.grad_part = grad_part; a.stat_part = stat_part; a.status = status; a.dbg_clock = nullptr;
-    a.tail = *tail;
-    const int rc = launch_tc2_cup(a, node_id, theta, P, ctas_per_policy, (cudaStream_t)stream);
+    const char* who = "ppo_train_step_tc_coupled";
+    TcTrainArgs a;
+    const int rc = tc_train_args(
+        a, who, theta && node_id,
+        [&]() -> int {
+            DDRL_REQUIRE(A == 2, DDRL_E_BADARG, "ppo_train_step_tc_coupled: LegCoupling needs A = 2 (num_outputs == 4), got A=%d", A);
+            DDRL_REQUIRE(P == 1, DDRL_E_BADARG,
+                         "ppo_train_step_tc_coupled: the coupled model is one shared policy (P = 1), got P=%d", P);
+            DDRL_REQUIRE(D == 19 || D == 20, DDRL_E_UNSUPPORTED_SHAPE,
+                         "ppo_train_step_tc_coupled: instantiated for SharedDecentralLegID (D = 19 or 20), got D=%d", D);
+            DDRL_REQUIRE(tail != nullptr, DDRL_E_BADARG, "ppo_train_step_tc_coupled: the fused tail is required (NP + 8 parameters)");
+            DDRL_REQUIRE(tail->theta == theta, DDRL_E_BADARG, "ppo_train_step_tc_coupled: tail->theta must be theta");
+            DDRL_REQUIRE(status != nullptr, DDRL_E_BADARG,
+                         "ppo_train_step_tc_coupled: status is required (it receives DDRL_STATUS_BAD_NODE for a node id outside 0..3)");
+            DDRL_REQUIRE(!tail->ll_ws, DDRL_E_BADARG, "ppo_train_step_tc_coupled: the LL tail is not supported with leg coupling");
+            DDRL_REQUIRE(g_tc_variant != 1, DDRL_E_BADARG,
+                         "ppo_train_step_tc_coupled: only the ping-pong kernel has a coupled instantiation (ddrl_tc_set_variant(1) is set)");
+            return DDRL_OK;
+        },
+        true, tc_img_p, obs, actions, old_logits, old_logp, vf_preds, adv, vtarg, P, R, D, A, MB, mb_perm, perm_stride,
+        step_ctr, kl_coeff, hyper, ctas_per_policy, grad_part, stat_part, status, tail);
     if (rc != DDRL_OK) return rc;
-    DDRL_CHECK_LAUNCH("ppo_train_step_tc_coupled");
+    const int lrc = launch_tc2_cup(a, node_id, theta, P, ctas_per_policy, (cudaStream_t)stream);
+    if (lrc != DDRL_OK) return lrc;
+    DDRL_CHECK_LAUNCH(who);
+    return DDRL_OK;
+}
+
+// The alignment check, TcTrainArgs and grid of the two tensor-core forwards: G CTAs per policy, at most sms / P of them.
+static int tc_forward_args(TcTrainArgs& a, int& G, const char* who, const void* tc_img_p, const float* obs, const double* norm,
+                           float clip, int P, int64_t R, int D, int A, float* obs_out, float* logits, float* value,
+                           const float* eps, float* action, float* logp, int* status) {
+    DDRL_REQUIRE(R <= 0x7fffffff, DDRL_E_UNSUPPORTED_SHAPE, "%s: R must fit 31 bits", who);
+    DDRL_REQUIRE((reinterpret_cast<uintptr_t>(tc_img_p) & 15) == 0, DDRL_E_BADARG,
+                 "%s: the weight image must be 16-byte aligned (TMA bulk copies)", who);
+    a = TcTrainArgs{};
+    a.img = (const unsigned char*)tc_img_p; a.obs = obs; a.R = R; a.D = D; a.A = A; a.MB = (int)R;
+    a.hp = ddrl_ppo_hyper{0.f, 0.f, 0.f, 0.f, 1.f};
+    a.status = status;
+    a.norm = norm; a.clip = clip; a.obs_out = obs_out; a.logits_out = logits; a.value_out = value; a.eps = eps;
+    a.action_out = action; a.logp_out = logp;
+    int dev = 0, sms = 0;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    G = (int)std::max<int64_t>(1, std::min<int64_t>((R + TC_ROWS - 1) / TC_ROWS, std::max(1, sms / P)));
     return DDRL_OK;
 }
 
@@ -788,20 +813,13 @@ extern "C" int ddrl_fcnet_forward_tc(const void* tc_img_p, const float* obs, con
     DDRL_REQUIRE(!eps || (action && logp), DDRL_E_BADARG, "fcnet_forward_tc: eps given without action / logp outputs");
     DDRL_REQUIRE(D >= 1 && D <= DDRL_MAX_OBS - 1 && (A == 1 || A == 2 || A == 4 || A == 8) && tc2_eligible(D, A),
                  DDRL_E_UNSUPPORTED_SHAPE, "fcnet_forward_tc: unsupported D=%d A=%d (A in {1,2,4,8}, D <= 47)", D, A);
-    DDRL_REQUIRE(R <= 0x7fffffff, DDRL_E_UNSUPPORTED_SHAPE, "fcnet_forward_tc: R must fit 31 bits");
     if (R == 0) return DDRL_OK;
-    TcTrainArgs a = {};
-    DDRL_REQUIRE((reinterpret_cast<uintptr_t>(tc_img_p) & 15) == 0, DDRL_E_BADARG, "fcnet_forward_tc: the weight image must be 16-byte aligned (TMA bulk copies)");
-    a.img = (const unsigned char*)tc_img_p; a.obs = obs; a.R = R; a.D = D; a.A = A; a.MB = (int)R;
-    a.hp = ddrl_ppo_hyper{0.f, 0.f, 0.f, 0.f, 1.f};
-    a.status = status; a.dbg_clock = nullptr; a.tail = SgdTail{};
-    a.norm = norm; a.clip = clip; a.obs_out = obs_out; a.logits_out = logits; a.value_out = value; a.eps = eps;
-    a.action_out = action; a.logp_out = logp;
-    int dev = 0, sms = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    const int G = (int)std::max<int64_t>(1, std::min<int64_t>((R + TC_ROWS - 1) / TC_ROWS, std::max(1, sms / P)));
-    const int rc = launch_tc2_forward(a, P, G, (cudaStream_t)stream);
+    TcTrainArgs a;
+    int G = 0;
+    int rc = tc_forward_args(a, G, "fcnet_forward_tc", tc_img_p, obs, norm, clip, P, R, D, A, obs_out, logits, value, eps,
+                             action, logp, status);
+    if (rc != DDRL_OK) return rc;
+    rc = launch_tc2_forward(a, P, G, (cudaStream_t)stream);
     if (rc != DDRL_OK) return rc;
     DDRL_CHECK_LAUNCH("fcnet_forward_tc");
     return DDRL_OK;
@@ -818,21 +836,12 @@ extern "C" int ddrl_fcnet_forward_tc_coupled(const void* tc_img_p, const int32_t
     DDRL_REQUIRE(!eps || (action && logp), DDRL_E_BADARG, "fcnet_forward_tc_coupled: eps given without action / logp outputs");
     DDRL_REQUIRE(D == 19 || D == 20, DDRL_E_UNSUPPORTED_SHAPE,
                  "fcnet_forward_tc_coupled: instantiated for SharedDecentralLegID (D = 19 or 20), got D=%d", D);
-    DDRL_REQUIRE(R <= 0x7fffffff, DDRL_E_UNSUPPORTED_SHAPE, "fcnet_forward_tc_coupled: R must fit 31 bits");
-    DDRL_REQUIRE((reinterpret_cast<uintptr_t>(tc_img_p) & 15) == 0, DDRL_E_BADARG,
-                 "fcnet_forward_tc_coupled: the weight image must be 16-byte aligned (TMA bulk copies)");
-    if (R == 0) return DDRL_OK;
-    TcTrainArgs a = {};
-    a.img = (const unsigned char*)tc_img_p; a.obs = obs; a.R = R; a.D = D; a.A = A; a.MB = (int)R;
-    a.hp = ddrl_ppo_hyper{0.f, 0.f, 0.f, 0.f, 1.f};
-    a.status = status; a.dbg_clock = nullptr; a.tail = SgdTail{};
-    a.norm = norm; a.clip = clip; a.obs_out = obs_out; a.logits_out = logits; a.value_out = value; a.eps = eps;
-    a.action_out = action; a.logp_out = logp;
-    int dev = 0, sms = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    const int G = (int)std::max<int64_t>(1, std::min<int64_t>((R + TC_ROWS - 1) / TC_ROWS, std::max(1, sms)));
-    const int rc = launch_tc2_forward_cup(a, node_id, coupling, G, (cudaStream_t)stream);
+    TcTrainArgs a;
+    int G = 0;
+    int rc = tc_forward_args(a, G, "fcnet_forward_tc_coupled", tc_img_p, obs, norm, clip, P, R, D, A, obs_out, logits, value, eps,
+                             action, logp, status);
+    if (rc != DDRL_OK || R == 0) return rc;
+    rc = launch_tc2_forward_cup(a, node_id, coupling, G, (cudaStream_t)stream);
     if (rc != DDRL_OK) return rc;
     DDRL_CHECK_LAUNCH("fcnet_forward_tc_coupled");
     return DDRL_OK;

@@ -213,16 +213,13 @@ static int g_tc2_cluster = 0;    // 0 = off (default: measured slower, DESIGN.md
 
 template <int A, bool FWD, bool LL, int DT = 0, bool DBG = false>
 static int launch_tc2_t(const TcTrainArgs& a, int P, int G, size_t smem, cudaStream_t st, int* used_cluster) {
-    static bool attr = false;
-    auto kern = fcnet_train_tc2_kernel<A, FWD, LL, DT, DBG>;
-    if (!attr) {
-        if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess) {
-            set_error("ppo_train_step_tc: cannot raise dynamic shared memory: %s", cudaGetErrorString(cudaGetLastError()));
-            return DDRL_E_CUDA;
-        }
+    constexpr auto kern = fcnet_train_tc2_kernel<A, FWD, LL, DT, DBG>;
+    if (int rc = raise_smem_once<kern>("ppo_train_step_tc")) return rc;
+    static bool cluster_attr = false;
+    if (!cluster_attr) {
         cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);   // clusters of 16 (opt-in size)
         cudaGetLastError();
-        attr = true;
+        cluster_attr = true;
     }
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(G, P);
@@ -264,51 +261,33 @@ static int launch_tc2_t(const TcTrainArgs& a, int P, int G, size_t smem, cudaStr
 
 static int g_tc2_last_cluster = 0;
 
-int launch_tc2(const TcTrainArgs& a_in, int P, int G, cudaStream_t st) {
-    TcTrainArgs a = a_in;
-    if (g_tc2_cluster != 0 || a.tail.ll_ws) a.tail.grad_acc = nullptr;   // the accumulation vector is the plain staged path's
+bool tc2_clusters_requested() { return g_tc2_cluster != 0; }
+
+int launch_tc2(const TcTrainArgs& a, int P, int G, cudaStream_t st) {
     const size_t smem = (size_t)tc2_smem(a.D, a.A).total;
+    int* const used = &g_tc2_last_cluster;
+    const char* const unsupported = "ppo_train_step_tc: ping-pong kernel supports A in {1,2,4,8}";
     // LL tail: fused tail with an LL workspace, no thread-block clusters requested, one slice element per thread
-    const bool ll = a.tail.theta && a.tail.ll_ws && g_tc2_cluster == 0 && sgd_slice_len(fc_offsets(a.D, a.A).NP, G) <= T2_NT;
-    if (ll) {
-        switch (a.A) {
-            case 1: return launch_tc2_t<1, false, true>(a, P, G, smem, st, &g_tc2_last_cluster);
-            case 2: return launch_tc2_t<2, false, true>(a, P, G, smem, st, &g_tc2_last_cluster);
-            case 4: return launch_tc2_t<4, false, true>(a, P, G, smem, st, &g_tc2_last_cluster);
-            case 8: return launch_tc2_t<8, false, true>(a, P, G, smem, st, &g_tc2_last_cluster);
-            default: set_error("ppo_train_step_tc: ping-pong kernel supports A in {1,2,4,8}"); return DDRL_E_UNSUPPORTED_SHAPE;
-        }
-    }
+    if (a.tail.theta && a.tail.ll_ws && g_tc2_cluster == 0 && sgd_slice_len(fc_offsets(a.D, a.A).NP, G) <= T2_NT)
+        return dispatch_A(a.A, unsupported,
+                          [&](auto A_) { return launch_tc2_t<decltype(A_)::value, false, true>(a, P, G, smem, st, used); });
     // the published architectures (policies.ARCHITECTURES: obs width with / without the target velocity, action width)
-    if (a.dbg_clock && a.D == 19 && a.A == 2) return launch_tc2_t<2, false, false, 19, true>(a, P, G, smem, st, &g_tc2_last_cluster);
+    if (a.dbg_clock && a.D == 19 && a.A == 2) return launch_tc2_t<2, false, false, 19, true>(a, P, G, smem, st, used);
 #define T2_PUBLISHED(DD, AA) \
-    if (a.D == DD && a.A == AA) return launch_tc2_t<AA, false, false, DD>(a, P, G, smem, st, &g_tc2_last_cluster);
+    if (a.D == DD && a.A == AA) return launch_tc2_t<AA, false, false, DD>(a, P, G, smem, st, used);
     T2_PUBLISHED(19, 2) T2_PUBLISHED(20, 2) T2_PUBLISHED(27, 2) T2_PUBLISHED(28, 2) T2_PUBLISHED(35, 2) T2_PUBLISHED(36, 2)
     T2_PUBLISHED(27, 4) T2_PUBLISHED(28, 4) T2_PUBLISHED(43, 8) T2_PUBLISHED(44, 8)
 #undef T2_PUBLISHED
-    switch (a.A) {
-        case 1: return launch_tc2_t<1, false, false>(a, P, G, smem, st, &g_tc2_last_cluster);
-        case 2: return launch_tc2_t<2, false, false>(a, P, G, smem, st, &g_tc2_last_cluster);
-        case 4: return launch_tc2_t<4, false, false>(a, P, G, smem, st, &g_tc2_last_cluster);
-        case 8: return launch_tc2_t<8, false, false>(a, P, G, smem, st, &g_tc2_last_cluster);
-        default: set_error("ppo_train_step_tc: ping-pong kernel supports A in {1,2,4,8}"); return DDRL_E_UNSUPPORTED_SHAPE;
-    }
+    return dispatch_A(a.A, unsupported,
+                      [&](auto A_) { return launch_tc2_t<decltype(A_)::value, false, false>(a, P, G, smem, st, used); });
 }
 
 // leg-coupled step: no clusters, no LL tail (the entry point rejects both); instantiated for SharedDecentralLegID's D = 19, 20
 template <int DT>
 static int launch_tc2_cup_t(const TcTrainArgs& a, const int32_t* node_id, const float* theta, int P, int G, cudaStream_t st) {
-    static bool attr = false;
-    auto kern = fcnet_train_tc2_cup_kernel<DT>;
-    if (!attr) {
-        if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess) {
-            set_error("ppo_train_step_tc_coupled: cannot raise dynamic shared memory: %s", cudaGetErrorString(cudaGetLastError()));
-            return DDRL_E_CUDA;
-        }
-        attr = true;
-    }
+    if (int rc = raise_smem_once<fcnet_train_tc2_cup_kernel<DT>>("ppo_train_step_tc_coupled")) return rc;
     const size_t smem = (size_t)tc2_smem(DT, 2, true).total;
-    kern<<<dim3(G, P), T2_NT, smem, st>>>(a, node_id, theta);
+    fcnet_train_tc2_cup_kernel<DT><<<dim3(G, P), T2_NT, smem, st>>>(a, node_id, theta);
     g_tc2_last_cluster = 1;
     return DDRL_OK;
 }
@@ -325,14 +304,7 @@ int launch_tc2_cup(const TcTrainArgs& a, const int32_t* node_id, const float* th
 }
 
 int launch_tc2_forward_cup(const TcTrainArgs& a, const int32_t* node_id, const float* coupling, int G, cudaStream_t st) {
-    static bool attr = false;
-    if (!attr) {
-        if (cudaFuncSetAttribute(fcnet_forward_tc2_cup_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess) {
-            set_error("fcnet_forward_tc_coupled: cannot raise dynamic shared memory: %s", cudaGetErrorString(cudaGetLastError()));
-            return DDRL_E_CUDA;
-        }
-        attr = true;
-    }
+    if (int rc = raise_smem_once<fcnet_forward_tc2_cup_kernel>("fcnet_forward_tc_coupled")) return rc;
     fcnet_forward_tc2_cup_kernel<<<dim3(G, 1), T2_NT, (size_t)tc2_smem(a.D, 2, true).total, st>>>(a, node_id, coupling);
     return DDRL_OK;
 }
@@ -340,13 +312,8 @@ int launch_tc2_forward_cup(const TcTrainArgs& a, const int32_t* node_id, const f
 int launch_tc2_forward(const TcTrainArgs& a, int P, int G, cudaStream_t st) {
     const size_t smem = (size_t)tc2_smem(a.D, a.A).total;
     int dummy = 0;
-    switch (a.A) {
-        case 1: return launch_tc2_t<1, true, false>(a, P, G, smem, st, &dummy);
-        case 2: return launch_tc2_t<2, true, false>(a, P, G, smem, st, &dummy);
-        case 4: return launch_tc2_t<4, true, false>(a, P, G, smem, st, &dummy);
-        case 8: return launch_tc2_t<8, true, false>(a, P, G, smem, st, &dummy);
-        default: set_error("fcnet_forward_tc: A must be 1, 2, 4 or 8"); return DDRL_E_UNSUPPORTED_SHAPE;
-    }
+    return dispatch_A(a.A, "fcnet_forward_tc: A must be 1, 2, 4 or 8",
+                      [&](auto A_) { return launch_tc2_t<decltype(A_)::value, true, false>(a, P, G, smem, st, &dummy); });
 }
 
 }  // namespace ddrl

@@ -3,6 +3,8 @@
 #pragma once
 #include <cuda_fp16.h>
 
+#include <type_traits>
+
 #include "common.cuh"
 #include "fcnet_tc_layout.cuh"
 #include "ppo_loss.cuh"
@@ -40,6 +42,20 @@ int launch_tc2_forward(const TcTrainArgs& a, int P, int G, cudaStream_t st);
 int launch_tc2_cup(const TcTrainArgs& a, const int32_t* node_id, const float* theta, int P, int G, cudaStream_t st);
 // leg-coupled inference forward (P = 1, A = 2, tc2_eligible D): node_id [R], coupling [4][2]
 int launch_tc2_forward_cup(const TcTrainArgs& a, const int32_t* node_id, const float* coupling, int G, cudaStream_t st);
+// true if ddrl_tc_set_cluster asked for thread-block clusters on the ping-pong step
+bool tc2_clusters_requested();
+
+// launch(std::integral_constant<int, A>) for the action widths the tensor-core kernels are instantiated for, A in {1,2,4,8}
+template <class Launch>
+int dispatch_A(int A, const char* unsupported, Launch&& launch) {
+    switch (A) {
+        case 1: return launch(std::integral_constant<int, 1>{});
+        case 2: return launch(std::integral_constant<int, 2>{});
+        case 4: return launch(std::integral_constant<int, 4>{});
+        case 8: return launch(std::integral_constant<int, 8>{});
+        default: set_error("%s", unsupported); return DDRL_E_UNSUPPORTED_SHAPE;
+    }
+}
 
 // Power-of-two operand scales (see header comment).  What matters is the absolute error relative to the tensor's
 // scale: entries too small for a normal lo half lose at most 2^-25/scale, negligible next to the entries that dominate.

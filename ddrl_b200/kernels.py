@@ -564,17 +564,9 @@ def fcnet_forward_tc(tc_img, obs, A: int, norm=None, clip: float = 0.0, eps=None
     value[, obs_out][, action, logp]).  ``out`` may carry preallocated tensors; a None entry skips that output."""
     P, R, D = obs.shape
     f32 = torch.float32
-    dev = obs.device
-    o = dict(out) if out is not None else {}
-    if out is None:
-        o["logits"] = torch.empty(P, R, 2 * A, dtype=f32, device=dev)
-        o["value"] = torch.empty(P, R, dtype=f32, device=dev)
-        o["obs_out"] = torch.empty(P, R, D, dtype=f32, device=dev) if norm is not None else None
-    if eps is not None:
-        o.setdefault("action", torch.empty(P, R, A, dtype=f32, device=dev))
-        o.setdefault("logp", torch.empty(P, R, dtype=f32, device=dev))
+    o = _forward_outputs(obs, A, eps, out, want_obs_out=norm is not None, samples_only=out is not None)
     if status is None:
-        status = torch.zeros(1, dtype=torch.int32, device=dev)
+        status = torch.zeros(1, dtype=torch.int32, device=obs.device)
     _lib.check(_lib.load().ddrl_fcnet_forward_tc(
         _p(tc_img, torch.uint8, "tc_img"), _p(obs, f32, "obs"), _p(norm, torch.float64, "norm"), float(clip or 0.0), P, R, D, A,
         _p(o.get("obs_out"), f32, "obs_out"), _p(o.get("logits"), f32, "logits"), _p(o.get("value"), f32, "value"),
@@ -584,16 +576,17 @@ def fcnet_forward_tc(tc_img, obs, A: int, norm=None, clip: float = 0.0, eps=None
     return o
 
 
-def _coupled_outputs(obs, A: int, eps, out: Optional[dict], want_obs_out: bool) -> dict:
+def _forward_outputs(obs, A: int, eps, out: Optional[dict], want_obs_out: bool, samples_only: bool = False) -> dict:
+    """Outputs of a forward wrapper: the entries of ``out`` (None skips that output) and a new float32 tensor for each missing
+    one (obs_out only if ``want_obs_out``; with ``samples_only`` only action / logp, and those only when eps is given)."""
     P, R, D = obs.shape
-    f32, dev = torch.float32, obs.device
     o = dict(out) if out is not None else {}
-    shapes = {"logits": (P, R, 2 * A), "value": (P, R), "obs_out": (P, R, D) if want_obs_out else None}
+    shapes = {} if samples_only else {"logits": (P, R, 2 * A), "value": (P, R), "obs_out": (P, R, D) if want_obs_out else None}
     if eps is not None:
         shapes.update(action=(P, R, A), logp=(P, R))
     for k, shp in shapes.items():
         if k not in o:
-            o[k] = torch.empty(shp, dtype=f32, device=dev) if shp is not None else None
+            o[k] = torch.empty(shp, dtype=torch.float32, device=obs.device) if shp is not None else None
     return o
 
 
@@ -606,7 +599,7 @@ def fcnet_forward_coupled(theta, obs, node_id, coupling, A: int = 2, norm=None, 
     0..3 sets STATUS_BAD_NODE in ``status`` (a new zeroed int32 [1] unless given); ``out`` entries set to None are skipped."""
     P, R, D = obs.shape
     f32 = torch.float32
-    o = _coupled_outputs(obs, A, eps, out, want_obs_out)
+    o = _forward_outputs(obs, A, eps, out, want_obs_out)
     if status is None:
         status = torch.zeros(1, dtype=torch.int32, device=obs.device)
     _lib.check(_lib.load().ddrl_fcnet_forward_coupled(
@@ -626,7 +619,7 @@ def fcnet_forward_tc_coupled(tc_img, obs, node_id, coupling, A: int = 2, norm=No
     fcnet_forward_coupled with the tensor-core weight image.  Bit-identical to fcnet_forward_tc -> leg_coupling_ -> dg_sample."""
     P, R, D = obs.shape
     f32 = torch.float32
-    o = _coupled_outputs(obs, A, eps, out, want_obs_out)
+    o = _forward_outputs(obs, A, eps, out, want_obs_out)
     if status is None:
         status = torch.zeros(1, dtype=torch.int32, device=obs.device)
     _lib.check(_lib.load().ddrl_fcnet_forward_tc_coupled(
@@ -657,19 +650,27 @@ def tc_pingpong_eligible(D: int, A: int) -> bool:
     return bool(_lib.load().ddrl_tc_pingpong_eligible(int(D), int(A)))
 
 
-def ppo_train_step_tc(tc_img, obs, actions, old_logits, old_logp, vf_preds, adv, vtarg, A: int, MB: int, mb_perm, step_ctr,
-                      kl_coeff, hyper: PPOHyper, ctas_per_policy: int, grad_part, stat_part, status=None,
-                      tail: Optional[SgdTail] = None):
+def _step_args(obs, actions, old_logits, old_logp, vf_preds, adv, vtarg, A: int, MB: int, mb_perm, step_ctr, kl_coeff,
+               hyper: PPOHyper, ctas_per_policy: int, grad_part, stat_part) -> list:
+    """The arguments obs ... stat_part that ddrl_ppo_train_step_tc, _tc_coupled and ddrl_ppo_train_step_coupled share."""
     P, R, D = obs.shape
     f32 = torch.float32
     perm_stride = mb_perm.shape[-1] if mb_perm is not None else 0
+    return [_p(obs, f32, "obs"), _p(actions, f32, "actions"), _p(old_logits, f32, "old_logits"), _p(old_logp, f32, "old_logp"),
+            _p(vf_preds, f32, "vf_preds"), _p(adv, f32, "adv"), _p(vtarg, f32, "vtarg"), P, R, D, A, MB,
+            _p(mb_perm, torch.int32, "mb_perm"), perm_stride, _p(step_ctr, torch.int32, "step_ctr"),
+            _p(kl_coeff, f32, "kl_coeff"), C.byref(hyper), ctas_per_policy, _p(grad_part, f32, "grad_part"),
+            _p(stat_part, torch.float64, "stat_part")]
+
+
+def ppo_train_step_tc(tc_img, obs, actions, old_logits, old_logp, vf_preds, adv, vtarg, A: int, MB: int, mb_perm, step_ctr,
+                      kl_coeff, hyper: PPOHyper, ctas_per_policy: int, grad_part, stat_part, status=None,
+                      tail: Optional[SgdTail] = None):
     _lib.check(_lib.load().ddrl_ppo_train_step_tc(
-        _p(tc_img, torch.uint8, "tc_img"), _p(obs, f32, "obs"), _p(actions, f32, "actions"),
-        _p(old_logits, f32, "old_logits"), _p(old_logp, f32, "old_logp"), _p(vf_preds, f32, "vf_preds"), _p(adv, f32, "adv"),
-        _p(vtarg, f32, "vtarg"), P, R, D, A, MB, _p(mb_perm, torch.int32, "mb_perm"), perm_stride,
-        _p(step_ctr, torch.int32, "step_ctr"), _p(kl_coeff, f32, "kl_coeff"), C.byref(hyper), ctas_per_policy,
-        _p(grad_part, f32, "grad_part"), _p(stat_part, torch.float64, "stat_part"), _p(status, torch.int32, "status"),
-        C.byref(tail) if tail is not None else None, _stream()), "ppo_train_step_tc")
+        _p(tc_img, torch.uint8, "tc_img"),
+        *_step_args(obs, actions, old_logits, old_logp, vf_preds, adv, vtarg, A, MB, mb_perm, step_ctr, kl_coeff, hyper,
+                    ctas_per_policy, grad_part, stat_part),
+        _p(status, torch.int32, "status"), C.byref(tail) if tail is not None else None, _stream()), "ppo_train_step_tc")
 
 
 STATUS_BAD_NODE = 128      # DDRL_STATUS_BAD_NODE: a node id outside 0..3 reached a leg-coupled step
@@ -680,15 +681,10 @@ def ppo_train_step_tc_coupled(tc_img, theta, node_id, obs, actions, old_logits, 
                               status, tail: SgdTail):
     """Leg-coupled tensor-core step (SharedDecentralLegID, ddrl_ppo_train_step_tc_coupled): theta [1, NP + 8] (FCNet
     variables, then leg_coupling [4, 2]), node_id [1, R] int32, grad_part [1, G, part_stride(NP + 8)]; fused tail required."""
-    P, R, D = obs.shape
-    f32 = torch.float32
-    perm_stride = mb_perm.shape[-1] if mb_perm is not None else 0
     _lib.check(_lib.load().ddrl_ppo_train_step_tc_coupled(
-        _p(tc_img, torch.uint8, "tc_img"), _p(theta, f32, "theta"), _p(node_id, torch.int32, "node_id"), _p(obs, f32, "obs"),
-        _p(actions, f32, "actions"), _p(old_logits, f32, "old_logits"), _p(old_logp, f32, "old_logp"),
-        _p(vf_preds, f32, "vf_preds"), _p(adv, f32, "adv"), _p(vtarg, f32, "vtarg"), P, R, D, A, MB,
-        _p(mb_perm, torch.int32, "mb_perm"), perm_stride, _p(step_ctr, torch.int32, "step_ctr"), _p(kl_coeff, f32, "kl_coeff"),
-        C.byref(hyper), ctas_per_policy, _p(grad_part, f32, "grad_part"), _p(stat_part, torch.float64, "stat_part"),
+        _p(tc_img, torch.uint8, "tc_img"), _p(theta, torch.float32, "theta"), _p(node_id, torch.int32, "node_id"),
+        *_step_args(obs, actions, old_logits, old_logp, vf_preds, adv, vtarg, A, MB, mb_perm, step_ctr, kl_coeff, hyper,
+                    ctas_per_policy, grad_part, stat_part),
         _p(status, torch.int32, "status"), C.byref(tail) if tail is not None else None, _stream()), "ppo_train_step_tc_coupled")
 
 
@@ -697,15 +693,10 @@ def ppo_train_step_coupled(theta, img, node_id, obs, actions, old_logits, old_lo
                            tail: SgdTail):
     """Leg-coupled FP32 step (ddrl_ppo_train_step_coupled): as ppo_train_step_tc_coupled with the packed FP32 image `img`
     of the first NP entries of theta; the device flag goes to tail.status."""
-    P, R, D = obs.shape
-    f32 = torch.float32
-    perm_stride = mb_perm.shape[-1] if mb_perm is not None else 0
     _lib.check(_lib.load().ddrl_ppo_train_step_coupled(
-        _p(theta, f32, "theta"), _p(img, f32, "img"), _p(node_id, torch.int32, "node_id"), _p(obs, f32, "obs"),
-        _p(actions, f32, "actions"), _p(old_logits, f32, "old_logits"), _p(old_logp, f32, "old_logp"),
-        _p(vf_preds, f32, "vf_preds"), _p(adv, f32, "adv"), _p(vtarg, f32, "vtarg"), P, R, D, A, MB,
-        _p(mb_perm, torch.int32, "mb_perm"), perm_stride, _p(step_ctr, torch.int32, "step_ctr"), _p(kl_coeff, f32, "kl_coeff"),
-        C.byref(hyper), ctas_per_policy, _p(grad_part, f32, "grad_part"), _p(stat_part, torch.float64, "stat_part"),
+        _p(theta, torch.float32, "theta"), _p(img, torch.float32, "img"), _p(node_id, torch.int32, "node_id"),
+        *_step_args(obs, actions, old_logits, old_logp, vf_preds, adv, vtarg, A, MB, mb_perm, step_ctr, kl_coeff, hyper,
+                    ctas_per_policy, grad_part, stat_part),
         C.byref(tail) if tail is not None else None, _stream()), "ppo_train_step_coupled")
 
 

@@ -325,27 +325,18 @@ class FCNetLearner(_LearnerBase):
                 self._peer_exchange(G).fill(tail)
         elif nsteps != 1:
             raise DDRLError("multi-step launches need the fused tail")
-        if self.coupled:
-            if tail is None:
-                raise DDRLError("leg_coupling: the coupled SGD step needs the fused tail")
-            if self.mode == "tc":
-                K.ppo_train_step_tc_coupled(self.tc_img, self.theta, src["node"], src["obs"], src["act"], src["logits"],
-                                            src["logp"], src["value"], src["adv"], src["vtarg"], self.A, MB, b["mb_perm"],
-                                            self.step_ctr, self.kl_coeff, hyper, G, b["grad_part"], b["stat_part"],
-                                            self.tc_status, tail)
-            else:
-                K.ppo_train_step_coupled(self.theta, self.img, src["node"], src["obs"], src["act"], src["logits"], src["logp"],
-                                         src["value"], src["adv"], src["vtarg"], self.A, MB, b["mb_perm"], self.step_ctr,
-                                         self.kl_coeff, hyper, G, b["grad_part"], b["stat_part"], tail)
-            return
-        if self.mode == "tc":
-            K.ppo_train_step_tc(self.tc_img, src["obs"], src["act"], src["logits"], src["logp"], src["value"], src["adv"],
-                                src["vtarg"], self.A, MB, b["mb_perm"], self.step_ctr, self.kl_coeff, hyper, G,
-                                b["grad_part"], b["stat_part"], self.tc_status, tail=tail)
+        if self.coupled and tail is None:
+            raise DDRLError("leg_coupling: the coupled SGD step needs the fused tail")
+        batch = (src["obs"], src["act"], src["logits"], src["logp"], src["value"], src["adv"], src["vtarg"], self.A, MB,
+                 b["mb_perm"], self.step_ctr, self.kl_coeff, hyper, G, b["grad_part"], b["stat_part"])
+        if self.mode == "tc" and self.coupled:
+            K.ppo_train_step_tc_coupled(self.tc_img, self.theta, src["node"], *batch, self.tc_status, tail)
+        elif self.mode == "tc":
+            K.ppo_train_step_tc(self.tc_img, *batch, self.tc_status, tail=tail)
+        elif self.coupled:
+            K.ppo_train_step_coupled(self.theta, self.img, src["node"], *batch, tail)
         else:
-            K.ppo_train_step(self.theta, src["obs"], src["act"], src["logits"], src["logp"], src["value"], src["adv"],
-                             src["vtarg"], self.A, MB, b["mb_perm"], self.step_ctr, self.kl_coeff, hyper, G,
-                             b["grad_part"], b["stat_part"], img=self.img, tail=tail)
+            K.ppo_train_step(self.theta, *batch, img=self.img, tail=tail)
         if tail is not None:
             return
         K.grad_reduce(b["grad_part"], b["stat_part"], self.P, G, self.NP, self.grad, b["step_stats"], self.step_ctr)
@@ -374,11 +365,9 @@ class FCNetLearner(_LearnerBase):
     # ---- everything before the SGD epochs: filter, inference forward, bootstrap, GAE, standardise, shuffle ----------------
     def _prepare(self, b, obs_flat, boot_obs, rewards, dones, eps_flat, shuffle, cols_per_env, update_filter, T, Cc):
         P, R, D = obs_flat.shape
-        cfg, A = self.cfg, self.A
+        cfg = self.cfg
         self.tc_status.zero_()
-        K.fcnet_pack(self.theta_fc, D, A, self.img)
-        if self.tc_img is not None:
-            K.fcnet_tc_pack(self.theta_fc, D, A, self.tc_img)
+        self._pack_images()
         # (i) filter + forward + sample ------------------------------------------------------------------
         if update_filter:
             if self.world > 1:
@@ -393,48 +382,56 @@ class FCNetLearner(_LearnerBase):
                 K.filter_merge(allp, R * self.world, self.filt_n, self.filt_M, self.filt_S, self.norm)
             else:
                 K.filter_update(obs_flat, self.filt_n, self.filt_M, self.filt_S, self.norm, b["filt_ws"])
-        if self.coupled:
-            # ONE launch: forward, LegCoupling on the mean logits, DiagGaussian sample + logp of the COUPLED distribution
-            # (the stored old logits are the coupled ones)
-            out = {"logits": b["logits"], "value": b["value"], "obs_out": b["obs"], "action": b["act"], "logp": b["logp"]}
-            coupling = self.theta[0, self.NPf:]
-            if self.tc_forward and self.tc_img is not None:
-                K.fcnet_forward_tc_coupled(self.tc_img, obs_flat, b["node"], coupling, A, norm=self.norm, clip=cfg.filter_clip,
-                                           eps=eps_flat, status=self.tc_status, out=out)
-            else:
-                K.fcnet_forward_coupled(self.theta_fc, obs_flat, b["node"], coupling, A, norm=self.norm, clip=cfg.filter_clip,
-                                        eps=eps_flat, status=self.tc_status, out=out, img=self.img)
-            if self.tc_forward and self.tc_img is not None:
-                K.fcnet_forward_tc(self.tc_img, boot_obs, A, norm=self.norm, clip=cfg.filter_clip,
-                                   out={"logits": None, "value": b["vboot"], "obs_out": None}, status=self.tc_status)
-            else:
-                K.fcnet_forward(self.theta_fc, boot_obs, A, norm=self.norm, clip=cfg.filter_clip,
-                                out={"logits": None, "value": b["vboot"], "obs_out": None}, img=self.img)
-        elif self.tc_forward and self.tc_img is not None and K.tc_pingpong_eligible(D, A):
-            # inference on the tensor cores (same pipeline as the training forward, ~3e-6 relative)
-            K.fcnet_forward_tc(self.tc_img, obs_flat, A, norm=self.norm, clip=cfg.filter_clip, eps=eps_flat,
-                               out={"logits": b["logits"], "value": b["value"], "obs_out": b["obs"], "action": b["act"],
-                                    "logp": b["logp"]}, status=self.tc_status)
-            K.fcnet_forward_tc(self.tc_img, boot_obs, A, norm=self.norm, clip=cfg.filter_clip,
-                               out={"logits": None, "value": b["vboot"], "obs_out": None}, status=self.tc_status)
-        else:
-            K.fcnet_forward(self.theta, obs_flat, A, norm=self.norm, clip=cfg.filter_clip, eps=eps_flat,
-                            out={"logits": b["logits"], "value": b["value"], "obs_out": b["obs"], "action": b["act"],
-                                 "logp": b["logp"]}, img=self.img)
-            K.fcnet_forward(self.theta, boot_obs, A, norm=self.norm, clip=cfg.filter_clip,
-                            out={"logits": None, "value": b["vboot"], "obs_out": None}, img=self.img)
+        # the rollout rows (coupled: the stored old logits are the COUPLED ones), then the bootstrap values
+        self._forward(obs_flat, {"logits": b["logits"], "value": b["value"], "obs_out": b["obs"], "action": b["act"],
+                                 "logp": b["logp"]}, eps=eps_flat, node=b["node"] if self.coupled else None)
+        self._forward(boot_obs, {"logits": None, "value": b["vboot"], "obs_out": None})
         # (ii) bootstrap + GAE + standardise -----------------------------------------------------------
         K.gae(rewards, b["value"].view(P, T, Cc), dones, b["vboot"], cols_per_env, cfg.gamma, cfg.lambda_,
               b["adv"].view(P, T, Cc), b["vtarg"].view(P, T, Cc), b["moments"], b["gae_ws"])
         if self.world > 1:
             self.dist.all_reduce(b["moments"])
         K.adv_standardize(b["adv"], b["moments"])
-        # shuffle (SampleBatch.shuffle) -----------------------------------------------------------------
         if shuffle is not None:
-            for nme in ("obs", "act", "logits", "logp", "value", "adv", "vtarg"):
-                K.gather_rows(b[nme], shuffle, b[nme + "_s"])
-            if self.coupled:      # the node ids travel with their rows (a 4-byte row copy: the int32 bits move unchanged)
-                K.gather_rows(b["node"].view(torch.float32), shuffle, b["node_s"].view(torch.float32))
+            self._shuffle(b, shuffle)
+
+    _COLUMNS = ("obs", "act", "logits", "logp", "value", "adv", "vtarg")
+
+    def _pack_images(self):
+        """The FP32 and tensor-core weight images, from the FCNet part of theta."""
+        K.fcnet_pack(self.theta_fc, self.D, self.A, self.img)
+        if self.tc_img is not None:
+            K.fcnet_tc_pack(self.theta_fc, self.D, self.A, self.tc_img)
+
+    def _shuffle(self, b, shuffle):
+        """SampleBatch.shuffle: the columns, row-permuted into their *_s buffers."""
+        for nme in self._COLUMNS:
+            K.gather_rows(b[nme], shuffle, b[nme + "_s"])
+        if self.coupled:      # the node ids travel with their rows (a 4-byte row copy: the int32 bits move unchanged)
+            K.gather_rows(b["node"].view(torch.float32), shuffle, b["node_s"].view(torch.float32))
+
+    def _src(self, b, shuffled: bool) -> dict:
+        """The columns the SGD phase reads: the shuffled *_s buffers or the prepared ones."""
+        names = self._COLUMNS + (("node",) if self.coupled else ())
+        return {n_: b[n_ + ("_s" if shuffled else "")] for n_ in names}
+
+    def _forward(self, obs, out: dict, eps=None, node=None):
+        """Inference forward of rows `obs` into `out` (filter normalisation with self.norm; with eps the DiagGaussian sample).
+        With `node` the leg-coupled model in ONE launch: forward, LegCoupling on the mean logits, sample + logp of the
+        coupled distribution.  On the tensor cores if tc_forward (same pipeline as the training forward, ~3e-6 relative) —
+        the uncoupled model only where the ping-pong kernel runs its shape — else on the FP32 kernel."""
+        kw = dict(norm=self.norm, clip=self.cfg.filter_clip, eps=eps, out=out)
+        tc = self.tc_forward and (self.coupled or K.tc_pingpong_eligible(self.D, self.A))
+        if node is not None:
+            coupling = self.theta[0, self.NPf:]
+            if tc:
+                K.fcnet_forward_tc_coupled(self.tc_img, obs, node, coupling, self.A, status=self.tc_status, **kw)
+            else:
+                K.fcnet_forward_coupled(self.theta_fc, obs, node, coupling, self.A, status=self.tc_status, img=self.img, **kw)
+        elif tc:
+            K.fcnet_forward_tc(self.tc_img, obs, self.A, status=self.tc_status, **kw)
+        else:
+            K.fcnet_forward(self.theta_fc, obs, self.A, img=self.img, **kw)
 
     def _prepare_cached(self, b, obs_flat, boot_obs, rewards, dones, eps_flat, shuffle, cols_per_env, update_filter, T, Cc):
         """The ~20 short launches of the preparation phase are captured once per set of input buffers and replayed (the
@@ -491,11 +488,8 @@ class FCNetLearner(_LearnerBase):
         b = self._alloc(T, Cc)
         obs_flat = raw_obs.reshape(P, R, D)
         eps_flat = eps.reshape(P, R, A)
-        names = ("obs", "act", "logits", "logp", "value", "adv", "vtarg") + (("node",) if self.coupled else ())
-        src_key = "s" if shuffle is not None else "u"
-        src = {n_: b[n_ + ("_s" if shuffle is not None else "")] for n_ in names}
         self._prepare_cached(b, obs_flat, boot_obs, rewards, dones, eps_flat, shuffle, cols_per_env, update_filter, T, Cc)
-        return self._sgd_phase(b, src, src_key, perms, R, T, Cc)
+        return self._sgd_phase(b, self._src(b, shuffle is not None), "s" if shuffle is not None else "u", perms, R, T, Cc)
 
     def _sgd_phase(self, b, src, src_key, perms, R: int, T: int, Cc: int) -> List[Dict[str, float]]:
         """(iii) minibatch SGD over the prepared columns `src` + (iv) stats and KL-coefficient update."""
@@ -623,24 +617,16 @@ class FCNetLearner(_LearnerBase):
                                 f"got {t.dtype} {tuple(t.shape)} on {t.device}")
         b = self._alloc(R, 1)
         self.tc_status.zero_()
-        K.fcnet_pack(self.theta_fc, D, A, self.img)
-        if self.tc_img is not None:
-            K.fcnet_tc_pack(self.theta_fc, D, A, self.tc_img)
+        self._pack_images()
         for name, (t, _) in cols.items():
             b[name].copy_(t)
-        if standardize:
-            self.standardize_advantages(b["adv"])
-        names = ("obs", "act", "logits", "logp", "value", "adv", "vtarg")
-        if shuffle is not None:
-            for nme in names:
-                K.gather_rows(b[nme], shuffle, b[nme + "_s"])
         if self.coupled:
             b["node"].copy_(node_idx)
-            if shuffle is not None:
-                K.gather_rows(b["node"].view(torch.float32), shuffle, b["node_s"].view(torch.float32))
-            names = names + ("node",)
-        src = {n_: b[n_ + ("_s" if shuffle is not None else "")] for n_ in names}
-        return self._sgd_phase(b, src, "s" if shuffle is not None else "u", perms, R, R, 1)
+        if standardize:
+            self.standardize_advantages(b["adv"])
+        if shuffle is not None:
+            self._shuffle(b, shuffle)
+        return self._sgd_phase(b, self._src(b, shuffle is not None), "s" if shuffle is not None else "u", perms, R, R, 1)
 
     def refresh_filter_norm(self):
         """Recompute the normalisation table (mean, 1/(std+1e-8)) from filt_n / filt_M / filt_S — after the state was
