@@ -49,6 +49,9 @@ PROTOTYPES = {
     "ddrl_filter_partial": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int64, C.c_int, C.c_void_p, c_stream]),
     "ddrl_filter_merge": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int64, c_i64p, c_f64p, c_f64p, c_f64p,
                                     c_stream]),
+    "ddrl_filter_stream_ws_bytes": (C.c_int64, [C.c_int, C.c_int, C.c_int64, C.c_int, C.c_int]),
+    "ddrl_filter_stream": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int64, C.c_int, C.c_int, c_i64p, c_f64p,
+                                     c_f64p, C.c_double, c_f32p, c_f64p, C.c_void_p, c_stream]),
     "ddrl_fcnet_forward": (C.c_int, [c_f32p, c_f32p, c_f32p, c_f64p, C.c_float, C.c_int, C.c_int64, C.c_int, C.c_int,
                                      c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_stream]),
     "ddrl_obs_gather": (C.c_int, [C.c_void_p, C.c_int, C.c_int64, C.c_int, c_i32p, C.c_int, C.c_int, C.c_int, c_f32p, c_stream]),

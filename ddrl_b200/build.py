@@ -12,7 +12,7 @@ import sys
 PKG = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG, "csrc")
 LIB = os.path.join(PKG, "libddrl_b200.so")
-SOURCES = ["stream.cu", "fcnet.cu", "graphnet.cu", "graphnet_tc.cu", "graphvar.cu", "tc.cu", "tc2.cu"]
+SOURCES = ["stream.cu", "filter_stream.cu", "fcnet.cu", "graphnet.cu", "graphnet_tc.cu", "graphvar.cu", "tc.cu", "tc2.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "--use_fast_math=false"]
 

@@ -448,6 +448,43 @@ def filter_merge(parts: torch.Tensor, R_total: int, n, M, S, norm: Optional[torc
     return norm
 
 
+def filter_stream_ws_bytes(P: int, T: int, C: int, W: int, D: int) -> int:
+    n = int(_lib.load().ddrl_filter_stream_ws_bytes(P, T, C, W, D))
+    if n < 0:
+        raise DDRLError(f"filter_stream: bad shape P={P} T={T} C={C} W={W} D={D} (C must be a multiple of W)")
+    return n
+
+
+def filter_stream(x: torch.Tensor, n: torch.Tensor, M: torch.Tensor, S: torch.Tensor, T: int, W: int, clip: float = 0.0,
+                  out: Optional[torch.Tensor] = None, parts: Optional[torch.Tensor] = None,
+                  ws: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Row-by-row MeanStdFilter streams (ddrl_filter_stream): x [P,R,D] f32/f64 with R = T*C rows in (t, c) order, W
+    streams per policy over equal column blocks, all starting from the running state n [P] i64, M,S [P,D] f64 (read only).
+    -> (out [P,R,D] f32 normalised rows, parts [P,W,D,3] f64 {count, mean, M2} of every stream); fold parts into the state
+    with `filter_merge(parts, R, n, M, S, norm)`."""
+    if x.dtype not in (torch.float32, torch.float64):
+        raise DDRLError("filter_stream: x must be float32 or float64")
+    P, R, D = x.shape
+    if T < 1 or R % T:
+        raise DDRLError(f"filter_stream: R={R} rows are not T={T} steps of whole rows")
+    C = R // T
+    lib = _lib.load()
+    nbytes = filter_stream_ws_bytes(P, T, C, W, D)
+    if out is None:
+        out = torch.empty(P, R, D, dtype=torch.float32, device=x.device)
+    if parts is None:
+        parts = torch.empty(P, W, D, 3, dtype=torch.float64, device=x.device)
+    if ws is None or ws.numel() * ws.element_size() < nbytes:
+        ws = torch.empty(max(nbytes, 8), dtype=torch.uint8, device=x.device)
+    if tuple(out.shape) != (P, R, D) or tuple(parts.shape) != (P, W, D, 3):
+        raise DDRLError(f"filter_stream: out must be {(P, R, D)} and parts {(P, W, D, 3)}")
+    _lib.check(lib.ddrl_filter_stream(_p(x, None, "x"), int(x.dtype == torch.float64), P, int(T), int(C), int(W), D,
+                                      _p(n, torch.int64, "n"), _p(M, torch.float64, "M"), _p(S, torch.float64, "S"),
+                                      float(clip), _p(out, torch.float32, "out"), _p(parts, torch.float64, "parts"),
+                                      _p(ws, None, "ws"), _stream()), "filter_stream")
+    return out, parts
+
+
 def ppo_loss_grad(logits, value, actions, old_logits, old_logp, vf_preds, adv, vtarg, A: int, kl_coeff,
                   hyper: PPOHyper, ctas: int, dlogits, dvalue, stat_part):
     """logits [P,R,2A], value [P,R] -> dlogits, dvalue (in the given buffers), stat_part [P,ctas,8] f64."""

@@ -146,7 +146,8 @@ class FCNetLearner(_LearnerBase):
     def __init__(self, P: int, D: int, A: int, cfg: PPOConfig, device="cuda", theta: Optional[torch.Tensor] = None,
                  use_graph: bool = True, ctas_per_policy: Optional[int] = None, mode: str = "tc", fuse_tail: bool = True,
                  persistent: bool = True, tc_forward: bool = True, ll_tail: bool = False, vf_share_layers: bool = False,
-                 free_log_std: bool = False, atomic_reduce: bool = True, leg_coupling: bool = False):
+                 free_log_std: bool = False, atomic_reduce: bool = True, leg_coupling: bool = False,
+                 filter_mode: str = "batch", filter_workers: int = 1):
         """mode: "tc"   = tensor-core (tcgen05) SGD step, fp16 hi/lo operand split (gradients within 5e-5 of scale);
                  "fp32" = FP32-FMA SGD step (1e-5 parity).  Inference / GAE / Adam are FP32 in both modes.
         vf_share_layers / free_log_std: the reference model's optional layouts (models/fcnet_glorot_uniform_init.py:30-36,
@@ -160,7 +161,22 @@ class FCNetLearner(_LearnerBase):
         of the ModelV2 class); m / v alike; default table LegCoupling.INIT.  The mean logits of a row are scaled by
         c[node id], node id = the agent's position in agent_names (FL, HL, HR, FR); the SGD steps are
         ddrl_ppo_train_step_tc_coupled / ddrl_ppo_train_step_coupled (fused tail required: the table is clipped and stepped
-        with the MLP weights)."""
+        with the MLP weights).
+        filter_mode: how an update of the observation filter normalises the rows it pushes.
+          "batch"  (default) = the vectorised `MeanStdFilter` call: push every row, then normalise all rows with the final
+                   statistics (`ddrl_filter_update`);
+          "stream" = what RLlib's rollout workers do: the sampler calls the filter once per row, so every row is normalised
+                   with the statistics of its worker's earlier rows plus itself (`ddrl_filter_stream`).  learn_on_rollout
+                   splits the environments of the rollout into `filter_workers` equal, contiguous groups (worker w owns
+                   environments [w*N/W, (w+1)*N/W) with all their agent columns), every worker starts from the running
+                   state, and the workers' own rows are folded into it in worker order (FilterManager.synchronize).  At
+                   world > 1 the workers of rank r follow those of rank r - 1.  compute_actions(update_filter=True) is one
+                   worker over the call's rows.
+        filter_workers: rollout workers per rank in "stream" mode (RLlib's num_workers; every published run used 2)."""
+        if filter_mode not in ("batch", "stream"):
+            raise DDRLError(f"filter_mode must be 'batch' or 'stream', got {filter_mode!r}")
+        if int(filter_workers) < 1:
+            raise DDRLError(f"filter_workers must be >= 1, got {filter_workers}")
         if mode not in ("tc", "fp32"):
             raise DDRLError(f"mode must be 'tc' or 'fp32', got {mode!r}")
         if not fcnet_mode_supports(D, A, mode):
@@ -222,6 +238,7 @@ class FCNetLearner(_LearnerBase):
         self.atomic_reduce = (atomic_reduce and os.environ.get("DDRL_FIXED_ORDER", "0") != "1" and mode == "tc"
                               and not self.ll_tail)
         self.D, self.A = D, A
+        self.filter_mode, self.filter_workers = filter_mode, int(filter_workers)
         dev = self.device
         self.filt_n = torch.zeros(P, dtype=torch.int64, device=dev)
         self.filt_M = torch.zeros(P, D, dtype=torch.float64, device=dev)
@@ -369,7 +386,22 @@ class FCNetLearner(_LearnerBase):
         self.tc_status.zero_()
         self._pack_images()
         # (i) filter + forward + sample ------------------------------------------------------------------
-        if update_filter:
+        stream = update_filter and self.filter_mode == "stream"
+        if stream:
+            # every worker filters its rows one by one from the running state, straight into the stored obs column; its
+            # own rows ({count, mean, M2} per stream) are then folded into the running state in worker (and rank) order
+            if b.get("fs_parts") is None:
+                W = self.filter_workers
+                b["fs_parts"] = torch.empty(P, W, D, 3, dtype=torch.float64, device=self.device)
+                b["fs_ws"] = torch.empty(max(8, K.filter_stream_ws_bytes(P, T, Cc, W, D)), dtype=torch.uint8, device=self.device)
+            K.filter_stream(obs_flat, self.filt_n, self.filt_M, self.filt_S, T, self.filter_workers, cfg.filter_clip,
+                            out=b["obs"], parts=b["fs_parts"], ws=b["fs_ws"])
+            parts = b["fs_parts"]
+            if self.world > 1:
+                W = self.filter_workers
+                parts = gather_stats_rank_order(parts.view(P, 1, W * D, 3), self.dist, self.world).view(P, self.world * W, D, 3)
+            K.filter_merge(parts, R * self.world, self.filt_n, self.filt_M, self.filt_S, self.norm)
+        elif update_filter:
             if self.world > 1:
                 # this rank's partials -> ONE {count, mean, M2} per (policy, feature) (Chan merge into a zero state), the
                 # ranks' triples gathered in rank order, then folded into the running state: identical bits on every rank
@@ -382,9 +414,13 @@ class FCNetLearner(_LearnerBase):
                 K.filter_merge(allp, R * self.world, self.filt_n, self.filt_M, self.filt_S, self.norm)
             else:
                 K.filter_update(obs_flat, self.filt_n, self.filt_M, self.filt_S, self.norm, b["filt_ws"])
-        # the rollout rows (coupled: the stored old logits are the COUPLED ones), then the bootstrap values
-        self._forward(obs_flat, {"logits": b["logits"], "value": b["value"], "obs_out": b["obs"], "action": b["act"],
-                                 "logp": b["logp"]}, eps=eps_flat, node=b["node"] if self.coupled else None)
+        # the rollout rows (coupled: the stored old logits are the COUPLED ones), then the bootstrap values.  Stream mode:
+        # the rows are already normalised in the obs column; the bootstrap rows are normalised with the merged end state
+        # and not pushed, as in batch mode
+        rows = {"logits": b["logits"], "value": b["value"], "obs_out": None if stream else b["obs"], "action": b["act"],
+                "logp": b["logp"]}
+        self._forward(b["obs"] if stream else obs_flat, rows, eps=eps_flat, node=b["node"] if self.coupled else None,
+                      normalise=not stream)
         self._forward(boot_obs, {"logits": None, "value": b["vboot"], "obs_out": None})
         # (ii) bootstrap + GAE + standardise -----------------------------------------------------------
         K.gae(rewards, b["value"].view(P, T, Cc), dones, b["vboot"], cols_per_env, cfg.gamma, cfg.lambda_,
@@ -415,12 +451,13 @@ class FCNetLearner(_LearnerBase):
         names = self._COLUMNS + (("node",) if self.coupled else ())
         return {n_: b[n_ + ("_s" if shuffled else "")] for n_ in names}
 
-    def _forward(self, obs, out: dict, eps=None, node=None):
+    def _forward(self, obs, out: dict, eps=None, node=None, normalise: bool = True):
         """Inference forward of rows `obs` into `out` (filter normalisation with self.norm; with eps the DiagGaussian sample).
         With `node` the leg-coupled model in ONE launch: forward, LegCoupling on the mean logits, sample + logp of the
         coupled distribution.  On the tensor cores if tc_forward (same pipeline as the training forward, ~3e-6 relative) —
-        the uncoupled model only where the ping-pong kernel runs its shape — else on the FP32 kernel."""
-        kw = dict(norm=self.norm, clip=self.cfg.filter_clip, eps=eps, out=out)
+        the uncoupled model only where the ping-pong kernel runs its shape — else on the FP32 kernel.  normalise=False: the
+        rows are network inputs already (stream-mode filter)."""
+        kw = dict(norm=self.norm if normalise else None, clip=self.cfg.filter_clip, eps=eps, out=out)
         tc = self.tc_forward and (self.coupled or K.tc_pingpong_eligible(self.D, self.A))
         if node is not None:
             coupling = self.theta[0, self.NPf:]
@@ -485,6 +522,9 @@ class FCNetLearner(_LearnerBase):
         if self.coupled and (cols_per_env != 4 or Cc % 4):
             raise DDRLError(f"leg_coupling: the rollout's columns must be env-major legs (cols_per_env=4, C % 4 == 0), got "
                             f"cols_per_env={cols_per_env}, C={Cc}")
+        if self.filter_mode == "stream" and (Cc % cols_per_env or (Cc // cols_per_env) % self.filter_workers):
+            raise DDRLError(f"filter_mode='stream': filter_workers={self.filter_workers} must divide the number of "
+                            f"environments (C={Cc} columns, cols_per_env={cols_per_env})")
         b = self._alloc(T, Cc)
         obs_flat = raw_obs.reshape(P, R, D)
         eps_flat = eps.reshape(P, R, A)
@@ -637,14 +677,21 @@ class FCNetLearner(_LearnerBase):
     # ---- plain inference (sampler side) ---------------------------------------------------------------------
     def compute_actions(self, raw_obs: torch.Tensor, eps: Optional[torch.Tensor] = None, update_filter: bool = False,
                         node_idx: Optional[torch.Tensor] = None):
-        """raw_obs [P,B,D] -> dict(logits, value[, action, logp]); optionally pushes the rows into the filter first
-        (RLlib sampler behaviour).  leg_coupling: node_idx [1,B] int32 (required); logits / action / logp are those of the
-        coupled distribution."""
+        """raw_obs [P,B,D] -> dict(logits, value[, action, logp]).  update_filter pushes the rows into the filter first:
+        filter_mode="batch" with ONE vectorised `MeanStdFilter` call (all rows pushed, then all normalised with the final
+        statistics); filter_mode="stream" row by row as RLlib's sampler calls the filter (row b normalised with the
+        statistics after pushing rows 0..b: one rollout worker over the call's rows).  leg_coupling: node_idx [1,B] int32
+        (required); logits / action / logp are those of the coupled distribution."""
         if self.coupled != (node_idx is not None):
             raise DDRLError("compute_actions: node_idx [1, B] int32 is required with leg_coupling and only then")
-        if update_filter:
-            K.filter_update(raw_obs, self.filt_n, self.filt_M, self.filt_S, self.norm)
-        use_norm = self.norm if int(self.filt_n.max().item()) > 0 else None
+        use_norm = None
+        if update_filter and self.filter_mode == "stream":
+            raw_obs, parts = K.filter_stream(raw_obs, self.filt_n, self.filt_M, self.filt_S, 1, 1, self.cfg.filter_clip)
+            K.filter_merge(parts, raw_obs.shape[1], self.filt_n, self.filt_M, self.filt_S, self.norm)
+        else:
+            if update_filter:
+                K.filter_update(raw_obs, self.filt_n, self.filt_M, self.filt_S, self.norm)
+            use_norm = self.norm if int(self.filt_n.max().item()) > 0 else None
         if not self.coupled:
             return K.fcnet_forward(self.theta, raw_obs, self.A, norm=use_norm, clip=self.cfg.filter_clip, eps=eps)
         P, B, _ = raw_obs.shape

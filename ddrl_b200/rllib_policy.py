@@ -213,7 +213,11 @@ class _PolicyGroupBase:
 
 
 class PPOPolicyGroup(_PolicyGroupBase):
-    """All policies of one `--policy_scope` behind one fused learner; see the module docstring."""
+    """All policies of one `--policy_scope` behind one fused learner; see the module docstring.  `learner_kw` goes to
+    `FCNetLearner`, among them filter_mode / filter_workers: with filter_mode="stream" every
+    `compute_actions(update_filter=True)` call filters its rows one by one, as the sampler of an RLlib rollout worker calls
+    the policy's MeanStdFilter once per observation — the mode an RLlib drop-in should use; the default "batch" is the
+    vectorised filter call (all rows pushed, then all normalised with the final statistics)."""
 
     def __init__(self, policy_scope: str, config: Optional[Dict[str, Any]] = None, device="cuda", seed: Optional[int] = None,
                  use_target_velocity: bool = False, **learner_kw):

@@ -89,6 +89,30 @@ int ddrl_filter_partial(const void* x, int x_is_f64, int P, int64_t R, int D, vo
 int ddrl_filter_merge(const void* parts, int nparts, int P, int D, int64_t R_total, int64_t* n,
                       double* M, double* S, double* norm, void* stream);
 
+/* Replaces: the sampler's row-by-row filter calls of RLlib rollout workers (evaluation/sampler.py
+ * _process_observations: one unvectorised MeanStdFilter.__call__ per observation row, i.e. RunningStat.push
+ * into rs and buffer, then (x - mean) / (std + 1e-8) with the UPDATED state), W workers per policy.
+ *   x        [P][R][D] float32 (x_is_f64=0) or float64 (x_is_f64=1), R = T*C rows in order t*C + c
+ *            (step-major, then environment, then the agent columns of an environment)
+ *   W        streams (rollout workers) per policy: stream w owns columns [w*C/W, (w+1)*C/W) and filters its
+ *            rows in (t, c) order; C % W == 0
+ *   n, M, S  [P] int64, [P][D], [P][D] float64: the running state every stream starts from (read only)
+ *   clip     >0: clip the normalised rows to [-clip, clip]; 0: none
+ *   out      [P][R][D] float32: row i normalised with its stream's state after pushing row i (float64
+ *            arithmetic in the reference's operation order, one rounding to float32)
+ *   parts    [P][W][D][3] float64 {count, mean, M2}: each stream's own rows (the worker's buffer), in the
+ *            layout of ddrl_filter_merge.  Folding them into n/M/S in worker order (ddrl_filter_merge with
+ *            R_total = R) is FilterManager.synchronize (apply_changes -> RunningStat.update).
+ *   ws       workspace of ddrl_filter_stream_ws_bytes(P, T, C, W, D) bytes (<0: bad shape)
+ * Fixed-order scan of chunk Welford states (no atomics): bit-identical from run to run and independent of
+ * the launch geometry; the first rows of every stream match the sequential reference bit for bit, later rows
+ * start from a merged state within 1e-12 relative of the sequential one.  D > DDRL_MAX_OBS returns
+ * DDRL_E_UNSUPPORTED_SHAPE. */
+int64_t ddrl_filter_stream_ws_bytes(int P, int T, int64_t C, int W, int D);
+int ddrl_filter_stream(const void* x, int x_is_f64, int P, int T, int64_t C, int W, int D, const int64_t* n,
+                       const double* M, const double* S, double clip, float* out, double* parts, void* ws,
+                       void* stream);
+
 /* Replaces: FullyConnectedNetwork_GlorotUniformInitializer.forward / value_function
  * (models/fcnet_glorot_uniform_init.py:120-125) for P grouped policies, with optional fused
  * prologue/epilogue:
