@@ -43,6 +43,42 @@ def test_reference_arm_other_ranks_exit_silently():
     assert out.returncode == 0 and out.stdout.strip() == ""
 
 
+def test_every_supplementary_job_has_an_oracle_test(monkeypatch):
+    """bench.run_supplementary's jobs, recorded without a GPU (time_fcnet / time_graphnet replaced by recorders), are the
+    workload table of tests/test_gpu_supplementary_workloads.py plus the two jobs covered elsewhere: the fp32 job by the
+    headline workload's fp32 mode, C4 by tests/test_gpu_graphnet_workload.py at its own envs and epochs."""
+    import argparse
+    import importlib
+    sys.path.insert(0, ROOT)
+    import bench
+    from tests import test_gpu_bench_workload as H
+    from tests import test_gpu_graphnet_workload as GN
+    from tests import test_gpu_supplementary_workloads as S
+    fc, gn = [], []
+    monkeypatch.setattr(bench, "time_fcnet", lambda *a, **kw: fc.append((a, kw)) or {})
+    monkeypatch.setattr(bench, "time_graphnet", lambda *a, **kw: gn.append((a, kw)) or (1.0, {"rows": 1}))
+    out = bench.run_supplementary(argparse.Namespace(envs=4096, minibatches=32))
+    assert not [v for v in out.values() if "error" in v], out
+    jobs = dict(zip([k for k in out if k != "C4_shared_GraphNet"], fc))
+    assert len(jobs) == len(fc) and set(out) == set(S.JOBS) | set(S.COVERED_ELSEWHERE)
+    for name, (args, kw) in jobs.items():
+        assert args[4:] == (3, 2) and not kw, (name, args, kw)           # steps, warmup as the table assumes
+        if name in S.JOBS:
+            assert args[:4] == S.JOBS[name], (name, args)
+            assert name in S.EXPECT and name in S.IDS, name
+    # the fp32 job: the headline's architecture and shape, which tests/test_gpu_bench_workload.py runs in its fp32 mode
+    W = bench.WORKLOAD
+    assert jobs["FullyDecentral_fp32_parity_kernel"][0][:4] == ("FullyDecentral", W["envs_per_gpu"], W["minibatches_per_epoch"], "fp32")
+    assert H.MODES["fp32"]["mode"] == "fp32"
+    # C4: time_graphnet(envs, epochs, steps, warmup) at the envs and epochs of the GraphNet workload test
+    assert gn == [((4096, W["epochs"], 2, 1), {})], gn
+    assert (GN.ENVS, GN.E_B) == gn[0][0][:2]
+    for name, (module, test, param) in S.COVERED_ELSEWHERE.items():
+        m = importlib.import_module(module)
+        assert callable(getattr(m, test, None)), (name, module, test)
+        assert param is None or param in m.MODES, (name, param)
+
+
 @pytest.mark.skipif(shutil.which("gcc") is None, reason="gcc not available")
 def test_header_is_plain_c():
     """include/ddrl_b200.h is the drop-in boundary: extern "C", plain pointers and sizes — it must compile as C99."""

@@ -13,10 +13,14 @@ first call, a capture-and-replay of the preparation phase and a replay of an exi
 - C: the persistent launch is bit-identical to one launch per step, which carries B over to the launch bench.py times.
 - D: a negative control: one repeated minibatch in one policy must be caught by A, at the right step and policy.
 
+The checks take a `Workload` record (shapes, inputs, the launch shape they claim to test), so that
+tests/test_gpu_supplementary_workloads.py runs the same checks on the other FCNet configurations bench.py times.
+
 Measured errors of these checks on a B200: profiles/r03_bench_workload_errors.txt."""
 import itertools
 import os
 from concurrent.futures import ThreadPoolExecutor
+from dataclasses import dataclass
 
 import numpy as np
 import pytest
@@ -27,16 +31,10 @@ from tests.util import assert_grad_per_variable, scaled_err
 
 pytestmark = pytest.mark.gpu
 
-W = WORKLOAD
-P, D, A, T, E, NB, ENVS = W["P"], W["D"], W["A"], W["T"], W["epochs"], W["minibatches_per_epoch"], W["envs_per_gpu"]
-_CFG = workload_config(ENVS, 1, NB, 2)
-R, MB = _CFG["rows_per_policy_per_gpu"], _CFG["sgd_minibatch_size_global"]
-C = R // T
-STEPS = E * NB
-ITER_SETS = (0, 1, 1)          # rollout set of each iteration: eager, capture + replay, replay
-MODES = {"tc-fixed": dict(mode="tc", atomic_reduce=False),      # what bench.py times
-         "tc-atomic": dict(mode="tc", atomic_reduce=True),      # the library default
-         "fp32": dict(mode="fp32", atomic_reduce=False)}        # the FP32-parity line: one-step launches, G = 37
+SMS = 148                      # the launch shapes below are those of a 148-SM B200
+MODES = {"tc-fixed": dict(mode="tc", atomic_reduce=False),      # what bench.py's headline times
+         "tc-atomic": dict(mode="tc", atomic_reduce=True),      # the library default (and bench.time_fcnet's)
+         "fp32": dict(mode="fp32", atomic_reduce=False)}        # the FP32-parity line: one-step launches
 COLS = ("obs", "act", "logits", "logp", "value", "adv", "vtarg")
 STEP_STATS = ("policy_loss", "kl", "vf_loss", "entropy", "vf_explained_var")
 
@@ -61,7 +59,61 @@ STAT_TOL_B = np.array([1e-5, 1e-5, 1e-5, 1e-5, 1e-4])
 # step included, nothing that depends on the update).  Everything else stays strict.  In the first iteration the
 # next-closest rows of policies 1 and 0 are 2.9e-6 and 6.8e-6 from a boundary; every path takes the same side there.
 NEAR_CLIP = 2e-6
-VALUE_BIAS = 11204              # flat index of value_out/bias for D = 19, A = 2
+
+
+@dataclass
+class Workload:
+    """One benchmarked FCNet configuration: its shapes, bench.py's inputs for it and the launch shape the checks claim to
+    test.  `sets` are rollout sets on the host (bench.synth_rollout's dict), `iter_sets` the set of each of the three
+    iterations, `theta0` [P, NP] the initial weights.  tc_setup / fp32_setup: what FCNetLearner._sgd_setup returns
+    (MB, nb, G) in each kernel family; tc_rows: the rows each of the G CTAs of a tensor-core step holds.  control:
+    (policy, step) of the repeated-minibatch control of D."""
+    name: str
+    P: int
+    D: int
+    A: int
+    T: int
+    C: int
+    E: int
+    NB: int
+    MB: int
+    sets: list
+    iter_sets: tuple
+    theta0: torch.Tensor
+    tc_setup: tuple
+    tc_rows: tuple
+    fp32_setup: tuple
+    control: tuple
+
+    @property
+    def R(self):
+        return self.T * self.C
+
+    @property
+    def STEPS(self):
+        return self.E * self.NB
+
+    @property
+    def VALUE_BIAS(self):
+        """Flat index of value_out/bias: the last variable of the FCNet layout (11204 for D = 19, A = 2)."""
+        return self.theta0.shape[1] - 1
+
+
+def _headline():
+    """bench.py's headline: FullyDecentral, rollout sets 0 and 1 of rank 0 (seeds 1234 + 100 s) on the host, three
+    iterations on sets 0, 1, 1 (eager, capture + replay, replay), policy 2's step 200 as the control."""
+    from ddrl_b200.modelv2 import fcnet_init_flat
+    W = WORKLOAD
+    P, D, A, T, E, NB, ENVS = W["P"], W["D"], W["A"], W["T"], W["epochs"], W["minibatches_per_epoch"], W["envs_per_gpu"]
+    cfg = workload_config(ENVS, 1, NB, 2)
+    R, MB = cfg["rows_per_policy_per_gpu"], cfg["sgd_minibatch_size_global"]
+    C = R // T
+    gen = torch.Generator().manual_seed(1234)
+    theta0 = torch.stack([fcnet_init_flat(D, 2 * A, gen) for _ in range(P)])       # as bench.py
+    sets = [synth_rollout(P, T, C, D, A, ENVS, NB, E, 1234 + 100 * s) for s in range(2)]
+    return Workload(name="FullyDecentral", P=P, D=D, A=A, T=T, C=C, E=E, NB=NB, MB=MB, sets=sets, iter_sets=(0, 1, 1),
+                    theta0=theta0, tc_setup=(4096, 32, 32), tc_rows=(128,) * 32, fp32_setup=(4096, 32, 37),
+                    control=(2, 200))
 
 
 def _oracle():
@@ -69,36 +121,39 @@ def _oracle():
     return O
 
 
-def _cfg_o():
-    return _oracle().PPOConfig(num_sgd_iter=E, sgd_minibatch_size=MB)
+def _cfg_o(w):
+    return _oracle().PPOConfig(num_sgd_iter=w.E, sgd_minibatch_size=w.MB)
 
 
-def _theta0():
-    from ddrl_b200.modelv2 import fcnet_init_flat
-    gen = torch.Generator().manual_seed(1234)
-    return torch.stack([fcnet_init_flat(D, 2 * A, gen) for _ in range(P)])       # as bench.py
-
-
-def _learner(mode, **kw):
-    """FCNetLearner with bench.py's arguments."""
+def _learner(w, mode, **kw):
+    """FCNetLearner with bench.py's arguments, in the kernel family / reduction of `mode`."""
     from ddrl_b200.config import PPOConfig
     from ddrl_b200.learner import FCNetLearner
-    return FCNetLearner(P, D, A, PPOConfig(num_sgd_iter=E, sgd_minibatch_size=MB), "cuda", theta=_theta0(), **MODES[mode], **kw)
+    return FCNetLearner(w.P, w.D, w.A, PPOConfig(num_sgd_iter=w.E, sgd_minibatch_size=w.MB), "cuda", theta=w.theta0,
+                        **MODES[mode], **kw)
 
 
-def _assert_bench_shape(L, mode, persistent=True):
+def cta_rows(MB, G):
+    """Rows of each of the G CTAs of a tensor-core step within one minibatch: rpc = ((MB + G - 1) / G + 7) & ~7 rows per
+    CTA in CTA order, the last ones ragged or empty (csrc/tc2_step_body.inc)."""
+    rpc = (((MB + G - 1) // G) + 7) & ~7
+    return tuple(min((bx + 1) * rpc, MB) - min(bx * rpc, MB) for bx in range(G))
+
+
+def _assert_bench_shape(w, L, mode, persistent=True):
     """The launch shape this file claims to test; fails if the learner's choice drifts."""
     from ddrl_b200 import kernels as K
-    MB_, nb, G = L._sgd_setup(R)
+    MB_, nb, G = L._sgd_setup(w.R)
+    assert L.sms == SMS, f"{L.sms} SMs: the launch shapes asserted here are those of the {SMS}-SM B200"
     if MODES[mode]["mode"] == "tc":
-        assert K.tc_pingpong_eligible(D, A)                    # the ping-pong kernel (persistent launch)
-        assert (MB_, nb, G) == (4096, 32, 32), (MB_, nb, G)
-        assert MB_ // G == 128                                 # one full 128-row tile per CTA
+        assert K.tc_pingpong_eligible(w.D, w.A)                # the ping-pong kernel (persistent launch)
+        assert (MB_, nb, G) == w.tc_setup, (MB_, nb, G)
+        assert cta_rows(MB_, G) == w.tc_rows, cta_rows(MB_, G)
         assert L._persistent_steps(G) == persistent
     else:
-        assert (MB_, nb, G) == (4096, 32, 37) and G * P == L.sms, (MB_, nb, G, L.sms)      # every SM of the B200
+        assert (MB_, nb, G) == w.fp32_setup, (MB_, nb, G, L.sms)
         assert not L._persistent_steps(G)
-    assert L.fuse_tail and G * P <= L.sms                      # reduce + clip + Adam inside the train kernel
+    assert L.fuse_tail and G * w.P <= L.sms                    # reduce + clip + Adam inside the train kernel
     assert L.atomic_reduce == MODES[mode]["atomic_reduce"], "partial-gradient reduction is not the intended one (DDRL_FIXED_ORDER?)"
 
 
@@ -123,22 +178,26 @@ def _clip_branch(logits, act, old_logp, adv, cfg):
 
 
 # ---- the float64 oracle trajectory --------------------------------------------------------------------------------------
-def _oracle_policy(p, theta0, sets):
-    """Three learner iterations of policy p (ITER_SETS) in float64, step by step, and in float32 (the torch twin).
-    -> one record per iteration; `cut` = the first step of the iteration with a row within NEAR_CLIP of the clip kink,
-    `after_cut` = an earlier iteration had one."""
+def _oracle_policy(w, p, sets):
+    """Three learner iterations of policy p (w.iter_sets) in float64, step by step, and in float32 (the torch twin).
+    -> one record per iteration; `cut` = the first step of the iteration with a row within NEAR_CLIP of the clip kink or
+    a row on which the twin takes the other side of the kink than float64 (`fork`: that step and the float64 distance of
+    such rows from the kink), `after_cut` = an earlier iteration had one."""
     O = _oracle()
-    cfg = _cfg_o()
+    cfg = _cfg_o(w)
+    P, D, A, T, C, E, R, MB = w.P, w.D, w.A, w.T, w.C, w.E, w.R, w.MB
+    theta0 = w.theta0[p]
     filt = O.MeanStdFilter((D,), clip=None)      # the learner's filter_clip = 0: RLlib's MeanStdFilter has clip=None
     state = {dt: [theta0.to(dt), O.AdamState.zeros(theta0.numel(), dt, cfg), cfg.kl_coeff] for dt in (torch.float64, torch.float32)}
     fwd = lambda th, x: O.fcnet_forward(th, x, 2 * A)
     out = []
-    forked = False      # an earlier iteration had a row at the clip kink: this trajectory is one of two valid ones
-    for s in ITER_SETS:
+    forked = False      # why this trajectory is one of several valid ones from here on (a row at the clip kink, ...)
+    for s in w.iter_sets:
         r = sets[s]
         obs = filt(r["raw"][p].reshape(R, D))                  # pushes every row, then normalises
         bobs = filt(r["boot"][p], update=False)
         rec = {"filt": (filt.rs.n, filt.rs._M.copy(), filt.rs._S.copy())}
+        sides, dist = {}, []      # per step: the rows' side of the kink in each dtype, their float64 distance from it
         for dt in (torch.float64, torch.float32):
             theta, adam, klc = state[dt]
             x = torch.from_numpy(obs.astype(np.float32)).to(dt)
@@ -154,25 +213,33 @@ def _oracle_policy(p, theta0, sets):
                      "advantages": torch.from_numpy(adv_std).to(dt), "value_targets": torch.from_numpy(vt.reshape(-1)).to(dt)}
             idx = torch.from_numpy(r["shuffle"][p].astype(np.int64))
             batch = {k: v[idx] for k, v in batch.items()}
-            thetas, steps, cut = [], [], None
+            theta_first = theta_last = None
+            steps, cut, sides[dt] = [], None, []
             for e in range(E):
                 last = {k: [] for k in O.STAT_KEYS}
                 for mb in r["perms"][p, e]:
                     rows = slice(int(mb) * MB, (int(mb) + 1) * MB)
                     if dt == torch.float64:      # O.sgd_minibatch_step + the rows near the clip kink
-                        thetas.append(theta)
+                        theta_last = theta
+                        theta_first = theta if theta_first is None else theta_first
                         th = theta.clone().requires_grad_(True)
                         lg, v = fwd(th, batch["obs"][rows])
                         loss, st = O.ppo_loss_from_outputs(lg, v, *(batch[k][rows] for k in (
                             "actions", "old_logits", "old_logp", "vf_preds", "advantages", "value_targets")), klc, cfg)
                         (g,) = torch.autograd.grad(loss, th)
-                        near = _clip_branch(lg.detach(), batch["actions"][rows], batch["old_logp"][rows],
-                                            batch["advantages"][rows], cfg)[2]
+                        ratio, flows, near = _clip_branch(lg.detach(), batch["actions"][rows], batch["old_logp"][rows],
+                                                          batch["advantages"][rows], cfg)
                         if cut is None and bool(near.any()):
                             cut = len(steps)
+                        sides[dt].append(flows.numpy())
+                        dist.append(torch.minimum((ratio - 1.0 + cfg.clip_param).abs(), (ratio - 1.0 - cfg.clip_param).abs()).numpy())
                         theta = O.adam_tf1_step(theta, O.clip_by_global_norm(g, cfg.grad_clip)[0], adam, cfg)
                         st = {k: float(x.detach()) for k, x in st.items()}
                     else:
+                        with torch.no_grad():
+                            lg = fwd(theta, batch["obs"][rows])[0]
+                        sides[dt].append(_clip_branch(lg, batch["actions"][rows], batch["old_logp"][rows],
+                                                      batch["advantages"][rows], cfg)[1].numpy())
                         theta, st, _, _ = O.sgd_minibatch_step(theta, adam, fwd, batch, rows, klc, cfg)
                     steps.append([st[k] for k in STEP_STATS])
                     for k in O.STAT_KEYS:
@@ -182,42 +249,55 @@ def _oracle_policy(p, theta0, sets):
             state[dt] = [theta, adam, klc]
             if dt == torch.float64:
                 rec.update(obs=obs, logits=logits.numpy(), value=value.numpy(), act=act.numpy(), logp=logp.numpy(),
-                           adv=adv_std, vtarg=vt.reshape(-1), step_stats=np.array(steps), thetas=torch.stack(thetas).numpy(),
-                           theta=theta.numpy(), m=adam.m.numpy().copy(), v=adam.v.numpy().copy(),
-                           beta_pow=(adam.beta1_power, adam.beta2_power), kl_coeff=klc, stats=stats, cut=cut,
-                           after_cut=forked)
-                forked = forked or cut is not None
+                           adv=adv_std, vtarg=vt.reshape(-1), step_stats=np.array(steps), theta_first=theta_first.numpy(),
+                           theta_last=theta_last.numpy(), theta=theta.numpy(), m=adam.m.numpy().copy(),
+                           v=adam.v.numpy().copy(), beta_pow=(adam.beta1_power, adam.beta2_power), kl_coeff=klc, stats=stats,
+                           cut=cut, after_cut=forked)
             else:
                 rec.update(twin_theta=theta.numpy().astype(np.float64), twin_m=adam.m.numpy().astype(np.float64),
                            twin_v=adam.v.numpy().astype(np.float64))
+        # a row far enough from the kink for NEAR_CLIP, on which float32 round-off still took the other side
+        fork = next((i for i, (a, b) in enumerate(zip(sides[torch.float64], sides[torch.float32])) if (a != b).any()), None)
+        if fork is not None:
+            flip = sides[torch.float64][fork] != sides[torch.float32][fork]
+            rec["fork"] = (fork, float(dist[fork][flip].min()))
+            rec["cut"] = fork if rec["cut"] is None else min(rec["cut"], fork)
+        # the end state resolves one wrong step only if float32 round-off alone (the twin) leaves it more than 10x closer
+        # to float64 than the trajectory without its last step; where it does not (Adam amplifies round-off on
+        # near-zero gradients), a float32 trajectory of this policy is one of many valid ones from here on
+        rec["resolved"] = _update_err(rec["theta_last"], rec) > 10.0 * max(10.0 * _update_err(rec["twin_theta"], rec), UPD_FLOOR)
+        forked = forked or ("reached the clip kink" if rec["cut"] is not None else
+                            "left the float32 trajectories unresolved" if not rec["resolved"] else False)
         out.append(rec)
     return out
 
 
-@pytest.fixture(scope="module")
-def rollouts():
-    """bench.py's rollout sets 0 and 1 of rank 0 (seeds 1234 + 100 s), on the host."""
-    return [synth_rollout(P, T, C, D, A, ENVS, NB, E, 1234 + 100 * s) for s in range(2)]
-
-
-@pytest.fixture(scope="module")
-def oracle(rollouts):
+def oracle_trajectory(w):
     """-> [iteration][policy] records of the float64 trajectory (+ the twin's final state).  The policies are independent and
     run on P host threads, as bench.CpuLearner does."""
-    sets = [{k: v.numpy() for k, v in r.items()} for r in rollouts]
-    theta0 = _theta0()
+    sets = [{k: v.numpy() for k, v in r.items()} for r in w.sets]
     threads = torch.get_num_threads()
-    torch.set_num_threads(max(1, (os.cpu_count() or 1) // P))
+    torch.set_num_threads(max(1, (os.cpu_count() or 1) // w.P))
     try:
-        with ThreadPoolExecutor(P) as ex:
-            per_policy = list(ex.map(lambda p: _oracle_policy(p, theta0[p], sets), range(P)))
+        with ThreadPoolExecutor(w.P) as ex:
+            per_policy = list(ex.map(lambda p: _oracle_policy(w, p, sets), range(w.P)))
     finally:
         torch.set_num_threads(threads)
-    return [[per_policy[p][i] for p in range(P)] for i in range(len(ITER_SETS))]
+    return [[per_policy[p][i] for p in range(w.P)] for i in range(len(w.iter_sets))]
+
+
+@pytest.fixture(scope="module")
+def headline():
+    return _headline()
+
+
+@pytest.fixture(scope="module")
+def oracle(headline):
+    return oracle_trajectory(headline)
 
 
 # ---- comparisons ----------------------------------------------------------------------------------------------------------
-def _device_step_stats(ss):
+def _device_step_stats(ss, MB):
     """step_stats [steps, P, 8] float64 sums over the MB rows of a step -> [steps, P, 5] in STEP_STATS order."""
     s = np.asarray(ss, dtype=np.float64) / MB
     ev = np.maximum(-1.0, 1.0 - (s[..., 7] - s[..., 6] ** 2) / (s[..., 5] - s[..., 4] ** 2))
@@ -235,7 +315,7 @@ def _stat_ratio(dev, ref, tol):
 
 def _update_err(theta, ref):
     """max |theta - theta64| over the size of the float64 update of the iteration."""
-    upd = ref["theta"] - ref["thetas"][0]
+    upd = ref["theta"] - ref["theta_first"]
     return float(np.abs(np.asarray(theta, dtype=np.float64) - ref["theta"]).max() / np.abs(upd).max())
 
 
@@ -247,14 +327,21 @@ def _beta_chain(steps):
     return out
 
 
-def _compare(L, stats, refs, it, tag):
+def compared_steps(w, ref):
+    """Steps of an iteration whose loss statistics A compares for one policy: all, up to the first step with a row at
+    the clip kink, or none after an earlier iteration had one."""
+    return 0 if ref["after_cut"] else w.STEPS if ref["cut"] is None else ref["cut"] + 1
+
+
+def _compare(w, L, stats, refs, it, tag):
     """One learn_on_rollout result against the oracle's iteration `it` -> (failures [(policy, message)], first off step or
     None, per-policy measurements).  Prints one line per policy with the measured errors.  A policy whose reference
     trajectory reached a row at the clip kink (NEAR_CLIP) is compared up to that step only; the filter, the normalised
     observations, the beta powers and tc_status do not depend on the weights and are checked always."""
+    P, R = w.P, w.R
     fails = []
     bufs = L._bufs
-    ss = _device_step_stats(bufs["step_stats"].cpu().numpy())
+    ss = _device_step_stats(bufs["step_stats"].cpu().numpy(), w.MB)
     ratio = np.stack([_stat_ratio(ss[:, p], refs[p]["step_stats"], STAT_TOL_A) for p in range(P)], axis=1)    # [steps, P]
     for p in range(P):
         if refs[p]["after_cut"]:
@@ -266,7 +353,7 @@ def _compare(L, stats, refs, it, tag):
     if first is not None:
         fails.append((first[1], f"it {it}: step statistics first off at step {first[0]}, policy {first[1]} "
                                 f"(error / tolerance {ratio[first]:.3g})"))
-    beta = _beta_chain(STEPS * (it + 1))
+    beta = _beta_chain(w.STEPS * (it + 1))
     theta, m, v = L.theta.cpu().numpy(), L.m.cpu().numpy(), L.v.cpu().numpy()
     bp, klc = L.beta_pow.cpu().numpy(), L.kl_coeff.cpu().numpy()
     meas = []
@@ -285,7 +372,7 @@ def _compare(L, stats, refs, it, tag):
         check(bp[p, 0] == beta[0] and bp[p, 1] == beta[1], f"beta powers {bp[p]} != float32 chain {beta}")
         if ref["after_cut"]:
             meas.append(None)
-            print(f"[A {tag} it={it} p={p}] weight-dependent checks skipped: an earlier iteration reached the clip kink")
+            print(f"[A {tag} it={it} p={p}] weight-dependent checks skipped: an earlier iteration {ref['after_cut']}")
             continue
         for name, tol in (("logits", 1e-5), ("value", 1e-5), ("act", 1e-5), ("logp", 1e-5), ("vtarg", 1e-5), ("adv", 2e-5)):
             e = scaled_err(bufs[name][p].cpu().numpy(), ref[name])
@@ -295,10 +382,17 @@ def _compare(L, stats, refs, it, tag):
             print(f"[A {tag} it={it} p={p}] step statistics compared up to step {ref['cut']} (a row at the clip kink), "
                   f"step_stats_err/tol={ratio[:, p].max():.3g}")
             continue
+        if not ref["resolved"]:
+            meas.append(None)
+            print(f"[A {tag} it={it} p={p}] step statistics compared over all steps, step_stats_err/tol="
+                  f"{ratio[:, p].max():.3g}; end state not compared: the float32 twin alone is "
+                  f"{_update_err(ref['twin_theta'], ref):.3g} of the update from float64, the trajectory without its last "
+                  f"step {_update_err(ref['theta_last'], ref):.3g}")
+            continue
         upd = _update_err(theta[p], ref)
         twin = _update_err(ref["twin_theta"], ref)
         bound = max(10.0 * twin, UPD_FLOOR)
-        guard = _update_err(ref["thetas"][-1], ref)          # the float64 trajectory without its last step
+        guard = _update_err(ref["theta_last"], ref)          # the float64 trajectory without its last step
         check(guard > 10.0 * bound, f"last-step guard {guard:.3g} is not 10x above the bound {bound:.3g}")
         check(upd < bound, f"update error {upd:.3g} >= {bound:.3g} (twin {twin:.3g})")
         em, ev_ = scaled_err(m[p], ref["m"]), scaled_err(v[p], ref["v"])
@@ -317,32 +411,38 @@ def _compare(L, stats, refs, it, tag):
     return fails, first, meas
 
 
-@pytest.mark.parametrize("mode", list(MODES))
-def test_bench_workload_iterations_match_oracle(mode, rollouts, oracle):
-    """Three bench-shaped iterations (sets 0, 1, 1): filter, preparation phase, the 320 steps' loss statistics and the
-    final weights / Adam state / beta powers / KL coefficient / returned stats of each, against the float64 oracle."""
-    sets = [_to_dev(r) for r in rollouts]
-    L = _learner(mode)
-    _assert_bench_shape(L, mode)
+def check_iterations(w, mode, oracle, tag):
+    """A: the three iterations of w.iter_sets on a bench-style learner against the float64 trajectory -> the failures."""
+    sets = [_to_dev(r) for r in w.sets]
+    L = _learner(w, mode)
+    _assert_bench_shape(w, L, mode)
     fails = []
-    for it, s in enumerate(ITER_SETS):
+    for it, s in enumerate(w.iter_sets):
         stats = _learn(L, sets[s])
         torch.cuda.synchronize()
-        fails += [msg for _, msg in _compare(L, stats, oracle[it], it, mode)[0]]
-    assert L._prep_graphs is not None and len(L._prep_graphs) == 1, getattr(L, "graph_error", None)
+        fails += [msg for _, msg in _compare(w, L, stats, oracle[it], it, tag)[0]]
+    assert L._prep_graphs is not None and len(L._prep_graphs) == len(set(w.iter_sets[1:])), getattr(L, "graph_error", None)
     if mode == "fp32":
         assert L._graph is not None, getattr(L, "graph_error", None)      # graph-captured one-step launches
+    return fails
+
+
+@pytest.mark.parametrize("mode", list(MODES))
+def test_bench_workload_iterations_match_oracle(mode, headline, oracle):
+    """Three bench-shaped iterations (sets 0, 1, 1): filter, preparation phase, the 320 steps' loss statistics and the
+    final weights / Adam state / beta powers / KL coefficient / returned stats of each, against the float64 oracle."""
+    fails = check_iterations(headline, mode, oracle, mode)
     assert not fails, "\n".join(fails)
 
 
-def _loss_grad(theta, cols, p, rows, klc, cfg, dtype):
+def _loss_grad(w, theta, cols, p, rows, klc, cfg, dtype):
     """autograd of the mean PPO loss over cols[*][p][rows] at theta -> (reference gradients, [5] stats in STEP_STATS
     order, max |v|).  The first gradient is torch's; float64 adds one per non-empty subset of the rows within NEAR_CLIP of
     the clip kink, with those rows on the other side of it."""
     O = _oracle()
     th = torch.from_numpy(theta).to(dtype).requires_grad_(True)
     c = {k: cols[k][p, rows].to(dtype) for k in COLS}
-    lg, v = O.fcnet_forward(th, c["obs"], 2 * A)
+    lg, v = O.fcnet_forward(th, c["obs"], 2 * w.A)
     loss, st = O.ppo_loss_from_outputs(lg, v, c["act"], c["logits"], c["logp"], c["value"], c["adv"], c["vtarg"], klc, cfg)
     near_rows = []
     if dtype == torch.float64:
@@ -360,20 +460,49 @@ def _loss_grad(theta, cols, p, rows, klc, cfg, dtype):
             float(v.detach().abs().max()))
 
 
-@pytest.mark.parametrize("mode", list(MODES))
-def test_every_step_matches_oracle_at_device_weights(mode, rollouts):
-    """First iteration, one eager launch per step (fused tail at the bench's G), teacher-forced: at every step the
-    device's reduced gradient against float64 autograd at the device's weights on the device's own shuffled columns, the
-    device's clip + Adam against float64 arithmetic from its own gradient and state, and the step's statistics."""
-    O = _oracle()
-    cfg = _cfg_o()
+def grad_check(w, mode, grad, th0, cols, p, rows, klc, cfg):
+    """B's gradient rule for one policy's step -> (scaled error, value-bias error over 1e-5 max|v|, kink rows present,
+    failure message or None).  Rows at the clip kink: the side the kernel took, and the twin's round-off around the side
+    it took."""
+    gtol = 5e-5 if MODES[mode]["mode"] == "tc" else 1e-5
+    shapes = [shp for _, shp in _oracle().fcnet_shapes(w.D, 2 * w.A)]
+    refs, st64, vmax = _loss_grad(w, th0, cols, p, rows, klc, cfg, torch.float64)
+    (g32,), _, _ = _loss_grad(w, th0, cols, p, rows, klc, cfg, torch.float32)
+    g64 = min(refs, key=lambda x: scaled_err(grad, x))
+    twin = g32 - min(refs, key=lambda x: scaled_err(g32, x)) + g64
+    e = scaled_err(grad, g64)
+    msg = f"gradient error {e:.3g} >= {gtol}" if e >= gtol else None
+    # value_out/bias = vf_loss_coeff * 2 * mean(v - R): its error is the mean error of the step's value forward,
+    # which the tensor-core path holds to 1e-5 of the value's scale (not a cancelling sum that round-off averages)
+    vb_allow = 2.0 * cfg.vf_loss_coeff * 1e-5 * vmax
+    allow = {w.VALUE_BIAS: vb_allow} if MODES[mode]["mode"] == "tc" else None
+    vb = abs(grad[w.VALUE_BIAS] - g64[w.VALUE_BIAS]) / vb_allow
+    try:
+        assert_grad_per_variable(grad, g64, twin, shapes, gtol, allow=allow)
+    except AssertionError as exc:
+        msg = f"{msg + '; ' if msg else ''}gradient per variable: {exc}"
+    return e, vb, len(refs) > 1, msg, st64
+
+
+def _step_rows(w, perms, p, s):
+    mb = int(perms[p, s // w.NB, s % w.NB])
+    return slice(mb * w.MB, (mb + 1) * w.MB)
+
+
+def check_every_step(w, mode, tag):
+    """B: the first iteration (set w.iter_sets[0]), one eager launch per step (fused tail at the bench's G), teacher-forced:
+    at every step the device's reduced gradient against float64 autograd at the device's weights on the device's own
+    shuffled columns, the device's clip + Adam against float64 arithmetic from its own gradient and state, and the step's
+    statistics.  Prints the worst errors per policy -> the failures (at most 20)."""
+    cfg = _cfg_o(w)
+    P = w.P
     f32 = lambda x: float(np.float32(x))
     b1, b2, lr, eps, clip = (f32(x) for x in (cfg.beta1, cfg.beta2, cfg.lr, cfg.adam_eps, cfg.grad_clip))
     gtol = 5e-5 if MODES[mode]["mode"] == "tc" else 1e-5
-    shapes = [shp for _, shp in O.fcnet_shapes(D, 2 * A)]
-    perms = rollouts[0]["perms"].numpy()
-    L = _learner(mode, persistent=False, use_graph=False)
-    _assert_bench_shape(L, mode, persistent=False)
+    r = w.sets[w.iter_sets[0]]
+    perms = r["perms"].numpy()
+    L = _learner(w, mode, persistent=False, use_graph=False)
+    _assert_bench_shape(w, L, mode, persistent=False)
     orig = L._sgd_step
     ctx = {"step": 0, "cols": None}
     fails = []
@@ -392,33 +521,19 @@ def test_every_step_matches_oracle_at_device_weights(mode, rollouts):
         torch.cuda.synchronize()
         grad, gn, th1, m1, v1 = (t.cpu().numpy().astype(np.float64) for t in (L.grad, L.gnorm, L.theta, L.m, L.v))
         bp1 = L.beta_pow.cpu().numpy()
-        ss = _device_step_stats(b["step_stats"][s:s + 1].cpu().numpy())[0]
+        ss = _device_step_stats(b["step_stats"][s:s + 1].cpu().numpy(), w.MB)[0]
         if ctx["cols"] is None:
             ctx["cols"] = {k: src[k].cpu() for k in COLS}
+
         def one(p):
-            mb = int(perms[p, s // NB, s % NB])
-            rows = slice(mb * MB, (mb + 1) * MB)
+            rows = _step_rows(w, perms, p, s)
             # 1. gradient
-            refs, st64, vmax = _loss_grad(th0[p], ctx["cols"], p, rows, klc[p], cfg, torch.float64)
-            (g32,), _, _ = _loss_grad(th0[p], ctx["cols"], p, rows, klc[p], cfg, torch.float32)
-            # rows at the clip kink: the side the kernel took, and the twin's round-off around the side it took
-            g64 = min(refs, key=lambda x: scaled_err(grad[p], x))
-            twin = g32 - min(refs, key=lambda x: scaled_err(g32, x)) + g64
-            if len(refs) > 1:
-                worst["kink"][p] += 1
-            e = scaled_err(grad[p], g64)
+            e, vb, kink, msg, st64 = grad_check(w, mode, grad[p], th0[p], ctx["cols"], p, rows, klc[p], cfg)
+            worst["kink"][p] += kink
             worst["grad"][p] = max(worst["grad"][p], e)
-            if e >= gtol:
-                fail(s, p, f"gradient error {e:.3g} >= {gtol}")
-            # value_out/bias = vf_loss_coeff * 2 * mean(v - R): its error is the mean error of the step's value forward,
-            # which the tensor-core path holds to 1e-5 of the value's scale (not a cancelling sum that round-off averages)
-            allow = {VALUE_BIAS: 2.0 * cfg.vf_loss_coeff * 1e-5 * vmax} if MODES[mode]["mode"] == "tc" else None
-            vb = abs(grad[p][VALUE_BIAS] - g64[VALUE_BIAS]) / (2.0 * cfg.vf_loss_coeff * 1e-5 * vmax)
             worst["vbias"][p] = max(worst["vbias"][p], vb)
-            try:
-                assert_grad_per_variable(grad[p], g64, twin, shapes, gtol, allow=allow)
-            except AssertionError as exc:
-                fail(s, p, f"gradient per variable: {exc}")
+            if msg is not None:
+                fail(s, p, msg)
             # 2. global-norm clip + TF1 Adam in float64 from the device's own gradient and state
             norm = float(np.sqrt((grad[p] ** 2).sum()))
             gc = grad[p] * (clip * min(1.0 / norm, 1.0 / clip))
@@ -444,60 +559,85 @@ def test_every_step_matches_oracle_at_device_weights(mode, rollouts):
         list(pool.map(one, range(P)))
 
     L._sgd_step = step
-    r = _to_dev(rollouts[0])
     threads = torch.get_num_threads()
     torch.set_num_threads(max(1, (os.cpu_count() or 1) // P))
     try:
         with ThreadPoolExecutor(P) as pool:      # the float64 autograd of the P policies side by side
-            _learn(L, r)
+            _learn(L, _to_dev(r))
     finally:
         torch.set_num_threads(threads)
     torch.cuda.synchronize()
-    assert ctx["step"] == STEPS
+    assert ctx["step"] == w.STEPS
     for p in range(P):
-        print(f"[B {mode} it=0 p={p}] grad_err={worst['grad'][p]:.3g} (tol {gtol}) gnorm_err={worst['gnorm'][p]:.3g} "
+        print(f"[B {tag} it=0 p={p}] grad_err={worst['grad'][p]:.3g} (tol {gtol}) gnorm_err={worst['gnorm'][p]:.3g} "
               f"m_err={worst['m'][p]:.3g} v_err={worst['v'][p]:.3g} theta_err/tol={worst['theta'][p]:.3g} "
               f"step_stats_err/tol={worst['stat'][p]:.3g} value_bias_err/(1e-5 max|v|)={worst['vbias'][p]:.3g} "
               f"steps_with_a_row_at_the_clip_kink={int(worst['kink'][p])}")
+    return fails
+
+
+@pytest.mark.parametrize("mode", list(MODES))
+def test_every_step_matches_oracle_at_device_weights(mode, headline):
+    """First iteration, one eager launch per step (fused tail at the bench's G), teacher-forced: at every step the
+    device's reduced gradient against float64 autograd at the device's weights on the device's own shuffled columns, the
+    device's clip + Adam against float64 arithmetic from its own gradient and state, and the step's statistics."""
+    fails = check_every_step(headline, mode, mode)
     assert not fails, "\n".join(fails)
 
 
-def test_persistent_launch_equals_one_step_launches(rollouts):
-    """Fixed-order reduction: the bench-style learner (ONE persistent launch of 320 steps, graph-replayed preparation) and
-    the learner of B (one eager launch per step) leave bit-identical state after each of three iterations."""
-    sets = [_to_dev(r) for r in rollouts]
-    La = _learner("tc-fixed")
-    Lb = _learner("tc-fixed", persistent=False, use_graph=False)
-    _assert_bench_shape(La, "tc-fixed")
-    _assert_bench_shape(Lb, "tc-fixed", persistent=False)
-    for it, s in enumerate(ITER_SETS):
+def check_persistent_equals_one_step(w):
+    """C: with the fixed-order reduction, the bench-style learner (ONE persistent launch per iteration, graph-replayed
+    preparation) and the learner of B (one eager launch per step) leave bit-identical state after each iteration."""
+    sets = [_to_dev(r) for r in w.sets]
+    La = _learner(w, "tc-fixed")
+    Lb = _learner(w, "tc-fixed", persistent=False, use_graph=False)
+    _assert_bench_shape(w, La, "tc-fixed")
+    _assert_bench_shape(w, Lb, "tc-fixed", persistent=False)
+    for it, s in enumerate(w.iter_sets):
         sa, sb = _learn(La, sets[s]), _learn(Lb, sets[s])
         torch.cuda.synchronize()
         a, b = La._bufs["step_stats"], Lb._bufs["step_stats"]
-        diff = (a != b).reshape(STEPS, -1).any(dim=1).nonzero()
+        diff = (a != b).reshape(w.STEPS, -1).any(dim=1).nonzero()
         assert len(diff) == 0, f"iteration {it}: step statistics first differ at step {int(diff[0])}"
         for name in ("theta", "m", "v", "beta_pow", "kl_coeff", "filt_n", "filt_M", "filt_S"):
             assert torch.equal(getattr(La, name), getattr(Lb, name)), (it, name)
         assert sa == sb, it
 
 
-def test_one_wrong_minibatch_is_caught(rollouts, oracle):
+def test_persistent_launch_equals_one_step_launches(headline):
+    """Fixed-order reduction: the bench-style learner (ONE persistent launch of 320 steps, graph-replayed preparation) and
+    the learner of B (one eager launch per step) leave bit-identical state after each of three iterations."""
+    check_persistent_equals_one_step(headline)
+
+
+def check_repeated_minibatch(w, oracle, tag):
+    """D: in the first iteration, policy q's step s (w.control) repeats the minibatch of step s - 1 of the same epoch.
+    Against the unmodified oracle, A must flag step s of policy q first and pass the other policies; if q's reference
+    trajectory is compared to its end, q's final weights must be off by more than 10x the bound."""
+    q, target = w.control
+    cut = oracle[0][q]["cut"]
+    assert cut is None or cut > target, f"policy {q}'s reference reaches the clip kink at step {cut}"
+    e, i = divmod(target, w.NB)
+    r = dict(w.sets[w.iter_sets[0]])
+    perms = r["perms"].clone()
+    assert i > 0 and perms[q, e, i] != perms[q, e, i - 1]
+    perms[q, e, i] = perms[q, e, i - 1]
+    r["perms"] = perms
+    L = _learner(w, "tc-fixed")
+    _assert_bench_shape(w, L, "tc-fixed")
+    stats = _learn(L, _to_dev(r))
+    torch.cuda.synchronize()
+    fails, first, meas = _compare(w, L, stats, oracle[0], 0, tag)
+    assert first == (target, q), first
+    if cut is None:
+        assert meas[q]["upd"] > 10.0 * meas[q]["bound"], meas[q]
+    assert not [msg for p, msg in fails if p != q], fails
+
+
+def test_one_wrong_minibatch_is_caught(headline, oracle):
     """Negative control at the bench shape, valid inputs: policy 2's step 200 (epoch 6, position 8) repeats the minibatch of
     step 199.  Against the unmodified oracle, A's checks must flag step 200 of policy 2 first and policy 2's final weights,
     and pass the other policies.  (Policy 2: its reference trajectory has no row at the clip kink in this iteration, so
     the whole trajectory is compared; the unfaulted learner passes the same checks in the iterations test.)"""
-    q = 2
-    assert oracle[0][q]["cut"] is None
-    r = dict(rollouts[0])
-    perms = r["perms"].clone()
-    assert perms[q, 6, 8] != perms[q, 6, 7]
-    perms[q, 6, 8] = perms[q, 6, 7]
-    r["perms"] = perms
-    L = _learner("tc-fixed")
-    _assert_bench_shape(L, "tc-fixed")
-    stats = _learn(L, _to_dev(r))
-    torch.cuda.synchronize()
-    fails, first, meas = _compare(L, stats, oracle[0], 0, "fault")
-    assert first == (200, q), first
-    assert meas[q]["upd"] > 10.0 * meas[q]["bound"], meas[q]
-    assert not [msg for p, msg in fails if p != q], fails
+    assert headline.control == (2, 200) and oracle[0][2]["cut"] is None
+    check_repeated_minibatch(headline, oracle, "fault")
